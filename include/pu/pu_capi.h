@@ -376,9 +376,20 @@ PU_API pu_status pu_channel_apply_batch(pu_ctx* ctx, const pu_channel_config* cf
 
 /* The CFO injector of the reference's tools (tools/test_iwaveform.cpp:67-118): analytic signal through FFT / inverse FFT over the next
  * power of two, rotation by the float phase recurrence, real part -- applied by the tools to the CLEAN transmit audio before the
- * channel (:501-506), which is where pu_linksim_run applies it (pu_sweep_mode.cfo_hz, once per TX pool waveform).  Host function, in
+ * channel (:501-506), which is where pu_linksim_run applies it (pu_sweep_mode.cfo_hz, once per TX pool waveform; fresh payloads take
+ * pu_tools_cfo_apply_batch below).  Host function, in
  * place; arrays shorter than 128 samples or |cfo| < 0.001 Hz are left untouched.  Bit-identical to the tool. */
 PU_API pu_status pu_tools_apply_cfo(float* samples, size_t n, float cfo_hz, float sample_rate);
+/* The same injector on the GPU for a batch of rows (csrc/tools_cfo_gpu.cu): a handle per (n, cfo_hz, sample_rate) holds the twiddles,
+ * the rotator of the phase recurrence (both built by the host function's own code) and 64 MiB of scratch.  apply_batch works in place
+ * on samples[b*stride .. b*stride + n) for b < B; every sample is bit-identical to pu_tools_apply_cfo on that row, and the samples
+ * between n and stride are not written.  For n < 128 or |cfo_hz| < 0.001 rows are untouched and nothing is launched.  n up to 2^20
+ * (PU_ERR_UNSUPPORTED above; the host function has no such limit).  PU_MEM_DEVICE enqueues on `stream` and does not synchronise the
+ * host; PU_MEM_HOST stages the rows through the device and returns when they are written back. */
+typedef struct pu_tools_cfo pu_tools_cfo;
+PU_API pu_status pu_tools_cfo_create(pu_ctx* ctx, size_t n, float cfo_hz, float sample_rate, pu_tools_cfo** out);
+PU_API void pu_tools_cfo_destroy(pu_tools_cfo* h);
+PU_API pu_status pu_tools_cfo_apply_batch(pu_tools_cfo* h, float* samples, size_t B, size_t stride, pu_memspace space, void* stream);
 
 /* WattersonChannel::applyCFO (hf_channel.hpp:173-232), the channel's optional carrier-frequency-offset injector, applied IN PLACE to
  * every row of samples[B][stride] (L samples each) with cfo_hz[b] and a CFO phase of 0 at the start of the row: down-mix around
@@ -465,7 +476,9 @@ typedef struct {
     float cfo_hz;               /* the tools' --cfo: pu_tools_apply_cfo on every TX waveform (silence included) before the channel; 0 = none */
     uint32_t fresh_payloads;    /* 1: a new payload per trial, encoded and modulated on the GPU (pu_*_tx_batch) inside the batch, as the tools do
                                  * (tools/test_dpsk_snr.cpp:40-60, tools/test_mode_snr.cpp:40-60), instead of the pool of TX waveforms; the
-                                 * payload is a pure function of (base_seed, mode, SNR index, trial).  Not with the chirp waveforms or cfo_hz. */
+                                 * payload is a pure function of (base_seed, mode, SNR index, trial).  Each row is built in the pool's order: body
+                                 * behind the lead silence and the chirp pair, peak normalisation over chirp and body, cfo_hz through
+                                 * pu_tools_cfo_apply_batch over the whole row, then the row's noise level. */
 } pu_sweep_mode;
 
 typedef struct {

@@ -252,6 +252,40 @@ def tools_apply_cfo(samples, cfo_hz, sample_rate=48000.0):
     return x
 
 
+class ToolsCfo:
+    """pu_tools_cfo: the same injector on the GPU for every row of a batch, bit-identical to tools_apply_cfo row by row."""
+
+    def __init__(self, ctx, n, cfo_hz, sample_rate=48000.0):
+        self.ctx, self.n = ctx, int(n)
+        self._h = C.c_void_p()
+        check(lib().pu_tools_cfo_create(ctx._h, C.c_size_t(self.n), C.c_float(cfo_hz), C.c_float(sample_rate), C.byref(self._h)))
+
+    def close(self):
+        if self._h:
+            lib().pu_tools_cfo_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def apply_batch(self, x):
+        """In place on the first n samples of every row of x [B, stride] (float32, rows contiguous; numpy => host, torch.cuda => device
+        on torch's current stream).  Returns x."""
+        if _is_torch(x):
+            import torch
+            assert x.dtype == torch.float32 and x.dim() == 2 and x.stride(1) == 1
+            B, stride = x.shape[0], x.stride(0)
+        else:
+            assert x.dtype == np.float32 and x.ndim == 2 and x.strides[1] == 4 and x.strides[0] % 4 == 0
+            B, stride = x.shape[0], x.strides[0] // 4
+        sp = _space(x)
+        check(lib().pu_tools_cfo_apply_batch(self._h, _ptr(x), C.c_size_t(B), C.c_size_t(stride), sp, _stream(sp)))
+        return x
+
+
 def chirp_phase_cycles():
     """Cycles per phase of the two-tier chirp search since the last call (pu_chirp_phase_cycles)."""
     out = (C.c_uint64 * 8)()

@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 
 #include <atomic>
+#include <complex>
 #include <cstdarg>
 #include <cstdint>
 #include <cstdio>
@@ -106,6 +107,10 @@ inline void chirp_dev_bind(ChirpDev& c, const float* dev_table) {
     c.lp = c.dec + 4 * static_cast<size_t>(c.nd);
 }
 void tools_apply_cfo(float* samples, size_t n, float cfo_hz, float sample_rate);     // tools_cfo.cpp
+// tables of tools_apply_cfo: tw[fft_size / 2] twiddles exp(-2 pi i k / fft_size) from the float angle, rot[n] = (cos, sin) of the float
+// phase recurrence; the device injector (tools_cfo_gpu.cu) uploads the same tables
+void tools_cfo_twiddles(size_t fft_size, std::complex<float>* tw);
+void tools_cfo_rotator(size_t n, float cfo_hz, float sample_rate, std::complex<float>* rot);
 float channel_power_sum(const float* tx, size_t L);                                   // channel.cu: the two halves of pu_channel_noise_std
 float channel_noise_std_from_sum(float acc, size_t L, float snr_db, int convention);
 cudaError_t chirp_search_stats(unsigned long long* out);

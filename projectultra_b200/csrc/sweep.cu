@@ -134,6 +134,28 @@ __global__ void fresh_payload_kernel(uint8_t* __restrict__ pay, size_t kb, uint3
     for (size_t k = 0; k < 8 && 8 * w + k < kb; ++k) pay[b * kb + 8 * w + k] = 8 * w + k < payload_bytes ? static_cast<uint8_t>(z >> (8 * k)) : 0;
 }
 
+// fresh payloads behind the chirp pair, one CTA per row: the pair into [lead, lead + chirp_len), then the tools' peak normalisation
+// w * (peak / max|w|) over chirp and body together -- the order of the host pool (ModeEngine::build)
+__global__ void chirp_peak_kernel(float* __restrict__ tx, size_t L, size_t lead, const float* __restrict__ chirp, size_t chirp_len, size_t body_len, float peak) {
+    __shared__ float red[32];
+    float* row = tx + blockIdx.x * L + lead;
+    const size_t len = chirp_len + body_len;
+    float mx = 0.0f;
+    for (size_t i = threadIdx.x; i < len; i += blockDim.x) {
+        const float v = i < chirp_len ? chirp[i] : row[i];
+        if (i < chirp_len) row[i] = v;
+        mx = fmaxf(mx, fabsf(v));
+    }
+    if (peak <= 0.0f) return;
+    for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = mx;
+    __syncthreads();
+    mx = red[0];
+    for (unsigned w = 1; w < blockDim.x / 32; ++w) mx = fmaxf(mx, red[w]);
+    const float g = __fdiv_rn(peak, mx);
+    for (size_t i = threadIdx.x; i < len; i += blockDim.x) row[i] = __fmul_rn(row[i], g);
+}
+
 __global__ void mask_short_kernel(uint8_t* __restrict__ ok, const int32_t* __restrict__ n_llr, size_t B) {
     // no sync / fewer than one codeword of soft bits is a lost frame (tools/test_mode_snr.cpp:72-77): override the decoder's verdict
     const size_t i = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x;
@@ -156,14 +178,18 @@ struct ModeEngine {
     std::vector<float> noise_std;        // [n_snr][pool]; fresh payloads: [n_snr] SNR factors of pu_channel_noise_std_batch
     Buffer d_tx, d_payload;              // [pool][L] floats, [pool][kb] bytes
     bool fresh = false;                  // pu_sweep_mode.fresh_payloads: TX inside the batch
-    size_t body_len = 0;                 // samples the transmitter writes per frame (L = lead + body + tail)
+    size_t body_len = 0;                 // samples the transmitter writes per frame (L = lead + chirp + body + tail)
+    size_t chirp_len = 0;                // fresh payloads of the chirp waveforms: the pair in d_chirp, written in front of every body
+    Buffer d_chirp;
+    pu_tools_cfo* tools_cfo = nullptr;   // fresh payloads with cfo_hz: the tools' injector over every row
 
     ~ModeEngine() {
         if (ofdm) pu_ofdm_destroy(ofdm);
         if (dpsk) pu_dpsk_destroy(dpsk);
         if (mcd) pu_mcdpsk_destroy(mcd);
         if (ldpc && own_ldpc) pu_ldpc_destroy(ldpc);
-        d_tx.release(); d_payload.release();
+        if (tools_cfo) pu_tools_cfo_destroy(tools_cfo);
+        d_tx.release(); d_payload.release(); d_chirp.release();
     }
 
     pu_status build(pu_ctx* c, const pu_sweep_mode* m, uint32_t mode_index, const SweepPlan& p, cudaStream_t st, pu_ldpc* shared_ldpc = nullptr) {
@@ -191,12 +217,25 @@ struct ModeEngine {
             if ((s = pu_mcdpsk_create(c, &m->mcdpsk, &mcd)) != PU_OK) return s;
         }
         const auto t1 = now();
+        const float fs = is_ofdm ? static_cast<float>(m->ofdm.sample_rate) : is_dpsk ? m->dpsk.sample_rate : m->mcdpsk.sample_rate;
+        std::vector<float> chirp;             // the pair does not depend on the payload (tx_cfo_hz for OFDM, 0 for MC-DPSK)
+        if (m->waveform == PU_WF_OFDM_CHIRP || m->waveform == PU_WF_MCDPSK_CHIRP) {
+            size_t n = 0;
+            pu_chirp_generate(fs, is_ofdm ? m->ofdm.tx_cfo_hz : 0.0f, nullptr, 0, &n);
+            chirp.resize(n);
+            if ((s = pu_chirp_generate(fs, is_ofdm ? m->ofdm.tx_cfo_hz : 0.0f, chirp.data(), n, &n)) != PU_OK) return s;
+        }
         fresh = m->fresh_payloads != 0;
         if (fresh) {
-            PU_REQUIRE(m->waveform != PU_WF_OFDM_CHIRP && m->waveform != PU_WF_MCDPSK_CHIRP && m->cfo_hz == 0.0f,
-                       "pu_linksim_run: fresh_payloads is not available with the chirp waveforms or cfo_hz (the preamble pair and the tools' CFO injector are built on the host)");
             if ((s = tx_batch(nullptr, 0, nullptr, 0, st)) != PU_OK) return s;      // queries body_len
-            L = m->lead_samples + body_len + m->tail_samples;
+            chirp_len = chirp.size();
+            L = m->lead_samples + chirp_len + body_len + m->tail_samples;
+            if (chirp_len) {
+                if ((s = d_chirp.reserve(chirp_len * sizeof(float))) != PU_OK) return s;
+                PU_CUDA_TRY(cudaMemcpyAsync(d_chirp.ptr, chirp.data(), chirp_len * sizeof(float), cudaMemcpyHostToDevice, st));
+                PU_CUDA_TRY(cudaStreamSynchronize(st));       // `chirp` is pageable and goes out of scope
+            }
+            if (m->cfo_hz != 0.0f && (s = pu_tools_cfo_create(c, L, m->cfo_hz, fs, &tools_cfo)) != PU_OK) return s;
             noise_std.resize(m->n_snr);
             for (uint32_t si = 0; si < m->n_snr; ++si) {
                 const float snr = m->snr_first_db + si * m->snr_step_db;
@@ -206,14 +245,6 @@ struct ModeEngine {
             return PU_OK;
         }
         // TX pool on the host (the reference's modulators run per trial on the CPU too): payload -> LDPC encode -> modulate [-> chirp in front]
-        std::vector<float> chirp;
-        if (m->waveform == PU_WF_OFDM_CHIRP || m->waveform == PU_WF_MCDPSK_CHIRP) {
-            const float fs = is_ofdm ? static_cast<float>(m->ofdm.sample_rate) : m->mcdpsk.sample_rate;
-            size_t n = 0;
-            pu_chirp_generate(fs, is_ofdm ? m->ofdm.tx_cfo_hz : 0.0f, nullptr, 0, &n);
-            chirp.resize(n);
-            if ((s = pu_chirp_generate(fs, is_ofdm ? m->ofdm.tx_cfo_hz : 0.0f, chirp.data(), n, &n)) != PU_OK) return s;
-        }
         std::vector<std::vector<float>> waves(pool);
         std::vector<uint8_t> payloads(static_cast<size_t>(pool) * kb, 0);
         for (uint32_t i = 0; i < pool; ++i) {
@@ -243,10 +274,7 @@ struct ModeEngine {
                 const float g = m->peak / mx;
                 for (float& v : w) v *= g;
             }
-            if (m->cfo_hz != 0.0f) {                          // the tools' --cfo: the clean audio, before the channel (test_iwaveform.cpp:501-506)
-                const float fs = is_ofdm ? static_cast<float>(m->ofdm.sample_rate) : is_dpsk ? m->dpsk.sample_rate : m->mcdpsk.sample_rate;
-                tools_apply_cfo(w.data(), w.size(), m->cfo_hz, fs);
-            }
+            if (m->cfo_hz != 0.0f) tools_apply_cfo(w.data(), w.size(), m->cfo_hz, fs);   // the tools' --cfo: the clean audio, before the channel (test_iwaveform.cpp:501-506)
             waves[i] = std::move(w);
         }
         const auto t2 = now();
@@ -270,16 +298,28 @@ struct ModeEngine {
         return PU_OK;
     }
 
-    // fresh payloads: LDPC encode + modulate B payloads on the device into out[B][L] at column lead_samples (the caller clears the rows when
-    // the mode has silence); B = 0 queries body_len
+    // fresh payloads: LDPC encode + modulate B payloads on the device into out[B][L] at column lead_samples + chirp_len (the caller clears
+    // the rows when the mode has silence); B = 0 queries body_len.  Behind a chirp the peak normalisation waits for the pair (finish_rows).
     pu_status tx_batch(const uint8_t* d_pay, size_t B, float* out, size_t row, cudaStream_t st) {
-        float* at = out ? out + md->lead_samples : nullptr;
+        float* at = out ? out + md->lead_samples + chirp_len : nullptr;
+        const float peak = chirp_len ? 0.0f : md->peak;
         const unsigned wf = md->waveform;
-        if (wf == PU_WF_OFDM || wf == PU_WF_OFDM_SC)
-            return pu_ofdm_tx_batch(ofdm, ldpc, d_pay, kb, md->payload_bytes, B, wf == PU_WF_OFDM_SC ? 1 : 0, md->peak, at, row, &body_len, PU_MEM_DEVICE, st);
+        if (wf == PU_WF_OFDM || wf == PU_WF_OFDM_SC || wf == PU_WF_OFDM_CHIRP)
+            return pu_ofdm_tx_batch(ofdm, ldpc, d_pay, kb, md->payload_bytes, B, wf == PU_WF_OFDM_SC ? 1 : 0, peak, at, row, &body_len, PU_MEM_DEVICE, st);
         if (wf == PU_WF_DPSK || wf == PU_WF_DPSK_ACQ)
-            return pu_dpsk_tx_batch(dpsk, ldpc, d_pay, kb, md->payload_bytes, B, md->peak, at, row, &body_len, PU_MEM_DEVICE, st);
-        return pu_mcdpsk_tx_batch(mcd, ldpc, d_pay, kb, md->payload_bytes, B, md->peak, at, row, &body_len, PU_MEM_DEVICE, st);
+            return pu_dpsk_tx_batch(dpsk, ldpc, d_pay, kb, md->payload_bytes, B, peak, at, row, &body_len, PU_MEM_DEVICE, st);
+        return pu_mcdpsk_tx_batch(mcd, ldpc, d_pay, kb, md->payload_bytes, B, peak, at, row, &body_len, PU_MEM_DEVICE, st);
+    }
+
+    // fresh payloads, after tx_batch: the chirp pair and the peak normalisation, then the tools' CFO injector over the whole row
+    pu_status finish_rows(float* out, size_t B, cudaStream_t st) {
+        if (chirp_len) {
+            chirp_peak_kernel<<<static_cast<unsigned>(B), 256, 0, st>>>(out, L, md->lead_samples, static_cast<const float*>(d_chirp.ptr), chirp_len,
+                                                                       body_len, md->peak);
+            ctx->launches.fetch_add(1);
+            PU_CUDA_TRY(cudaGetLastError());
+        }
+        return tools_cfo ? pu_tools_cfo_apply_batch(tools_cfo, out, B, L, PU_MEM_DEVICE, st) : PU_OK;
     }
 
     // demodulate -> decode (device pointers, stream st); scratch: llr [B][648], n_llr [B], sync [B][8] (int/float)
@@ -661,6 +701,7 @@ pu_status pu_linksim_run(pu_ctx* ctx, const pu_sweep_desc* d, uint64_t* counters
                     PU_CUDA_TRY(cudaGetLastError());
                     if (d->modes[m].lead_samples || d->modes[m].tail_samples) PU_CUDA_TRY(cudaMemsetAsync(ftx, 0, B * L * sizeof(float), st));
                     if ((s2 = eng.tx_batch(pay, B, ftx, L, st)) != PU_OK) return s2;
+                    if ((s2 = eng.finish_rows(ftx, B, st)) != PU_OK) return s2;
                     if ((s2 = pu_channel_noise_std_batch(ctx, ftx, L, L, B, stds, eng.convention, static_cast<float*>(d_fstd.ptr), st)) != PU_OK) return s2;
                     tx_pool = ftx; stds = static_cast<const float*>(d_fstd.ptr); payloads = pay; pool_count = B;
                 }

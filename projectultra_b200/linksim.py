@@ -128,14 +128,18 @@ class LinkSim:
     cfg selects the waveform: capi.ModemConfig (OFDM, presynced frame = 2 LTS + data, tools/test_ofdm_chirp_pilots.cpp:
     183-191), capi.DpskConfig (single-carrier DPSK, Barker preamble + data, tools/test_dpsk_snr.cpp:47-52, genie data
     start) or capi.McDpskConfig (multi-carrier DPSK, training + reference + data, tools/test_mc_dpsk.cpp:180-196).
-    peak=0.5 applies the tools' peak normalisation (tools/test_mode_snr.cpp:54-56).
+    peak=0.5 applies the tools' peak normalisation (tools/test_mode_snr.cpp:54-56).  tools_cfo_hz applies the tools' tuning error
+    (tools/test_iwaveform.cpp:501-506) to every clean TX waveform after it: capi.tools_apply_cfo on the pool, capi.ToolsCfo on fresh frames.
+    lead_samples / tail_samples (layout 'chirp') surround every frame with silence before both, as the tools do (test_iwaveform.cpp:396-459):
+    a positive tuning error moves the up chirp's apparent start in front of the frame, so without a lead the chirp's timing is lost.
 
     Frames are identified by (snr index, trial index); frame -> (tx waveform, seed) is a pure function, so any
     frame can be regenerated, and ranks take disjoint trial ranges with no data exchange (SURVEY §8e)."""
 
     def __init__(self, ctx, cfg, channel="awgn", payload_bytes=40, pool=64, snr_convention=None, pool_seed=12345,
                  max_iter=50, device=None, code_rate=None, peak=None, layout="presynced", chunk=960, fresh_payload=False,
-                 acquire=False, precision="exact", payloads=None):
+                 acquire=False, precision="exact", payloads=None, tools_cfo_hz=0.0,
+                 lead_samples=0, tail_samples=0):
         import torch
         self.ctx, self.cfg = ctx, cfg
         self.precision = precision
@@ -156,8 +160,8 @@ class LinkSim:
             # setFrequencyOffset -> process (tools/test_iwaveform.cpp:127-160)
             assert layout in ("presynced", "sc", "chirp")
             self.layout, self.chunk = layout, chunk
+            chirp = capi.chirp_generate(float(cfg.sample_rate), float(cfg.tx_cfo_hz)) if layout == "chirp" else None
             if layout == "chirp":
-                chirp = capi.chirp_generate(float(cfg.sample_rate), float(cfg.tx_cfo_hz))
                 build = lambda coded: np.concatenate([chirp, ofdm_tx(cfg, coded, 0)])
             else:
                 build = lambda coded: ofdm_tx(cfg, coded, 1 if layout == "sc" else 0)
@@ -167,6 +171,7 @@ class LinkSim:
             self.demod = capi.DpskDemodulator(ctx, cfg)
             self.data_start = 39 * cfg.samples_per_symbol                 # Barker-13 x 3 (dpsk.hpp:202-204)
             self.layout = "presynced"
+            chirp = None
             build = lambda coded: capi.dpsk_tx(cfg, coded, 0)
         elif isinstance(cfg, capi.McDpskConfig):
             self.kind = "mcdpsk"
@@ -177,8 +182,8 @@ class LinkSim:
             # or with fewer than 648 soft bits is lost
             assert layout in ("presynced", "chirp")
             self.layout = layout
+            chirp = capi.chirp_generate(float(cfg.sample_rate), 0.0) if layout == "chirp" else None
             if layout == "chirp":
-                chirp = capi.chirp_generate(float(cfg.sample_rate), 0.0)
                 build = lambda coded: np.concatenate([chirp, capi.mcdpsk_tx(cfg, coded)])
             else:
                 build = lambda coded: capi.mcdpsk_tx(cfg, coded)
@@ -194,15 +199,22 @@ class LinkSim:
         assert not self.acquire or self.kind == "dpsk", "acquire=True is the DPSK Barker path; OFDM uses layout='sc'"
         self.fresh_payload = bool(fresh_payload)
         self.peak = peak
-        assert not self.fresh_payload or self.layout != "chirp", "fresh payloads behind a chirp: use the host-built pool"
+        self.chirp = None if chirp is None else torch.from_numpy(chirp).to(self.device)
+        self.sample_rate = float(cfg.sample_rate)
+        self.tools_cfo_hz = float(tools_cfo_hz)
+        self.tools_cfo = None                  # capi.ToolsCfo of the fresh frames, made for their length on first use
+        self.lead, self.tail = int(lead_samples), int(tail_samples)
+        assert not (self.lead or self.tail) or self.layout == "chirp", "silence around a frame needs the acquiring receiver (layout='chirp')"
         self.payload_bytes = payload_bytes
         rng = np.random.default_rng(pool_seed)
         # payloads: explicit [pool, payload_bytes] array (e.g. the splitmix64 pool of the C++ sweep driver, capi.Sweep.payload)
         self.payloads = (rng.integers(0, 256, (pool, payload_bytes), dtype=np.uint8) if payloads is None
                          else np.ascontiguousarray(payloads, dtype=np.uint8).reshape(pool, payload_bytes))
-        waves = [build(capi.ldpc_encode(rate, p)) for p in self.payloads]
+        waves = [np.pad(build(capi.ldpc_encode(rate, p)), (self.lead, self.tail)) for p in self.payloads]
         if peak is not None:
             waves = [(w * (np.float32(peak) / np.abs(w).max())).astype(np.float32) for w in waves]
+        if self.tools_cfo_hz != 0.0:
+            waves = [capi.tools_apply_cfo(w, self.tools_cfo_hz, self.sample_rate) for w in waves]
         self.L = len(waves[0])
         self.tx_host = np.stack(waves)
         self.tx_pool = torch.from_numpy(self.tx_host).to(self.device)
@@ -263,8 +275,9 @@ class LinkSim:
                     host=dict(tx_index=tx_index, noise_std=std, seed=seeds, snr_idx=snr_idx))
 
     def fresh_frames(self, batch, snr_points):
-        """Payloads drawn on the device (torch Philox stream keyed by the batch's first frame seed), pu_ofdm_tx_batch, and the
-        per-frame noise level of the tools' SNR convention.  Returns (payload [B, kb] uint8 zero-padded, tx [B, L], noise_std [B])."""
+        """Payloads drawn on the device (torch Philox stream keyed by the batch's first frame seed), pu_*_tx_batch, and the per-frame
+        noise level of the tools' SNR convention.  Rows are built in the pool's order: chirp pair + body, peak normalisation over both,
+        tools_cfo_hz through capi.ToolsCfo.  Returns (payload [B, kb] uint8 zero-padded, tx [B, L], noise_std [B])."""
         import torch
         B = batch["seed"].shape[0]
         g = torch.Generator(device=self.device)
@@ -272,12 +285,20 @@ class LinkSim:
         kb = self.ldpc.info_bytes
         payload = torch.zeros((B, kb), dtype=torch.uint8, device=self.device)
         payload[:, :self.payload_bytes] = torch.randint(0, 256, (B, self.payload_bytes), dtype=torch.uint8, device=self.device, generator=g)
-        assert self.layout != "chirp", "fresh payloads behind a chirp: build the pool on the host (layout='chirp' without fresh_payload)"
+        # behind a chirp the peak is taken over chirp and body: the transmitter leaves the body unscaled
+        peak = float(self.peak) if self.peak and self.chirp is None else 0.0
         if self.kind == "ofdm":
-            tx = self.demod.tx_batch(self.ldpc, payload[:, :self.payload_bytes], layout=1 if self.layout == "sc" else 0,
-                                     peak=float(self.peak) if self.peak else 0.0)
+            tx = self.demod.tx_batch(self.ldpc, payload[:, :self.payload_bytes], layout=1 if self.layout == "sc" else 0, peak=peak)
         else:     # pu_dpsk_tx_batch / pu_mcdpsk_tx_batch
-            tx = self.demod.tx_batch(self.ldpc, payload[:, :self.payload_bytes], peak=float(self.peak) if self.peak else 0.0)
+            tx = self.demod.tx_batch(self.ldpc, payload[:, :self.payload_bytes], peak=peak)
+        if self.chirp is not None:
+            tx = torch.nn.functional.pad(torch.cat([self.chirp.expand(B, -1), tx], dim=1), (self.lead, self.tail))
+            if self.peak:
+                tx = tx * (torch.tensor(float(self.peak), dtype=torch.float32, device=self.device) / tx.abs().amax(dim=1, keepdim=True))
+        if self.tools_cfo_hz != 0.0:
+            if self.tools_cfo is None or self.tools_cfo.n != tx.shape[1]:
+                self.tools_cfo = capi.ToolsCfo(self.ctx, tx.shape[1], self.tools_cfo_hz, self.sample_rate)
+            self.tools_cfo.apply_batch(tx)
         snr = np.asarray(snr_points, np.float32)
         fac = (np.power(np.float32(10.0), -snr / np.float32(20.0)) if self.snr_convention == 0
                else np.power(np.float32(10.0), snr / np.float32(10.0))).astype(np.float32)

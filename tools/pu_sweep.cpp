@@ -158,7 +158,7 @@ int env_int(const char* n, int d) { const char* v = getenv(n); return v ? atoi(v
 int main(int argc, char** argv) {
     const int rank = env_int("RANK", 0), world = env_int("WORLD_SIZE", 1), local = env_int("LOCAL_RANK", rank);
     const std::string table = arg(argc, argv, "--table", "smoke");
-    const bool fresh = flag(argc, argv, "--fresh");      // a new payload per trial (TX on the GPU inside the batch) wherever the waveform allows it
+    const bool fresh = flag(argc, argv, "--fresh");      // a new payload per trial in every mode (TX, chirp pair and tuning error on the GPU inside the batch)
     const std::string manifest = arg(argc, argv, "--manifest", "");
     const std::string out_path = arg(argc, argv, "--out", "");
     const std::string rdv = arg(argc, argv, "--rendezvous", manifest.empty() ? "/tmp" : manifest.c_str());
@@ -204,8 +204,7 @@ int main(int argc, char** argv) {
 
     std::vector<pu_sweep_mode> modes = make_table(table, fast);
     if (fresh)
-        for (auto& m : modes)
-            if (m.waveform != PU_WF_OFDM_CHIRP && m.waveform != PU_WF_MCDPSK_CHIRP && m.cfo_hz == 0.0f) m.fresh_payloads = 1;
+        for (auto& m : modes) m.fresh_payloads = 1;
     pu_sweep_desc d{};
     d.modes = modes.data();
     d.n_modes = static_cast<uint32_t>(modes.size());
