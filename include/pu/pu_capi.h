@@ -204,10 +204,21 @@ PU_API pu_status pu_chirp_phase_cycles(uint64_t cycles[8]);
  * (src/ofdm/modulator.cpp:348-580) for B payloads at once; peak > 0 rescales every frame to that peak amplitude as the
  * tools do (tools/test_mode_snr.cpp:52-56).  `code` supplies the code rate (its tables double as the encoder's).
  * out[B][out_stride] receives *frame_len samples per row; call with B = 0 to query *frame_len.  Waveforms are
- * bit-identical to pu_ldpc_encode + pu_ofdm_tx. */
+ * bit-identical to pu_ldpc_encode + pu_ofdm_tx.  PU_MEM_HOST leaves each row's samples beyond *frame_len as they were. */
 PU_API pu_status pu_ofdm_tx_batch(pu_ofdm* h, const pu_ldpc* code, const uint8_t* payload, size_t payload_stride,
                                   size_t payload_bytes, size_t B, int layout, float peak, float* out, size_t out_stride,
                                   size_t* frame_len, pu_memspace space, void* stream);
+/* Multi-codeword frames (SURVEY 8f next-4): v2::encodeFrameWithLDPC (src/protocol/frame_v2.cpp:1079-1127: CW0 = the first
+ * bytes_per_codeword frame bytes, CW1+ = {0xD5, index, next bytes_per_codeword - 2 bytes}, zero padded, each LDPC-encoded at the rate
+ * of `code`) + OFDMModulator::generateTrainingSymbols(2) (layout 0) / generatePreamble() (layout 1) + modulate() over all
+ * n_codewords x 648 coded bits back to back (src/ofdm/modulator.cpp:348-580: differential state carried across codewords, the last
+ * symbol filled as far as the bits go), for B frames of frame_bytes bytes each (row b at frames + b * frame_stride).  peak > 0
+ * rescales each frame as pu_ofdm_tx_batch does.  B = 0 queries *frame_len and *n_codewords (1..255; more is PU_ERR_INVALID).
+ * Bit-identical to pu_frame_encode + pu_ofdm_tx(layout); pu_ofdm_tx_batch is its one-codeword case.  One CTA per frame, the coded
+ * bits in shared memory (255 codewords: 20.7 KB). */
+PU_API pu_status pu_frame_tx_batch(pu_ofdm* h, const pu_ldpc* code, const uint8_t* frames, size_t frame_stride, size_t frame_bytes,
+                                   size_t B, int layout, float peak, float* out, size_t out_stride, size_t* frame_len,
+                                   size_t* n_codewords, pu_memspace space, void* stream);
 
 /* ---------------------------------------------------------------- OFDM acquisition (Schmidl-Cox path, SURVEY 8f next-1)
  * Replaces the SEARCHING state of ultra::OFDMDemodulator::process (src/ofdm/demodulator.cpp:474-600) with
@@ -479,6 +490,14 @@ typedef struct {
                                  * payload is a pure function of (base_seed, mode, SNR index, trial).  Each row is built in the pool's order: body
                                  * behind the lead silence and the chirp pair, peak normalisation over chirp and body, cfo_hz through
                                  * pu_tools_cfo_apply_batch over the whole row, then the row's noise level. */
+    uint32_t frame_payload_bytes; /* > 0: every trial is a protocol-v2 DATA frame with this many payload bytes (several codewords in one
+                                 * OFDM frame; PU_WF_OFDM, PU_WF_OFDM_SC and PU_WF_OFDM_CHIRP only, at most 65535 bytes and 255 codewords)
+                                 * and the counters of its SNR points are whole-frame counters {frames, frame_errors, codewords_failed,
+                                 * codewords sent, header_failures, 0}: a frame is lost unless RxPipeline::decodeFrame (rx_pipeline.cpp:
+                                 * 348-445) returns exactly the frame sent.  The frame is DataFrame::serialize of {type 0x30, flags 0x01,
+                                 * src 0x123456, dst 0xABCDEF}: pool waveform i carries pu_sweep_payload(base_seed, mode, i) with seq i + 1,
+                                 * a fresh frame the fresh payload bytes with seq = trial & 0xFFFF.  Acquired frames deliver
+                                 * min(n_cw, soft bits / 648) codewords to the decoder.  payload_bytes is unused (0 allowed); 0 = codeword mode */
 } pu_sweep_mode;
 
 typedef struct {
@@ -519,7 +538,8 @@ PU_API pu_status pu_sweep_unit(const pu_sweep_desc* d, uint64_t u, uint32_t* mod
 /* payload bytes of TX waveform `index` of mode `mode` (splitmix64 stream; lets any host regenerate the pool) */
 PU_API void pu_sweep_payload(uint64_t base_seed, uint32_t mode, uint32_t index, uint8_t* out, size_t n_bytes);
 /* counters[pu_sweep_point_count][6] (HOST, uint64) = this rank's {frames, frame_errors, bit_errors, payload_bits, decode_failures,
- * iteration_sum} per (mode, SNR point), rank 0 additionally holding the resumed units; stats may be NULL. */
+ * iteration_sum} per (mode, SNR point) -- whole-frame counters for frame modes (pu_sweep_mode.frame_payload_bytes) --, rank 0
+ * additionally holding the resumed units; stats may be NULL. */
 PU_API pu_status pu_linksim_run(pu_ctx* ctx, const pu_sweep_desc* d, uint64_t* counters, pu_sweep_stats* stats);
 /* Sum n uint64 counters over the ranks of an NCCL communicator (ncclComm_t passed as void*; libnccl is resolved at run time with
  * dlopen, the library does not link it).  PU_MEM_HOST stages through the context; comm == NULL is a no-op (single rank). */

@@ -468,6 +468,33 @@ class OfdmDemodulator:
                                      C.c_float(peak), _ptr(out), C.c_size_t(ostride), C.byref(n), sp, _stream(sp)))
         return out
 
+    def frame_tx_batch(self, ldpc, frames, layout=0, peak=0.0, out=None):
+        """pu_frame_tx_batch: frames [B, frame_bytes] uint8 (numpy or torch.cuda) -> waveforms [B, L] float32: v2::encodeFrameWithLDPC at the
+        rate of `ldpc` + training symbols / Schmidl-Cox preamble + every codeword modulated back to back, optionally rescaled to `peak`.
+        `out` may be wider than L (its padding is left as it is).  Returns (out, n_codewords)."""
+        tor = _is_torch(frames)
+        B, nbytes = frames.shape
+        L, ncw = C.c_size_t(0), C.c_size_t(0)
+        check(lib().pu_frame_tx_batch(self._h, ldpc._h, None, C.c_size_t(nbytes), C.c_size_t(nbytes), C.c_size_t(0), int(layout), C.c_float(0.0),
+                                      None, C.c_size_t(0), C.byref(L), C.byref(ncw), 0, None))
+        if tor:
+            import torch
+            assert frames.dtype == torch.uint8 and frames.dim() == 2 and frames.stride(1) == 1
+            stride = frames.stride(0)
+            if out is None:
+                out = torch.empty((B, L.value), dtype=torch.float32, device=frames.device)
+        else:
+            frames = np.ascontiguousarray(frames, dtype=np.uint8)
+            stride = frames.shape[1]
+            if out is None:
+                out = np.zeros((B, L.value), np.float32)
+        assert out.shape[0] == B and out.shape[1] >= L.value
+        sp = _space(frames, out)
+        ostride = out.stride(0) if tor else out.strides[0] // 4
+        check(lib().pu_frame_tx_batch(self._h, ldpc._h, _ptr(frames), C.c_size_t(stride), C.c_size_t(nbytes), C.c_size_t(B), int(layout),
+                                      C.c_float(peak), _ptr(out), C.c_size_t(ostride), C.byref(L), C.byref(ncw), sp, _stream(sp)))
+        return out, int(ncw.value)
+
     def chirp_receive_batch(self, samples, threshold=0.15, llr_stride=648, want_llr=True):
         """pu_ofdm_chirp_receive_batch: dual-chirp detectSync + setFrequencyOffset + process + getSoftBits for every row of
         samples [B, L] -> (llr [B, llr_stride], n_llr [B], sync_info [B, 4] int32, sync_values [B, 4] float32, snr_db [B])."""
@@ -817,7 +844,7 @@ class SweepMode(C.Structure):
                 ("code_rate", C.c_uint32), ("payload_bytes", C.c_uint32), ("channel", C.c_uint32), ("n_snr", C.c_uint32),
                 ("snr_first_db", C.c_float), ("snr_step_db", C.c_float), ("peak", C.c_float), ("precision", C.c_uint32),
                 ("chunk", C.c_uint32), ("cost", C.c_float), ("lead_samples", C.c_uint32), ("tail_samples", C.c_uint32),
-                ("cfo_hz", C.c_float), ("fresh_payloads", C.c_uint32)]
+                ("cfo_hz", C.c_float), ("fresh_payloads", C.c_uint32), ("frame_payload_bytes", C.c_uint32)]
 
     @property
     def snr_points(self):
@@ -838,7 +865,9 @@ class SweepStats(C.Structure):
 
 
 def sweep_mode(waveform, cfg, code_rate, payload_bytes, channel, snr_first, snr_step, n_snr, peak=0.0, precision="exact", chunk=0, cost=0.0,
-               lead_samples=0, tail_samples=0, cfo_hz=0.0, fresh_payloads=False):
+               lead_samples=0, tail_samples=0, cfo_hz=0.0, fresh_payloads=False, frame_payload_bytes=0):
+    """One pu_sweep_mode.  frame_payload_bytes > 0 makes every trial a protocol-v2 DATA frame of that many payload bytes (OFDM waveforms;
+    payload_bytes is then unused) with whole-frame counters (linksim.FRAME_COUNTER_NAMES)."""
     m = SweepMode()
     m.waveform = waveform
     if isinstance(cfg, ModemConfig):
@@ -851,6 +880,7 @@ def sweep_mode(waveform, cfg, code_rate, payload_bytes, channel, snr_first, snr_
     m.snr_first_db, m.snr_step_db, m.peak = float(snr_first), float(snr_step), float(peak or 0.0)
     m.precision, m.chunk, m.cost = {"exact": 0, "fast": 1}[precision], int(chunk), float(cost)
     m.lead_samples, m.tail_samples, m.cfo_hz, m.fresh_payloads = int(lead_samples), int(tail_samples), float(cfo_hz), int(bool(fresh_payloads))
+    m.frame_payload_bytes = int(frame_payload_bytes)
     return m
 
 
@@ -885,7 +915,9 @@ class Sweep:
         return m.value, s.value, t0.value, nt.value
 
     def payload(self, mode, index):
-        out = np.zeros(self.modes[mode].payload_bytes, np.uint8)
+        """Payload of TX pool waveform `index` of mode `mode` (the DATA frame's payload in frame modes)."""
+        m = self.modes[mode]
+        out = np.zeros(m.frame_payload_bytes or m.payload_bytes, np.uint8)
         lib().pu_sweep_payload(C.c_uint64(self.desc.base_seed), C.c_uint32(mode), C.c_uint32(index), _ptr(out), C.c_size_t(len(out)))
         return out
 

@@ -10,40 +10,24 @@
 #include <cstring>
 #include <vector>
 
+#include "frame_v2.cuh"
 #include "pu_internal.h"
 
 namespace pu {
 
-__host__ __device__ inline uint16_t frame_crc16(const uint8_t* d, int len) {   // ControlFrame::calculateCRC, frame_v2.cpp:111-124
-    uint16_t crc = 0xFFFF;
-    for (int i = 0; i < len; ++i) {
-        crc ^= static_cast<uint16_t>(static_cast<uint16_t>(d[i]) << 8);
-        for (int j = 0; j < 8; ++j) crc = (crc & 0x8000) ? static_cast<uint16_t>((crc << 1) ^ 0x1021) : static_cast<uint16_t>(crc << 1);
-    }
-    return crc;
-}
-
-inline int frame_bytes_per_codeword(int rate) {   // getBytesPerCodeword, frame_v2.hpp:551-566
-    switch (rate) {
-        case PU_RATE_1_4: return 162 / 8;
-        case PU_RATE_1_3: return 216 / 8;
-        case PU_RATE_1_2: return 324 / 8;
-        case PU_RATE_2_3: return 432 / 8;
-        case PU_RATE_3_4: return 486 / 8;
-        case PU_RATE_5_6: return 540 / 8;
-        default: return 162 / 8;
-    }
-}
-
-// info[b] = {success, frame_type, codewords_ok, codewords_failed, expected codewords}; frame_len[b] = bytes written to frame_out[b]
+// info[b] = {success, frame_type, codewords_ok, codewords_failed, expected codewords}; frame_len[b] = bytes written to frame_out[b].
+// Frame b owns ncw_stride codewords; it has ncw_b = ncw_per ? ncw_per[b] : ncw_stride of them (the soft bits an acquiring receiver
+// delivered): codewords beyond ncw_b are never looked at.
 __global__ void __launch_bounds__(128) frame_assemble_kernel(const uint8_t* __restrict__ cw_bytes, size_t cw_stride, const uint8_t* __restrict__ cw_ok,
-                                                             int B, int ncw, int bpc, int kbytes, uint8_t* __restrict__ frame_out,
-                                                             size_t frame_cap, int32_t* __restrict__ frame_len, int32_t* __restrict__ info) {
+                                                             int B, int ncw_stride, const int32_t* __restrict__ ncw_per, int bpc, int kbytes,
+                                                             uint8_t* __restrict__ frame_out, size_t frame_cap, int32_t* __restrict__ frame_len,
+                                                             int32_t* __restrict__ info) {
     const int lane = threadIdx.x & 31;
     const int b = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     if (b >= B) return;
-    const uint8_t* cw = cw_bytes + static_cast<size_t>(b) * ncw * cw_stride;
-    const uint8_t* ok = cw_ok + static_cast<size_t>(b) * ncw;
+    const uint8_t* cw = cw_bytes + static_cast<size_t>(b) * ncw_stride * cw_stride;
+    const uint8_t* ok = cw_ok + static_cast<size_t>(b) * ncw_stride;
+    const int ncw = ncw_per ? min(ncw_per[b], ncw_stride) : ncw_stride;
     int success = 0, type = 0, n_ok = 0, n_fail = 0, expected = 0, out_len = 0;
     do {
         if (ncw < 1) break;                                              // soft_bits.size() < LDPC_BLOCK (:352-354)
@@ -105,6 +89,22 @@ __global__ void __launch_bounds__(128) frame_assemble_kernel(const uint8_t* __re
     }
 }
 
+pu_status frame_decode_enqueue(pu_ctx* ctx, pu_ldpc* dec, const float* llr, size_t B, int num_codewords, const int32_t* ncw_per,
+                               uint8_t* cw_bytes, uint8_t* cw_ok, int32_t* cw_iters, uint8_t* frame_out, size_t frame_cap, int32_t* frame_len,
+                               int32_t* info, cudaStream_t st) {
+    const int kbytes = (pu_ldpc_info_bits(dec) + 7) / 8, bpc = frame_bytes_per_codeword(pu_ldpc_rate(dec));
+    const pu_status s = pu_ldpc_decode_batch(dec, llr, PU_LDPC_N, B * static_cast<size_t>(num_codewords), cw_bytes, static_cast<size_t>(kbytes),
+                                             cw_ok, cw_iters, PU_MEM_DEVICE, st);
+    if (s != PU_OK) return s;
+    const int warps = 4;
+    (void)cudaGetLastError();
+    frame_assemble_kernel<<<static_cast<unsigned>((B + warps - 1) / warps), warps * 32, 0, st>>>(
+        cw_bytes, static_cast<size_t>(kbytes), cw_ok, static_cast<int>(B), num_codewords, ncw_per, bpc, kbytes, frame_out, frame_cap, frame_len, info);
+    ctx->launches.fetch_add(1);
+    PU_CUDA_TRY(cudaGetLastError());
+    return PU_OK;
+}
+
 }  // namespace pu
 
 extern "C" {
@@ -117,7 +117,7 @@ pu_status pu_frame_decode_batch(pu_ctx* ctx, pu_ldpc* dec, const float* llr, siz
     PU_REQUIRE(num_codewords >= 1 && num_codewords <= 255 && frame_cap > 0 && B * num_codewords < (1u << 30), "pu_frame_decode_batch: bad size");
     PU_CUDA_TRY(cudaSetDevice(ctx->device));
     cudaStream_t st = pu::pick_stream(ctx, stream, space);
-    const int rate = pu_ldpc_rate(dec), kbytes = (pu_ldpc_info_bits(dec) + 7) / 8, bpc = pu::frame_bytes_per_codeword(rate);
+    const int kbytes = (pu_ldpc_info_bits(dec) + 7) / 8;
     const size_t ncw = B * num_codewords;
     // grow-only scratch on the context (the calling convention is one thread per context, as for the reference's objects)
     pu_status s;
@@ -139,18 +139,9 @@ pu_status pu_frame_decode_batch(pu_ctx* ctx, pu_ldpc* dec, const float* llr, siz
     if ((s = ctx->f_bytes.reserve(ncw * static_cast<size_t>(kbytes))) != PU_OK) return s;
     if ((s = ctx->f_ok.reserve(ncw)) != PU_OK) return s;
     if ((s = ctx->f_iters.reserve(ncw * sizeof(int32_t))) != PU_OK) return s;
-    uint8_t* d_bytes = static_cast<uint8_t*>(ctx->f_bytes.ptr);
-    uint8_t* d_ok = static_cast<uint8_t*>(ctx->f_ok.ptr);
-    s = pu_ldpc_decode_batch(dec, d_llr, PU_LDPC_N, ncw, d_bytes, static_cast<size_t>(kbytes), d_ok, static_cast<int32_t*>(ctx->f_iters.ptr),
-                             PU_MEM_DEVICE, st);
+    s = pu::frame_decode_enqueue(ctx, dec, d_llr, B, static_cast<int>(num_codewords), nullptr, static_cast<uint8_t*>(ctx->f_bytes.ptr),
+                                 static_cast<uint8_t*>(ctx->f_ok.ptr), static_cast<int32_t*>(ctx->f_iters.ptr), d_out, frame_cap, d_len, d_info, st);
     if (s != PU_OK) return s;
-    const int warps = 4;
-    (void)cudaGetLastError();
-    pu::frame_assemble_kernel<<<static_cast<unsigned>((B + warps - 1) / warps), warps * 32, 0, st>>>(
-        d_bytes, static_cast<size_t>(kbytes), d_ok, static_cast<int>(B),
-        static_cast<int>(num_codewords), bpc, kbytes, d_out, frame_cap, d_len, d_info);
-    ctx->launches.fetch_add(1);
-    PU_CUDA_TRY(cudaGetLastError());
     if (space == PU_MEM_HOST) {
         PU_CUDA_TRY(cudaMemcpyAsync(frame_out, d_out, B * frame_cap, cudaMemcpyDeviceToHost, st));
         PU_CUDA_TRY(cudaMemcpyAsync(frame_len, d_len, B * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
@@ -165,7 +156,7 @@ pu_status pu_frame_decode_batch(pu_ctx* ctx, pu_ldpc* dec, const float* llr, siz
 pu_status pu_frame_encode(int code_rate, const uint8_t* frame, size_t n_bytes, uint8_t* out, size_t out_cap, size_t* n_codewords) {
     PU_REQUIRE(n_codewords && (frame || n_bytes == 0), "pu_frame_encode: NULL argument");
     const size_t bpc = static_cast<size_t>(pu::frame_bytes_per_codeword(code_rate)), pay = bpc - 2;
-    const size_t ncw = n_bytes <= bpc ? 1 : 1 + (n_bytes - bpc + pay - 1) / pay;
+    const size_t ncw = pu::frame_codewords(code_rate, n_bytes);
     *n_codewords = ncw;
     if (!out) return PU_OK;
     PU_REQUIRE(out_cap >= ncw * 81, "pu_frame_encode: output buffer too small");

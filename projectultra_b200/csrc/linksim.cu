@@ -61,6 +61,48 @@ __global__ void __launch_bounds__(1024) count_errors_kernel(const uint8_t* __res
         if (local[i]) atomicAdd(&counters[i], local[i]);
 }
 
+// Whole-frame rule (linksim.FrameLinkSim): a trial succeeds iff decodeFrame succeeded, the reassembled frame has the length of the frame
+// sent and the same bytes.  One warp per frame; counters[bin][6] = {frames, frame_errors, codewords_failed, codewords, header_failures, 0}.
+__global__ void __launch_bounds__(256) count_frame_errors_kernel(const uint8_t* __restrict__ frame_out, size_t frame_cap,
+                                                                 const int32_t* __restrict__ frame_len, const int32_t* __restrict__ info,
+                                                                 const uint8_t* __restrict__ sent, size_t sent_stride,
+                                                                 const uint32_t* __restrict__ tx_index, const uint32_t* __restrict__ bin,
+                                                                 int sent_len, int n_cw, size_t B, unsigned long long* __restrict__ counters) {
+    const int lane = threadIdx.x & 31;
+    const size_t b = blockIdx.x * static_cast<size_t>(blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (b >= B) return;
+    const int32_t* in = info + b * 5;
+    bool good = in[0] == 1 && frame_len[b] == sent_len;
+    if (good) {
+        const uint8_t* got = frame_out + b * frame_cap;
+        const uint8_t* want = sent + static_cast<size_t>(tx_index ? tx_index[b] : 0) * sent_stride;
+        bool same = true;
+        for (int i = lane; i < sent_len; i += 32) same &= got[i] == want[i];
+        good = __all_sync(0xffffffffu, same);
+    }
+    if (lane != 0) return;
+    unsigned long long* c = counters + static_cast<size_t>(bin ? bin[b] : 0) * 6;
+    atomicAdd(&c[0], 1ull);
+    if (!good) atomicAdd(&c[1], 1ull);
+    if (in[3]) atomicAdd(&c[2], static_cast<unsigned long long>(in[3]));
+    atomicAdd(&c[3], static_cast<unsigned long long>(n_cw));
+    if (in[4] == 0) atomicAdd(&c[4], 1ull);
+}
+
+pu_status count_frame_errors(pu_ctx* ctx, const uint8_t* frame_out, size_t frame_cap, const int32_t* frame_len, const int32_t* info,
+                             const uint8_t* sent, size_t sent_stride, const uint32_t* tx_index, const uint32_t* bin, size_t sent_len, int n_cw,
+                             size_t B, uint64_t* counters, cudaStream_t st) {
+    PU_REQUIRE(sent_len <= frame_cap && sent_len <= sent_stride, "count_frame_errors: frame longer than its buffers");
+    if (B == 0) return PU_OK;
+    (void)cudaGetLastError();
+    count_frame_errors_kernel<<<static_cast<unsigned>((B + 7) / 8), 256, 0, st>>>(frame_out, frame_cap, frame_len, info, sent, sent_stride, tx_index,
+                                                                                 bin, static_cast<int>(sent_len), n_cw, B,
+                                                                                 reinterpret_cast<unsigned long long*>(counters));
+    ctx->launches.fetch_add(1);
+    PU_CUDA_TRY(cudaGetLastError());
+    return PU_OK;
+}
+
 }  // namespace pu
 
 extern "C" {

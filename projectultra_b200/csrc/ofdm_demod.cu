@@ -29,6 +29,7 @@
 
 #include "ofdm_plan.h"
 #include "pu_async.cuh"
+#include "frame_v2.cuh"
 #include "pu_internal.h"
 #include "ref_math.cuh"
 #include "ofdm_dev.cuh"
@@ -1001,8 +1002,8 @@ struct TxDev {
     const float* preamble;
     const float2* points;
 };
-cudaError_t ofdm_tx_launch(const TxDev& t, const uint8_t* payload, size_t payload_stride, int payload_bytes, size_t B, float peak, float* out,
-                           size_t out_stride, cudaStream_t st);
+cudaError_t ofdm_tx_launch(const TxDev& t, const uint8_t* frames, size_t frame_stride, int frame_bytes, int n_cw, int bpc, size_t B, float peak,
+                           float* out, size_t out_stride, cudaStream_t st);
 std::vector<float> ofdm_modulate_frame(const OfdmPlan& p, int layout, const uint8_t* data, size_t n_bytes);   // ofdm_tx.cpp
 cfloat ofdm_constellation_point(uint32_t bits, uint32_t mod);
 
@@ -1535,16 +1536,19 @@ pu_status pu_chirp_generate(float sample_rate, float tx_cfo_hz, float* out, size
     return PU_OK;
 }
 
-pu_status pu_ofdm_tx_batch(pu_ofdm* h, const pu_ldpc* code, const uint8_t* payload, size_t payload_stride, size_t payload_bytes, size_t B,
-                           int layout, float peak, float* out, size_t out_stride, size_t* frame_len, pu_memspace space, void* stream) {
-    PU_REQUIRE(h && code && frame_len, "pu_ofdm_tx_batch: NULL argument");
-    PU_REQUIRE(layout == 0 || layout == 1, "pu_ofdm_tx_batch: layout must be 0 (training) or 1 (Schmidl-Cox preamble)");
+}  // extern "C"
+
+namespace pu {
+namespace {
+// The transmitter behind pu_ofdm_tx_batch (n_cw = 1, bpc = k / 8) and pu_frame_tx_batch: B frames of frame_bytes bytes -> n_cw codewords
+// each (bpc frame bytes in CW0) -> one OFDM frame per row.  B == 0 or out == NULL: *frame_len only.
+pu_status ofdm_tx_frames(pu_ofdm* h, const pu_ldpc* code, const uint8_t* frames, size_t frame_stride, size_t frame_bytes, int n_cw, int bpc, size_t B,
+                         int layout, float peak, float* out, size_t out_stride, size_t* frame_len, pu_memspace space, void* stream) {
     const pu::OfdmPlan& p = h->plan;
     pu_ctx* ctx = h->ctx;
     PU_CUDA_TRY(cudaSetDevice(ctx->device));
     pu::TxDev t{};
     pu_ldpc_encoder_view(code, &t.k, &t.m, &t.cn_ninfo, &t.cn_check, &t.cn_var);
-    PU_REQUIRE(payload_bytes * 8 <= static_cast<size_t>(t.k) && payload_bytes <= payload_stride, "pu_ofdm_tx_batch: payload longer than one codeword's information bits");
     pu_status s;
     if (h->tx_pre_len[layout] < 0) {                 // generateTrainingSymbols / generatePreamble: payload independent
         std::vector<float> pre = pu::ofdm_modulate_frame(p, layout, nullptr, 0);
@@ -1566,12 +1570,12 @@ pu_status pu_ofdm_tx_batch(pu_ofdm* h, const pu_ldpc* code, const uint8_t* paylo
         if ((s = h->d_tx_points.upload(pts.data(), pts.size())) != PU_OK) return s;
     }
     const int per_sym = p.n_data * p.bps;
-    t.n_sym = (PU_LDPC_N + per_sym - 1) / per_sym;
+    t.n_sym = (n_cw * PU_LDPC_N + per_sym - 1) / per_sym;
     t.pre_len = h->tx_pre_len[layout];
     t.frame_len = t.pre_len + t.n_sym * p.sym_len;
     *frame_len = static_cast<size_t>(t.frame_len);
     if (B == 0 || !out) return PU_OK;                // length query
-    PU_REQUIRE(payload && out_stride >= static_cast<size_t>(t.frame_len), "pu_ofdm_tx_batch: output rows shorter than a frame");
+    PU_REQUIRE(frames && out_stride >= static_cast<size_t>(t.frame_len), "pu_ofdm_tx_batch: output rows shorter than a frame");
     t.osc_start = layout == 0 ? t.pre_len : 2 * (p.nfft + p.cp);
     if (h->tx_osc_len < static_cast<size_t>(t.frame_len)) {
         std::vector<pu::cfloat> osc = p.nco(static_cast<float>(p.cfg.center_freq) + p.cfg.tx_cfo_hz, static_cast<size_t>(t.frame_len) + 1);
@@ -1587,21 +1591,47 @@ pu_status pu_ofdm_tx_batch(pu_ofdm* h, const pu_ldpc* code, const uint8_t* paylo
     t.points = static_cast<const float2*>(h->d_tx_points.p);
     cudaStream_t st = pu::pick_stream(ctx, stream, space);
     (void)cudaGetLastError();
+    const int fb = static_cast<int>(frame_bytes);
     if (space == PU_MEM_DEVICE) {
-        PU_CUDA_TRY(pu::ofdm_tx_launch(t, payload, payload_stride, static_cast<int>(payload_bytes), B, peak, out, out_stride, st));
+        PU_CUDA_TRY(pu::ofdm_tx_launch(t, frames, frame_stride, fb, n_cw, bpc, B, peak, out, out_stride, st));
         ctx->launches.fetch_add(1);
         return PU_OK;
     }
+    // host memory: stage through the device; the padding of every output row beyond *frame_len comes back as it went in
     pu::DevMem dp, dout;
-    if ((s = dp.upload(payload, B * payload_stride)) != PU_OK) return s;
-    std::vector<float> z(B * out_stride, 0.0f);
-    if ((s = dout.upload(z.data(), z.size())) != PU_OK) return s;
-    PU_CUDA_TRY(pu::ofdm_tx_launch(t, static_cast<const uint8_t*>(dp.p), payload_stride, static_cast<int>(payload_bytes), B, peak,
-                                   static_cast<float*>(dout.p), out_stride, st));
+    if ((s = dp.upload(frames, (B - 1) * frame_stride + frame_bytes)) != PU_OK) return s;
+    if ((s = dout.upload(out, (B - 1) * out_stride + static_cast<size_t>(t.frame_len))) != PU_OK) return s;
+    PU_CUDA_TRY(pu::ofdm_tx_launch(t, static_cast<const uint8_t*>(dp.p), frame_stride, fb, n_cw, bpc, B, peak, static_cast<float*>(dout.p), out_stride, st));
     ctx->launches.fetch_add(1);
     PU_CUDA_TRY(cudaStreamSynchronize(st));
-    PU_CUDA_TRY(cudaMemcpy(out, dout.p, B * out_stride * sizeof(float), cudaMemcpyDeviceToHost));
+    PU_CUDA_TRY(cudaMemcpy(out, dout.p, ((B - 1) * out_stride + static_cast<size_t>(t.frame_len)) * sizeof(float), cudaMemcpyDeviceToHost));
     return PU_OK;
+}
+}  // namespace
+}  // namespace pu
+
+extern "C" {
+
+pu_status pu_ofdm_tx_batch(pu_ofdm* h, const pu_ldpc* code, const uint8_t* payload, size_t payload_stride, size_t payload_bytes, size_t B,
+                           int layout, float peak, float* out, size_t out_stride, size_t* frame_len, pu_memspace space, void* stream) {
+    PU_REQUIRE(h && code && frame_len, "pu_ofdm_tx_batch: NULL argument");
+    PU_REQUIRE(layout == 0 || layout == 1, "pu_ofdm_tx_batch: layout must be 0 (training) or 1 (Schmidl-Cox preamble)");
+    const int k = pu_ldpc_info_bits(code);
+    PU_REQUIRE(payload_bytes * 8 <= static_cast<size_t>(k) && payload_bytes <= payload_stride, "pu_ofdm_tx_batch: payload longer than one codeword's information bits");
+    return pu::ofdm_tx_frames(h, code, payload, payload_stride, payload_bytes, 1, k / 8, B, layout, peak, out, out_stride, frame_len, space, stream);
+}
+
+pu_status pu_frame_tx_batch(pu_ofdm* h, const pu_ldpc* code, const uint8_t* frames, size_t frame_stride, size_t frame_bytes, size_t B, int layout,
+                            float peak, float* out, size_t out_stride, size_t* frame_len, size_t* n_codewords, pu_memspace space, void* stream) {
+    PU_REQUIRE(h && code && frame_len && n_codewords, "pu_frame_tx_batch: NULL argument");
+    PU_REQUIRE(layout == 0 || layout == 1, "pu_frame_tx_batch: layout must be 0 (training) or 1 (Schmidl-Cox preamble)");
+    const int rate = pu_ldpc_rate(code);
+    const uint64_t ncw = pu::frame_codewords(rate, frame_bytes);
+    *n_codewords = static_cast<size_t>(ncw);
+    PU_REQUIRE(ncw <= 255, "pu_frame_tx_batch: frame needs more than 255 codewords");
+    PU_REQUIRE(B == 0 || frame_bytes <= frame_stride, "pu_frame_tx_batch: frame longer than its row");
+    return pu::ofdm_tx_frames(h, code, frames, frame_stride, frame_bytes, static_cast<int>(ncw), pu::frame_bytes_per_codeword(rate), B, layout, peak,
+                              out, out_stride, frame_len, space, stream);
 }
 
 pu_status pu_ofdm_acquire_batch(pu_ofdm* h, const float* samples, size_t B, size_t L, size_t chunk, float sync_threshold,

@@ -1,11 +1,16 @@
-// projectultra_b200/csrc/ofdm_tx_gpu.cu — batched transmitter on the GPU (SURVEY §8f next-3): LDPC encode + OFDM modulate,
-// one frame per CTA, so that every Monte-Carlo frame can carry a fresh random payload like the reference's tools do
-// instead of drawing from a host-built pool of waveforms.
+// projectultra_b200/csrc/ofdm_tx_gpu.cu — batched transmitter on the GPU (SURVEY §8f next-3/next-4): codeword chunking + LDPC
+// encode + OFDM modulate, one frame per CTA, so that every Monte-Carlo frame can carry a fresh random payload like the reference's
+// tools do instead of drawing from a host-built pool of waveforms.  One kernel serves both entry points: pu_ofdm_tx_batch is the
+// one-codeword frame (a payload of at most k / 8 bytes is CW0 of its own zero-padded frame), pu_frame_tx_batch any frame of 1..255
+// codewords modulated back to back.
 //
-// Reference behaviour (bit-identical waveforms; the host twin is csrc/ofdm_tx.cpp + ldpc_code.cpp: ldpc_encode):
+// Reference behaviour (bit-identical waveforms; the host twin is csrc/ofdm_tx.cpp + ldpc_code.cpp: ldpc_encode + frame_v2.cu):
+//   v2::encodeFrameWithLDPC (chunking)                    src/protocol/frame_v2.cpp:1079-1127
 //   LDPCEncoder::encode                                   src/fec/ldpc_encoder.cpp:193-257  (parity_i = XOR of H_data row i)
 //   OFDMModulator::modulate / mapBits                     src/ofdm/modulator.cpp:348-477, :76-106
-//   differential encoding, pilots, IFFT + CP, passband    :393-470 (state carried per carrier over the symbols of a frame)
+//   differential encoding, pilots, IFFT + CP, passband    :393-470 (state carried per carrier over the symbols of a frame, across
+//                                                         codeword boundaries; the last symbol carries the carriers that still
+//                                                         have a first bit, the rest of its carriers stay empty)
 //   generatePreamble / generateTrainingSymbols            :479-580  (payload independent: built once on the host, copied)
 //   peak normalisation of the tools                       tools/test_mode_snr.cpp:52-56
 // The inverse FFT is the reference's radix-2 DIT with conjugated twiddles and 1/N scaling on a shared-memory buffer
@@ -35,31 +40,64 @@ struct TxDev {
     const float2* points;              // [1 << bps] constellation points (coherent) or differential steps
 };
 
+// Shared memory of one CTA: the n_cw * 81 coded bytes packed MSB first (255 codewords: 20.7 KB), then the inverse of the parity
+// placement (parity bit r of a codeword = check p with cn_check[p] == r).
+inline size_t ofdm_tx_smem(int n_cw, int m) { return static_cast<size_t>(n_cw) * (PU_LDPC_N / 8) + static_cast<size_t>(m) * sizeof(uint16_t) + 16; }
+
 template <int NFFT>
-__global__ void __launch_bounds__(128) ofdm_tx_kernel(TxDev t, const uint8_t* __restrict__ payload, size_t payload_stride, int payload_bytes,
-                                                      float peak, float* __restrict__ out, size_t out_stride) {
+__global__ void __launch_bounds__(128) ofdm_tx_kernel(TxDev t, const uint8_t* __restrict__ frames, size_t frame_stride, int frame_bytes, int n_cw,
+                                                      int bpc, float peak, float* __restrict__ out, size_t out_stride) {
     __shared__ float2 buf[NFFT];
-    __shared__ uint8_t bits[PU_LDPC_N];
     __shared__ float red[4];
+    extern __shared__ __align__(16) uint8_t tx_smem[];
+    constexpr int kCwBytes = PU_LDPC_N / 8;               // 648 = 81 bytes exactly: codewords stay byte aligned back to back
+    uint8_t* coded = tx_smem;
+    uint16_t* parity_of = reinterpret_cast<uint16_t*>(tx_smem + ((static_cast<size_t>(n_cw) * kCwBytes + 1) & ~size_t(1)));
     const int tid = threadIdx.x, T = blockDim.x;
-    const uint8_t* pl = payload + static_cast<size_t>(blockIdx.x) * payload_stride;
+    const uint8_t* fr = frames + static_cast<size_t>(blockIdx.x) * frame_stride;
     float* w = out + static_cast<size_t>(blockIdx.x) * out_stride;
 
-    // ---- LDPCEncoder::encode of one block: k information bits (payload, zero padded), then the m parity bits
-    for (int j = tid; j < t.k; j += T) bits[j] = (j < payload_bytes * 8) ? ((pl[j >> 3] >> (7 - (j & 7))) & 1) : 0;
-    __syncthreads();
-    for (int p = tid; p < t.m; p += T) {
-        unsigned acc = 0;
-        const int ninfo = t.cn_ninfo[p];
-        for (int e = 0; e < ninfo; ++e) acc ^= bits[t.cn_var[e * t.m + p]];
-        bits[t.k + t.cn_check[p]] = static_cast<uint8_t>(acc);
+    // ---- v2::encodeFrameWithLDPC chunking: CW0 = frame bytes [0, bpc), CWi = {0xD5, i, bytes [bpc + (i-1)(bpc-2), ...)}, zero padded
+    // to the codeword's k information bits (bpc * 8 <= k; the bits from bpc * 8 to k are zero)
+    for (int j = tid; j < n_cw * bpc; j += T) {
+        const int i = j / bpc, q = j - i * bpc;
+        int src = q;
+        uint8_t v;
+        if (i == 0) v = q < frame_bytes ? fr[q] : 0;
+        else if (q < 2) v = q == 0 ? 0xD5 : static_cast<uint8_t>(i);
+        else { src = bpc + (i - 1) * (bpc - 2) + q - 2; v = src < frame_bytes ? fr[src] : 0; }
+        coded[i * kCwBytes + q] = v;
     }
+    for (int p = tid; p < t.m; p += T) parity_of[t.cn_check[p]] = static_cast<uint16_t>(p);
     for (int i = tid; i < t.pre_len; i += T) w[i] = __ldg(&t.preamble[i]);
     __syncthreads();
+    // ---- LDPCEncoder::encode of every codeword: k information bits, then parity bit r = XOR of H_data row parity_of[r]; one thread per
+    // output byte from byte bpc on (whole bytes, so no two threads write one byte)
+    const int info_bits = bpc * 8;
+    for (int j = tid; j < n_cw * (kCwBytes - bpc); j += T) {
+        const int i = j / (kCwBytes - bpc), q = bpc + (j - i * (kCwBytes - bpc));
+        const uint8_t* cw = coded + i * kCwBytes;
+        unsigned byte = 0;
+        for (int e = 0; e < 8; ++e) {
+            const int bit = q * 8 + e;
+            unsigned acc = 0;
+            if (bit >= t.k) {
+                const int p = parity_of[bit - t.k];
+                const int ninfo = t.cn_ninfo[p];
+                for (int x = 0; x < ninfo; ++x) {
+                    const int v = t.cn_var[x * t.m + p];
+                    if (v < info_bits) acc ^= (cw[v >> 3] >> (7 - (v & 7))) & 1u;
+                }
+            }
+            byte = (byte << 1) | acc;
+        }
+        coded[i * kCwBytes + q] = static_cast<uint8_t>(byte);
+    }
+    __syncthreads();
 
-    const int total_bits = t.k + t.m;                     // 648 = 81 bytes exactly
+    const int total_bits = n_cw * PU_LDPC_N;
     const int per_sym = t.n_data * t.bps;
-    float2 diff = make_float2(1.0f, 0.0f);                // this thread's carrier (tid < n_data), carried over the symbols
+    float2 diff = make_float2(1.0f, 0.0f);                // this thread's carrier (tid < n_data), carried over the symbols of the frame
     float mx = 0.0f;
     if (peak > 0.0f)
         for (int i = tid; i < t.pre_len; i += T) mx = fmaxf(mx, fabsf(__ldg(&t.preamble[i])));
@@ -70,7 +108,10 @@ __global__ void __launch_bounds__(128) ofdm_tx_kernel(TxDev t, const uint8_t* __
             const int b0 = s * per_sym + tid * t.bps;
             if (b0 < total_bits) {                        // a carrier exists while data remains at its first bit (:418-436)
                 unsigned v = 0;
-                for (int b = 0; b < t.bps; ++b) v = (v << 1) | ((b0 + b < total_bits) ? bits[b0 + b] : 0u);
+                for (int b = 0; b < t.bps; ++b) {
+                    const int bit = b0 + b;
+                    v = (v << 1) | ((bit < total_bits) ? ((coded[bit >> 3] >> (7 - (bit & 7))) & 1u) : 0u);
+                }
                 float2 sym = __ldg(&t.points[v]);
                 if (t.differential) {
                     sym = cmul(diff, sym);                // diff_state * step
@@ -104,13 +145,14 @@ __global__ void __launch_bounds__(128) ofdm_tx_kernel(TxDev t, const uint8_t* __
     }
 }
 
-cudaError_t ofdm_tx_launch(const TxDev& t, const uint8_t* payload, size_t payload_stride, int payload_bytes, size_t B, float peak, float* out,
-                           size_t out_stride, cudaStream_t st) {
+cudaError_t ofdm_tx_launch(const TxDev& t, const uint8_t* frames, size_t frame_stride, int frame_bytes, int n_cw, int bpc, size_t B, float peak,
+                           float* out, size_t out_stride, cudaStream_t st) {
     if (B == 0) return cudaSuccess;
+    const size_t smem = ofdm_tx_smem(n_cw, t.m);
     if (t.nfft == 512)
-        ofdm_tx_kernel<512><<<static_cast<unsigned>(B), 128, 0, st>>>(t, payload, payload_stride, payload_bytes, peak, out, out_stride);
+        ofdm_tx_kernel<512><<<static_cast<unsigned>(B), 128, smem, st>>>(t, frames, frame_stride, frame_bytes, n_cw, bpc, peak, out, out_stride);
     else
-        ofdm_tx_kernel<1024><<<static_cast<unsigned>(B), 128, 0, st>>>(t, payload, payload_stride, payload_bytes, peak, out, out_stride);
+        ofdm_tx_kernel<1024><<<static_cast<unsigned>(B), 128, smem, st>>>(t, frames, frame_stride, frame_bytes, n_cw, bpc, peak, out, out_stride);
     return cudaGetLastError();
 }
 

@@ -68,11 +68,12 @@ struct pu_ctx {
     pu::PipeSlot pipe[2];
     cudaEvent_t pipe_ev = nullptr;
     // scratch of pu_linksim_run (sweep.cu), grow-only and reused across calls: [0..6] batch buffers (rx, llr, info, ok, iters, n_llr, sync),
-    // [7 + 4 s .. 10 + 4 s] slot s = {pinned descriptors, device descriptors, device counters, pinned counters}
+    // [7 + 4 s .. 10 + 4 s] slot s = {pinned descriptors, device descriptors, device counters, pinned counters},
+    // [15..17] fresh payloads {TX rows, payload rows, noise levels}, [18..19] frame modes {reassembled frames, frame_len + info + ncw}
     pu::Buffer cfo_mix;            // pu_channel_apply_cfo_batch: (cos, sin)(2 pi 1500 i / fs) per sample index, host libm
     size_t cfo_mix_len = 0;
     uint32_t cfo_mix_fs = 0;
-    pu::Buffer sweep[18];
+    pu::Buffer sweep[20];
     cudaEvent_t sweep_ev[2] = {nullptr, nullptr};
 };
 
@@ -111,6 +112,18 @@ void tools_apply_cfo(float* samples, size_t n, float cfo_hz, float sample_rate);
 // phase recurrence; the device injector (tools_cfo_gpu.cu) uploads the same tables
 void tools_cfo_twiddles(size_t fft_size, std::complex<float>* tw);
 void tools_cfo_rotator(size_t n, float cfo_hz, float sample_rate, std::complex<float>* rot);
+// frame_v2.cu: the body of pu_frame_decode_batch, enqueue only, on caller-owned device scratch: llr[B][num_codewords][648] ->
+// cw_bytes[B * num_codewords][k / 8], cw_ok, cw_iters -> frame_out[B][frame_cap], frame_len[B], info[B][5].  ncw_per[b] (NULL = all
+// num_codewords) is the number of codewords frame b delivered, as RxPipeline::decodeFrame's num_codewords.
+pu_status frame_decode_enqueue(pu_ctx* ctx, pu_ldpc* dec, const float* llr, size_t B, int num_codewords, const int32_t* ncw_per,
+                               uint8_t* cw_bytes, uint8_t* cw_ok, int32_t* cw_iters, uint8_t* frame_out, size_t frame_cap, int32_t* frame_len,
+                               int32_t* info, cudaStream_t st);
+// linksim.cu: whole-frame counters (linksim.FRAME_COUNTER_NAMES) of frames decoded by frame_decode_enqueue against the frames sent
+// (row tx_index[b] of sent[][sent_stride], sent_len bytes each, n_cw codewords): counters[bin[b]][6] += {1, lost, info[3], n_cw,
+// info[4] == 0, 0}
+pu_status count_frame_errors(pu_ctx* ctx, const uint8_t* frame_out, size_t frame_cap, const int32_t* frame_len, const int32_t* info,
+                             const uint8_t* sent, size_t sent_stride, const uint32_t* tx_index, const uint32_t* bin, size_t sent_len, int n_cw,
+                             size_t B, uint64_t* counters, cudaStream_t st);
 float channel_power_sum(const float* tx, size_t L);                                   // channel.cu: the two halves of pu_channel_noise_std
 float channel_noise_std_from_sum(float acc, size_t L, float snr_db, int convention);
 cudaError_t chirp_search_stats(unsigned long long* out);

@@ -6,7 +6,9 @@
 // (tests/regression_matrix.sh:139-243, tools/test_iwaveform.cpp:597-806, tools/test_mode_snr.cpp:40-105); see pu_capi.h for the
 // contract.  Work units (mode, SNR point, seed block) -> ranks by longest-processing-time-first on a cost estimate; a rank runs its
 // units mode by mode in batches that mix SNR points and seed blocks (counter bin = unit), two batches in flight so that descriptor
-// preparation and the manifest append of batch k overlap the kernels of batch k+1.
+// preparation and the manifest append of batch k overlap the kernels of batch k+1.  Frame modes (pu_sweep_mode.frame_payload_bytes) carry
+// a protocol-v2 DATA frame of several codewords per trial (v2::encodeFrameWithLDPC, frame_v2.cpp:1079-1127) and count whole frames as
+// RxPipeline::decodeFrame (rx_pipeline.cpp:348-445) delivers them.
 #include <dlfcn.h>
 #include <sys/stat.h>
 #include <dirent.h>
@@ -23,6 +25,8 @@
 #include <string>
 #include <vector>
 
+#include "frame_v2.cuh"
+#include "ofdm_plan.h"
 #include "pu_internal.h"
 
 namespace pu {
@@ -36,7 +40,27 @@ struct SweepPlan {
     std::vector<uint64_t> unit0;      // first unit id of mode m (size n_modes + 1)
     std::vector<uint32_t> point0;     // first counter row of mode m (size n_modes + 1)
     uint64_t blocks;                  // seed blocks per (mode, SNR point)
+    std::vector<uint32_t> n_cw;       // codewords per trial of mode m (1 in codeword mode)
+    std::vector<double> frame_scale;  // OFDM symbols of a frame of mode m over those of a one-codeword frame (1 in codeword mode)
 };
+
+// frame mode (pu_sweep_mode.frame_payload_bytes): the OFDM waveforms only, DataFrame::serialize's 16-bit length, at most the 255
+// codewords TOTAL_CW can count.  n_cw and the frame's length in OFDM symbols relative to one codeword's (for the partitioner's cost).
+bool frame_mode_shape(const pu_sweep_mode& md, uint32_t* n_cw, double* scale) {
+    *n_cw = 1;
+    *scale = 1.0;
+    if (!md.frame_payload_bytes) return true;
+    if (md.waveform > PU_WF_OFDM_CHIRP || md.frame_payload_bytes > 65535) return false;
+    const uint64_t ncw = frame_codewords(static_cast<int>(md.code_rate), uint64_t(md.frame_payload_bytes) + kV2FrameOverhead);
+    if (ncw > 255) return false;
+    OfdmPlan plan;
+    const char* why = "";
+    if (!make_ofdm_plan(md.ofdm, &plan, &why)) return false;
+    const uint64_t per_sym = static_cast<uint64_t>(plan.n_data) * plan.bps;
+    *n_cw = static_cast<uint32_t>(ncw);
+    *scale = (2.0 + static_cast<double>((ncw * PU_LDPC_N + per_sym - 1) / per_sym)) / (2.0 + static_cast<double>((PU_LDPC_N + per_sym - 1) / per_sym));
+    return true;
+}
 
 bool make_plan(const pu_sweep_desc* d, SweepPlan* p) {
     if (!d || !d->modes || d->n_modes == 0 || d->trials_per_point == 0 || d->world == 0 || d->rank >= d->world) return false;
@@ -52,6 +76,11 @@ bool make_plan(const pu_sweep_desc* d, SweepPlan* p) {
     for (uint32_t m = 0; m < d->n_modes; ++m) {
         const pu_sweep_mode& md = d->modes[m];
         if (md.n_snr == 0 || md.n_snr > 255 || md.waveform > PU_WF_MCDPSK_CHIRP || md.channel > PU_CH_ITU_FLUTTER) return false;
+        uint32_t ncw;
+        double scale;
+        if (!frame_mode_shape(md, &ncw, &scale)) return false;
+        p->n_cw.push_back(ncw);
+        p->frame_scale.push_back(scale);
         p->unit0.push_back(p->unit0.back() + static_cast<uint64_t>(md.n_snr) * p->blocks);
         p->point0.push_back(p->point0.back() + md.n_snr);
     }
@@ -79,11 +108,13 @@ double mode_cost(const pu_sweep_mode& m) {
     }
 }
 // LDPC share: ~50 iterations at the bottom of the grid, ~2 at the top; in units of the demodulator cost of the cheapest mode
-// (0.87 ms LDPC against 0.37 ms demod per 53 248 frames at 17 average iterations: ~0.14 per iteration).
-double unit_cost(const pu_sweep_mode& m, uint32_t snr_index, uint32_t n_trials) {
+// (0.87 ms LDPC against 0.37 ms demod per 53 248 frames at 17 average iterations: ~0.14 per iteration).  A frame-mode trial costs
+// its frame's length in demodulation and n_cw codewords in LDPC.
+double unit_cost(const SweepPlan& p, const pu_sweep_mode& m, uint32_t mode, uint32_t snr_index, uint32_t n_trials) {
     const double f = m.n_snr > 1 ? 1.0 - static_cast<double>(snr_index) / (m.n_snr - 1) : 0.5;
     const double iters = 2.0 + 48.0 * f * f;
-    return n_trials * (mode_cost(m) + 0.14 * iters);
+    const double demod = m.cost > 0 ? m.cost : mode_cost(m) * p.frame_scale[mode];      // a table's own cost is per trial already
+    return n_trials * (demod + 0.14 * iters * p.n_cw[mode]);
 }
 
 void unit_decode(const pu_sweep_desc* d, const SweepPlan& p, uint64_t u, uint32_t* mode, uint32_t* snr, uint64_t* t0, uint32_t* nt) {
@@ -122,16 +153,42 @@ uint64_t desc_key(const pu_sweep_desc* d, const SweepPlan& p) {      // FNV-1a o
 
 // fresh_payloads: byte i of frame b's payload = byte (i & 7) of splitmix64(seed[b] ^ kPayloadStream ^ (i >> 3) * golden ratio); rows are kb bytes,
 // zero past payload_bytes.  The frame seed also drives the channel; the stream constant keeps the two independent.
+__device__ inline uint64_t fresh_payload_word(uint64_t seed, size_t w) {
+    uint64_t z = (seed ^ 0x5041594c4f414421ull) + 0x9e3779b97f4a7c15ull * (w + 1);
+    z = (z ^ (z >> 30)) * 0xbf58476d1ce4e5b9ull;
+    z = (z ^ (z >> 27)) * 0x94d049bb133111ebull;
+    return z ^ (z >> 31);
+}
 __global__ void fresh_payload_kernel(uint8_t* __restrict__ pay, size_t kb, uint32_t payload_bytes, const uint64_t* __restrict__ seed, size_t B) {
     const size_t i = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x;
     const size_t words = (kb + 7) / 8;
     if (i >= B * words) return;
     const size_t b = i / words, w = i - b * words;
-    uint64_t z = (seed[b] ^ 0x5041594c4f414421ull) + 0x9e3779b97f4a7c15ull * (w + 1);
-    z = (z ^ (z >> 30)) * 0xbf58476d1ce4e5b9ull;
-    z = (z ^ (z >> 27)) * 0x94d049bb133111ebull;
-    z ^= z >> 31;
+    const uint64_t z = fresh_payload_word(seed[b], w);
     for (size_t k = 0; k < 8 && 8 * w + k < kb; ++k) pay[b * kb + 8 * w + k] = 8 * w + k < payload_bytes ? static_cast<uint8_t>(z >> (8 * k)) : 0;
+}
+
+// frame modes: row b of frames[B][stride] = the DATA frame around the same payload byte stream (payload_bytes bytes at offset 17), seq =
+// the low 16 bits of the frame seed (= trial & 0xFFFF); one warp per frame, lane 0 serialises header and CRCs
+__global__ void fresh_frame_kernel(uint8_t* __restrict__ frames, size_t stride, uint32_t payload_bytes, int rate, const uint64_t* __restrict__ seed, size_t B) {
+    const int lane = threadIdx.x & 31;
+    const size_t b = blockIdx.x * static_cast<size_t>(blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (b >= B) return;
+    uint8_t* f = frames + b * stride;
+    const uint64_t sd = seed[b];
+    for (size_t w = lane; w < (payload_bytes + 7) / 8; w += 32) {
+        const uint64_t z = fresh_payload_word(sd, w);
+        for (size_t k = 0; k < 8 && 8 * w + k < payload_bytes; ++k) f[kV2DataHeader + 8 * w + k] = static_cast<uint8_t>(z >> (8 * k));
+    }
+    __syncwarp();
+    if (lane == 0) v2_data_frame_in_place(f, static_cast<int>(payload_bytes), rate, static_cast<uint16_t>(sd & 0xFFFF));
+}
+
+// frame modes behind an acquiring receiver: the codewords of frame b that RxPipeline::decodeFrame gets = whole codewords of soft bits
+// (0 without sync); codewords past them are never decoded into the result (an all-zero LLR block would "decode" to zeros)
+__global__ void frame_codewords_kernel(int32_t* __restrict__ ncw, const int32_t* __restrict__ n_llr, int n_cw, size_t B) {
+    const size_t i = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x;
+    if (i < B) ncw[i] = min(n_cw, max(0, n_llr[i]) / PU_LDPC_N);
 }
 
 // fresh payloads behind the chirp pair, one CTA per row: the pair into [lead, lead + chirp_len), then the tools' peak normalisation
@@ -182,6 +239,10 @@ struct ModeEngine {
     size_t chirp_len = 0;                // fresh payloads of the chirp waveforms: the pair in d_chirp, written in front of every body
     Buffer d_chirp;
     pu_tools_cfo* tools_cfo = nullptr;   // fresh payloads with cfo_hz: the tools' injector over every row
+    bool frames = false;                 // pu_sweep_mode.frame_payload_bytes > 0: a protocol-v2 DATA frame per trial
+    uint32_t n_cw = 1;                   // codewords per trial
+    size_t frame_bytes = 0;              // frame modes: bytes of the DATA frame (payload + 19)
+    size_t pay_stride = 0;               // bytes per row of d_payload / the fresh payload rows: kb, or frame_bytes in frame modes
 
     ~ModeEngine() {
         if (ofdm) pu_ofdm_destroy(ofdm);
@@ -206,7 +267,14 @@ struct ModeEngine {
         else if ((s = pu_ldpc_create(c, static_cast<int>(m->code_rate), static_cast<int>(p.max_iter), &ldpc)) != PU_OK) return s;
         const auto t_ldpc = now();
         kb = static_cast<size_t>((pu_ldpc_info_bits(ldpc) + 7) / 8);
-        PU_REQUIRE(m->payload_bytes >= 1 && m->payload_bytes <= kb, "pu_linksim_run: payload_bytes exceeds the code's information bytes");
+        frames = m->frame_payload_bytes != 0;
+        if (frames) {
+            frame_bytes = m->frame_payload_bytes + kV2FrameOverhead;
+            n_cw = static_cast<uint32_t>(frame_codewords(static_cast<int>(m->code_rate), frame_bytes));
+        } else {
+            PU_REQUIRE(m->payload_bytes >= 1 && m->payload_bytes <= kb, "pu_linksim_run: payload_bytes exceeds the code's information bytes");
+        }
+        pay_stride = frames ? frame_bytes : kb;
         const bool is_ofdm = m->waveform <= PU_WF_OFDM_CHIRP, is_dpsk = m->waveform == PU_WF_DPSK || m->waveform == PU_WF_DPSK_ACQ;
         if (is_ofdm) {
             if ((s = pu_ofdm_create(c, &m->ofdm, &ofdm)) != PU_OK) return s;
@@ -246,19 +314,28 @@ struct ModeEngine {
         }
         // TX pool on the host (the reference's modulators run per trial on the CPU too): payload -> LDPC encode -> modulate [-> chirp in front]
         std::vector<std::vector<float>> waves(pool);
-        std::vector<uint8_t> payloads(static_cast<size_t>(pool) * kb, 0);
+        // (frame modes: the payload inside DataFrame::serialize, seq i + 1 -> v2::encodeFrameWithLDPC -> all codewords modulated)
+        std::vector<uint8_t> payloads(static_cast<size_t>(pool) * pay_stride, 0);
+        std::vector<uint8_t> coded(static_cast<size_t>(n_cw) * (PU_LDPC_N / 8));
         for (uint32_t i = 0; i < pool; ++i) {
-            uint8_t* pay = payloads.data() + static_cast<size_t>(i) * kb;
-            pu_sweep_payload(p.base_seed, mode_index, i, pay, m->payload_bytes);
-            uint8_t coded[96];
+            uint8_t* pay = payloads.data() + static_cast<size_t>(i) * pay_stride;
             size_t nc = 0;
-            if ((s = pu_ldpc_encode(static_cast<int>(m->code_rate), pay, m->payload_bytes, coded, sizeof coded, &nc)) != PU_OK) return s;
+            if (frames) {
+                pu_sweep_payload(p.base_seed, mode_index, i, pay + kV2DataHeader, m->frame_payload_bytes);
+                v2_data_frame_in_place(pay, static_cast<int>(m->frame_payload_bytes), static_cast<int>(m->code_rate), static_cast<uint16_t>(i + 1));
+                if ((s = pu_frame_encode(static_cast<int>(m->code_rate), pay, frame_bytes, coded.data(), coded.size(), &nc)) != PU_OK) return s;
+                PU_REQUIRE(nc == n_cw, "pu_linksim_run: frame codeword count differs from the plan");
+                nc *= PU_LDPC_N / 8;
+            } else {
+                pu_sweep_payload(p.base_seed, mode_index, i, pay, m->payload_bytes);
+                if ((s = pu_ldpc_encode(static_cast<int>(m->code_rate), pay, m->payload_bytes, coded.data(), coded.size(), &nc)) != PU_OK) return s;
+            }
             size_t n = 0;
             std::vector<float> w;
             auto tx = [&](float* out, size_t cap, size_t* len) -> pu_status {
-                if (is_ofdm) return pu_ofdm_tx(&m->ofdm, m->waveform == PU_WF_OFDM_SC ? 1 : 0, coded, nc, out, cap, len);
-                if (is_dpsk) return pu_dpsk_tx(&m->dpsk, 0, coded, nc, out, cap, len);
-                return pu_mcdpsk_tx(&m->mcdpsk, coded, nc, out, cap, len);
+                if (is_ofdm) return pu_ofdm_tx(&m->ofdm, m->waveform == PU_WF_OFDM_SC ? 1 : 0, coded.data(), nc, out, cap, len);
+                if (is_dpsk) return pu_dpsk_tx(&m->dpsk, 0, coded.data(), nc, out, cap, len);
+                return pu_mcdpsk_tx(&m->mcdpsk, coded.data(), nc, out, cap, len);
             };
             // every waveform of a mode has the same length: the host modulators are asked for it once (a query runs the whole modulation)
             if (body_len == 0) { tx(nullptr, 0, &n); body_len = n; }
@@ -304,6 +381,11 @@ struct ModeEngine {
         float* at = out ? out + md->lead_samples + chirp_len : nullptr;
         const float peak = chirp_len ? 0.0f : md->peak;
         const unsigned wf = md->waveform;
+        if (frames) {
+            size_t ncw = 0;
+            return pu_frame_tx_batch(ofdm, ldpc, d_pay, pay_stride, frame_bytes, B, wf == PU_WF_OFDM_SC ? 1 : 0, peak, at, row, &body_len, &ncw,
+                                     PU_MEM_DEVICE, st);
+        }
         if (wf == PU_WF_OFDM || wf == PU_WF_OFDM_SC || wf == PU_WF_OFDM_CHIRP)
             return pu_ofdm_tx_batch(ofdm, ldpc, d_pay, kb, md->payload_bytes, B, wf == PU_WF_OFDM_SC ? 1 : 0, peak, at, row, &body_len, PU_MEM_DEVICE, st);
         if (wf == PU_WF_DPSK || wf == PU_WF_DPSK_ACQ)
@@ -320,6 +402,30 @@ struct ModeEngine {
             PU_CUDA_TRY(cudaGetLastError());
         }
         return tools_cfo ? pu_tools_cfo_apply_batch(tools_cfo, out, B, L, PU_MEM_DEVICE, st) : PU_OK;
+    }
+
+    // frame modes: demodulate every codeword of the frame (llr [B][n_cw * 648]) -> decodeFrame (cw_* [B * n_cw] codeword scratch) ->
+    // frame_out [B][frame_bytes], frame_len [B], info [B][5]; ncw [B] = codewords the acquiring receivers delivered
+    pu_status receive_frames(const float* rx, size_t B, float* llr, int32_t* n_llr, int32_t* sync_i, float* sync_f, uint8_t* cw_bytes, uint8_t* cw_ok,
+                             int32_t* cw_iters, uint8_t* frame_out, int32_t* frame_len, int32_t* info, int32_t* ncw, cudaStream_t st) {
+        pu_status s = PU_OK;
+        const size_t stride = static_cast<size_t>(n_cw) * PU_LDPC_N;
+        const unsigned wf = md->waveform;
+        if (wf == PU_WF_OFDM) {
+            if ((s = pu_ofdm_presynced_batch(ofdm, rx, B, L, 2, nullptr, nullptr, llr, stride, nullptr, nullptr, PU_MEM_DEVICE, st)) != PU_OK) return s;
+            ncw = nullptr;
+        } else {
+            PU_CUDA_TRY(cudaMemsetAsync(llr, 0, B * stride * sizeof(float), st));
+            if (wf == PU_WF_OFDM_SC)
+                s = pu_ofdm_process_batch(ofdm, rx, B, L, md->chunk ? md->chunk : 960, 0.0f, llr, stride, n_llr, sync_i, sync_f, nullptr, PU_MEM_DEVICE, st);
+            else
+                s = pu_ofdm_chirp_receive_batch(ofdm, rx, B, L, 0.0f, llr, stride, n_llr, sync_i, sync_f, nullptr, PU_MEM_DEVICE, st);
+            if (s != PU_OK) return s;
+            frame_codewords_kernel<<<static_cast<unsigned>((B + 255) / 256), 256, 0, st>>>(ncw, n_llr, static_cast<int>(n_cw), B);
+            ctx->launches.fetch_add(1);
+            PU_CUDA_TRY(cudaGetLastError());
+        }
+        return frame_decode_enqueue(ctx, ldpc, llr, B, static_cast<int>(n_cw), ncw, cw_bytes, cw_ok, cw_iters, frame_out, frame_bytes, frame_len, info, st);
     }
 
     // demodulate -> decode (device pointers, stream st); scratch: llr [B][648], n_llr [B], sync [B][8] (int/float)
@@ -436,7 +542,7 @@ void partition(const pu_sweep_desc* d, const SweepPlan& p, const uint8_t* done, 
     for (uint64_t u = 0; u < n; ++u) {
         uint32_t m, s, nt; uint64_t t0;
         unit_decode(d, p, u, &m, &s, &t0, &nt);
-        cost[u] = unit_cost(d->modes[m], s, nt);
+        cost[u] = unit_cost(p, d->modes[m], m, s, nt);
         owner[u] = kNoOwner;
         if (!(done && done[u])) order.push_back(u);
     }
@@ -569,7 +675,8 @@ pu_status pu_linksim_run(pu_ctx* ctx, const pu_sweep_desc* d, uint64_t* counters
     // ---- batches in flight
     pu::Slot slots[2];
     pu::Buffer &d_rx = ctx->sweep[0], &d_llr = ctx->sweep[1], &d_info = ctx->sweep[2], &d_ok = ctx->sweep[3], &d_iters = ctx->sweep[4],
-               &d_nllr = ctx->sweep[5], &d_sync = ctx->sweep[6], &d_ftx = ctx->sweep[15], &d_fpay = ctx->sweep[16], &d_fstd = ctx->sweep[17];
+               &d_nllr = ctx->sweep[5], &d_sync = ctx->sweep[6], &d_ftx = ctx->sweep[15], &d_fpay = ctx->sweep[16], &d_fstd = ctx->sweep[17],
+               &d_fout = ctx->sweep[18], &d_finfo = ctx->sweep[19];
     for (int i = 0; i < 2; ++i) {
         pu::Slot& sl = slots[i];
         sl.h_desc = &ctx->sweep[7 + 4 * i]; sl.d_desc = &ctx->sweep[8 + 4 * i]; sl.d_cnt = &ctx->sweep[9 + 4 * i]; sl.h_cnt = &ctx->sweep[10 + 4 * i];
@@ -622,16 +729,20 @@ pu_status pu_linksim_run(pu_ctx* ctx, const pu_sweep_desc* d, uint64_t* counters
         if (std::getenv("PU_SWEEP_TRACE"))
             fprintf(stderr, "[pu_linksim_run] rank %u mode %u waveform %u: engine set-up %.3f s (%zu samples per frame, pool %u)\n", d->rank, m,
                     d->modes[m].waveform, t_build, eng.L, eng.pool);
-        const size_t L = eng.L, kb = eng.kb;
-        // (fresh payloads keep the clean TX batch next to the received one: half as many frames per batch)
-        const size_t max_frames = std::max<size_t>(1, std::min<uint64_t>(p.batch_bytes / (L * sizeof(float) * (eng.fresh ? 2 : 1)), (uint64_t(1) << 22)));
+        const size_t L = eng.L, kb = eng.kb, ncw = eng.n_cw;
+        // (fresh payloads keep the clean TX batch next to the received one: half as many frames per batch; frame modes count their soft bits)
+        const size_t bytes_per_trial = L * sizeof(float) * (eng.fresh ? 2 : 1) + (eng.frames ? ncw * PU_LDPC_N * sizeof(float) : 0);
+        const size_t max_frames = std::max<size_t>(1, std::min<uint64_t>(p.batch_bytes / bytes_per_trial, (uint64_t(1) << 22)));
         const size_t cap = std::max<size_t>(max_frames, p.block);      // a unit is never split: the smallest batch is one unit
-        if ((rs = d_rx.reserve(cap * L * sizeof(float))) != PU_OK || (rs = d_llr.reserve(cap * PU_LDPC_N * sizeof(float))) != PU_OK ||
-            (rs = d_info.reserve(cap * kb)) != PU_OK || (rs = d_ok.reserve(cap)) != PU_OK || (rs = d_iters.reserve(cap * 4)) != PU_OK ||
+        if ((rs = d_rx.reserve(cap * L * sizeof(float))) != PU_OK || (rs = d_llr.reserve(cap * ncw * PU_LDPC_N * sizeof(float))) != PU_OK ||
+            (rs = d_info.reserve(cap * ncw * kb)) != PU_OK || (rs = d_ok.reserve(cap * ncw)) != PU_OK || (rs = d_iters.reserve(cap * ncw * 4)) != PU_OK ||
             (rs = d_nllr.reserve(cap * 4)) != PU_OK || (rs = d_sync.reserve(cap * 12 * 4)) != PU_OK)
             break;
-        if (eng.fresh && ((rs = d_ftx.reserve(cap * L * sizeof(float))) != PU_OK || (rs = d_fpay.reserve(cap * kb)) != PU_OK ||
+        if (eng.fresh && ((rs = d_ftx.reserve(cap * L * sizeof(float))) != PU_OK || (rs = d_fpay.reserve(cap * eng.pay_stride)) != PU_OK ||
                           (rs = d_fstd.reserve(cap * sizeof(float))) != PU_OK))
+            break;
+        // frame modes: reassembled frames; frame_len [cap], info [cap][5], codewords delivered [cap]
+        if (eng.frames && ((rs = d_fout.reserve(cap * eng.frame_bytes)) != PU_OK || (rs = d_finfo.reserve(cap * 7 * sizeof(int32_t))) != PU_OK))
             break;
         size_t next = 0;
         while (next < mine.size() && budget > 0 && rs == PU_OK) {
@@ -694,9 +805,14 @@ pu_status pu_linksim_run(pu_ctx* ctx, const pu_sweep_desc* d, uint64_t* counters
                 if (eng.fresh) {                 // payload -> encode -> modulate for every frame of the batch, then its own noise level
                     uint8_t* pay = static_cast<uint8_t*>(d_fpay.ptr);
                     float* ftx = static_cast<float*>(d_ftx.ptr);
-                    const size_t words = B * ((kb + 7) / 8);
-                    pu::fresh_payload_kernel<<<static_cast<unsigned>((words + 255) / 256), 256, 0, st>>>(pay, kb, d->modes[m].payload_bytes,
-                                                                                                       reinterpret_cast<const uint64_t*>(dd + off_seed), B);
+                    const uint64_t* seeds = reinterpret_cast<const uint64_t*>(dd + off_seed);
+                    if (eng.frames) {
+                        pu::fresh_frame_kernel<<<static_cast<unsigned>((B + 7) / 8), 256, 0, st>>>(pay, eng.pay_stride, d->modes[m].frame_payload_bytes,
+                                                                                                   static_cast<int>(d->modes[m].code_rate), seeds, B);
+                    } else {
+                        const size_t words = B * ((kb + 7) / 8);
+                        pu::fresh_payload_kernel<<<static_cast<unsigned>((words + 255) / 256), 256, 0, st>>>(pay, kb, d->modes[m].payload_bytes, seeds, B);
+                    }
                     ctx->launches.fetch_add(1);
                     PU_CUDA_TRY(cudaGetLastError());
                     if (d->modes[m].lead_samples || d->modes[m].tail_samples) PU_CUDA_TRY(cudaMemsetAsync(ftx, 0, B * L * sizeof(float), st));
@@ -711,11 +827,25 @@ pu_status pu_linksim_run(pu_ctx* ctx, const pu_sweep_desc* d, uint64_t* counters
                 uint8_t* info = static_cast<uint8_t*>(d_info.ptr);
                 uint8_t* ok = static_cast<uint8_t*>(d_ok.ptr);
                 int32_t* iters = static_cast<int32_t*>(d_iters.ptr);
-                s2 = eng.receive(rx, B, static_cast<float*>(d_llr.ptr), static_cast<int32_t*>(d_nllr.ptr), static_cast<int32_t*>(d_sync.ptr),
-                                 reinterpret_cast<float*>(static_cast<int32_t*>(d_sync.ptr) + 4 * cap), info, ok, iters, st);
-                if (s2 != PU_OK) return s2;
-                s2 = pu_count_errors(ctx, info, kb, ok, iters, payloads, kb, reinterpret_cast<const uint32_t*>(dd),
-                                     reinterpret_cast<const uint32_t*>(dd + off_bin), d->modes[m].payload_bytes, B, static_cast<uint64_t*>(sl.d_cnt->ptr), st);
+                const uint32_t* tx_index = reinterpret_cast<const uint32_t*>(dd);
+                const uint32_t* bins = reinterpret_cast<const uint32_t*>(dd + off_bin);
+                uint64_t* cnt = static_cast<uint64_t*>(sl.d_cnt->ptr);
+                if (eng.frames) {
+                    uint8_t* fout = static_cast<uint8_t*>(d_fout.ptr);
+                    int32_t* flen = static_cast<int32_t*>(d_finfo.ptr);
+                    int32_t* finfo = flen + cap;
+                    s2 = eng.receive_frames(rx, B, static_cast<float*>(d_llr.ptr), static_cast<int32_t*>(d_nllr.ptr), static_cast<int32_t*>(d_sync.ptr),
+                                            reinterpret_cast<float*>(static_cast<int32_t*>(d_sync.ptr) + 4 * cap), info, ok, iters, fout, flen, finfo,
+                                            finfo + 5 * cap, st);
+                    if (s2 != PU_OK) return s2;
+                    s2 = pu::count_frame_errors(ctx, fout, eng.frame_bytes, flen, finfo, payloads, eng.pay_stride, tx_index, bins, eng.frame_bytes,
+                                                static_cast<int>(ncw), B, cnt, st);
+                } else {
+                    s2 = eng.receive(rx, B, static_cast<float*>(d_llr.ptr), static_cast<int32_t*>(d_nllr.ptr), static_cast<int32_t*>(d_sync.ptr),
+                                     reinterpret_cast<float*>(static_cast<int32_t*>(d_sync.ptr) + 4 * cap), info, ok, iters, st);
+                    if (s2 != PU_OK) return s2;
+                    s2 = pu_count_errors(ctx, info, kb, ok, iters, payloads, kb, tx_index, bins, d->modes[m].payload_bytes, B, cnt, st);
+                }
                 if (s2 != PU_OK) return s2;
                 PU_CUDA_TRY(cudaMemcpyAsync(sl.h_cnt->ptr, sl.d_cnt->ptr, nu * 6 * 8, cudaMemcpyDeviceToHost, st));
                 PU_CUDA_TRY(cudaEventRecord(sl.ev, st));

@@ -421,9 +421,11 @@ class FrameLinkSim:
         v2_data_frame -> pu_frame_encode -> pu_ofdm_tx (pool, host)  |  pu_channel_apply_batch -> pu_ofdm_presynced_batch (all
         codewords of the frame, llr_stride = n_cw * 648) -> pu_frame_decode_batch -> compare with the frame sent -> counters
 
-    counters [n_snr, 6] = FRAME_COUNTER_NAMES."""
+    counters [n_snr, 6] = FRAME_COUNTER_NAMES.  payloads: explicit [pool, payload_bytes] array (e.g. the sweep driver's pool,
+    capi.Sweep.payload; frame i then carries seq i + 1 as there); peak: the tools' peak normalisation of every TX waveform."""
 
-    def __init__(self, ctx, cfg, channel="awgn", payload_bytes=200, pool=16, pool_seed=12345, max_iter=50, precision="exact", code_rate=None):
+    def __init__(self, ctx, cfg, channel="awgn", payload_bytes=200, pool=16, pool_seed=12345, max_iter=50, precision="exact", code_rate=None,
+                 payloads=None, peak=None):
         import torch
         assert isinstance(cfg, capi.ModemConfig), "whole frames ride on the OFDM waveforms"
         self.ctx, self.cfg = ctx, cfg
@@ -434,12 +436,19 @@ class FrameLinkSim:
         self.ofdm = capi.OfdmDemodulator(ctx, cfg)
         self.ofdm.set_precision(precision)
         self.ldpc = capi.LdpcDecoder(ctx, self.rate, max_iter)
-        rng = np.random.default_rng(pool_seed)
-        self.frames_host = [v2_data_frame(rng.integers(0, 256, payload_bytes, dtype=np.uint8), self.rate, seq=i + 1) for i in range(pool)]
+        if payloads is None:
+            rng = np.random.default_rng(pool_seed)
+            payloads = [rng.integers(0, 256, payload_bytes, dtype=np.uint8) for _ in range(pool)]
+        else:
+            payloads = np.ascontiguousarray(payloads, dtype=np.uint8).reshape(pool, payload_bytes)
+        self.frames_host = [v2_data_frame(payloads[i], self.rate, seq=i + 1) for i in range(pool)]
         cws = [capi.frame_encode(self.rate, f) for f in self.frames_host]
         self.n_cw = len(cws[0])
         assert all(len(c) == self.n_cw for c in cws)
-        self.tx_host = np.stack([ofdm_tx(cfg, c.reshape(-1), 0) for c in cws])
+        waves = [ofdm_tx(cfg, c.reshape(-1), 0) for c in cws]
+        if peak is not None:
+            waves = [(w * (np.float32(peak) / np.abs(w).max())).astype(np.float32) for w in waves]
+        self.tx_host = np.stack(waves)
         self.L = self.tx_host.shape[1]
         assert self.ofdm.n_llr(self.L) >= self.n_cw * 648
         self.tx_pool = torch.from_numpy(self.tx_host).to(self.device)

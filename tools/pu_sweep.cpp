@@ -4,8 +4,9 @@
 // SNR, CFO) matrix of tests/regression_matrix.sh:139-243 over the trial loop of tools/test_iwaveform.cpp:597-806.
 //
 //   torchrun-style launch (RANK / WORLD_SIZE / LOCAL_RANK in the environment), or a single process:
-//     projectultra_b200/pu_sweep --table reduced --trials 16384 [--block 2048] [--manifest DIR] [--out rows.jsonl] [--fresh]
-//   tables: smoke (4 modes, seconds), reduced (one mode per waveform family and channel + the chirp-acquired CFO rows of the regression matrix), config5 (105 modes x 40 SNR points)
+//     projectultra_b200/pu_sweep --table reduced --trials 16384 [--block 2048] [--manifest DIR] [--out rows.jsonl] [--fresh] [--frame-bytes N]
+//   tables: smoke (4 modes, seconds), reduced (one mode per waveform family and channel + the chirp-acquired CFO rows of the regression matrix), config5 (105 modes x 40 SNR points),
+//   frames (whole-frame FER of protocol-v2 DATA frames of 200 and 1000 payload bytes, or N with --frame-bytes, over AWGN / good / poor)
 //
 // Rank 0 prints one JSON object per (mode, SNR point) with the Wilson 95 % interval of the FER, then one summary line with the
 // per-rank run times (scaling efficiency = mean / max of the ranks' times: ranks never wait for each other before the final sum).
@@ -91,9 +92,24 @@ pu_sweep_mode mcdpsk_mode(unsigned wf, unsigned carriers, unsigned rate, unsigne
     return m;
 }
 
-std::vector<pu_sweep_mode> make_table(const std::string& name, bool fast) {
+std::vector<pu_sweep_mode> make_table(const std::string& name, bool fast, unsigned frame_bytes) {
     std::vector<pu_sweep_mode> t;
-    if (name == "smoke") {
+    if (name == "frames") {
+        // link-level FER: does a DATA frame of this many payload bytes arrive intact (several codewords in one OFDM frame)?
+        std::vector<unsigned> sizes = frame_bytes ? std::vector<unsigned>{frame_bytes} : std::vector<unsigned>{200, 1000};
+        for (unsigned bytes : sizes)
+            for (unsigned ch : {PU_CH_AWGN, PU_CH_GOOD, PU_CH_POOR}) {
+                const float step = ch == PU_CH_AWGN ? 1.0f : 2.0f;
+                pu_sweep_mode rows[] = {ofdm_mode(PU_WF_OFDM, 512, PU_MOD_DQPSK, PU_RATE_1_2, ch, -2, step, 12, fast),
+                                        ofdm_mode(PU_WF_OFDM, 512, PU_MOD_QAM16, PU_RATE_1_2, ch, 6, step, 12, fast),
+                                        ofdm_mode(PU_WF_OFDM, 1024, PU_MOD_QAM32, PU_RATE_3_4, ch, 10, step, 12, fast),
+                                        ofdm_mode(PU_WF_OFDM_CHIRP, 512, PU_MOD_DQPSK, PU_RATE_1_2, ch, 0, step, 12, fast)};
+                for (pu_sweep_mode& m : rows) {
+                    m.frame_payload_bytes = bytes;
+                    t.push_back(m);
+                }
+            }
+    } else if (name == "smoke") {
         t.push_back(ofdm_mode(PU_WF_OFDM, 512, PU_MOD_DQPSK, PU_RATE_1_2, PU_CH_AWGN, -4, 1, 13, fast));
         t.push_back(ofdm_mode(PU_WF_OFDM, 1024, PU_MOD_QAM32, PU_RATE_3_4, PU_CH_GOOD, 8, 2, 6, fast));
         t.push_back(dpsk_mode(PU_WF_DPSK, 1, PU_RATE_1_4, PU_CH_POOR, -11, 4, 8));
@@ -202,7 +218,8 @@ int main(int argc, char** argv) {
         if (rank == 0) remove(path);
     }
 
-    std::vector<pu_sweep_mode> modes = make_table(table, fast);
+    const unsigned frame_bytes = static_cast<unsigned>(atoi(arg(argc, argv, "--frame-bytes", "0")));
+    std::vector<pu_sweep_mode> modes = make_table(table, fast, frame_bytes);
     if (fresh)
         for (auto& m : modes) m.fresh_payloads = 1;
     pu_sweep_desc d{};
@@ -250,6 +267,15 @@ int main(int argc, char** argv) {
                 double lo, hi;
                 pu_wilson_interval(c[1], c[0], 1.96, &lo, &hi);
                 frames_all += c[0];
+                if (md.frame_payload_bytes) {     // whole-frame counters {frames, frame_errors, codewords_failed, codewords, header_failures, 0}
+                    fprintf(out, "{\"mode\": %u, \"waveform\": \"%s\", \"modem\": \"%s\", \"code_rate\": \"%s\", \"channel\": \"%s\", \"cfo_hz\": %.1f, \"snr_db\": %.2f, "
+                                 "\"frame_payload_bytes\": %u, \"codewords\": %llu, \"frames\": %llu, \"frame_errors\": %llu, \"fer\": %.6g, \"fer_ci95\": [%.6g, %.6g], "
+                                 "\"codeword_fail_rate\": %.6g, \"header_fail_rate\": %.6g}\n",
+                            m, kWaveform[md.waveform], desc, kRate[md.code_rate], kChannel[md.channel], md.cfo_hz, md.snr_first_db + s * md.snr_step_db,
+                            md.frame_payload_bytes, (unsigned long long)(c[0] ? c[3] / c[0] : 0), (unsigned long long)c[0], (unsigned long long)c[1],
+                            c[0] ? double(c[1]) / c[0] : 0.0, lo, hi, c[3] ? double(c[2]) / c[3] : 0.0, c[0] ? double(c[4]) / c[0] : 0.0);
+                    continue;
+                }
                 fprintf(out, "{\"mode\": %u, \"waveform\": \"%s\", \"modem\": \"%s\", \"code_rate\": \"%s\", \"channel\": \"%s\", \"cfo_hz\": %.1f, \"snr_db\": %.2f, "
                              "\"frames\": %llu, \"frame_errors\": %llu, \"fer\": %.6g, \"fer_ci95\": [%.6g, %.6g], \"ber\": %.6g, \"decode_fail\": %.6g, "
                              "\"avg_iters\": %.4g}\n",
