@@ -344,30 +344,21 @@ pu_status pu_channel_apply_cfo_batch(pu_ctx* ctx, float* samples, size_t B, size
         ctx->cfo_mix_len = L;
         ctx->cfo_mix_fs = sample_rate;
     }
-    float* d_x = samples;
-    const float* d_cfo = cfo_hz;
-    float *dx = nullptr, *dc = nullptr;
-    if (space == PU_MEM_HOST) {
-        PU_CUDA_TRY(cudaMalloc(&dx, B * stride * sizeof(float)));
-        PU_CUDA_TRY(cudaMalloc(&dc, B * sizeof(float)));
-        PU_CUDA_TRY(cudaMemcpyAsync(dx, samples, B * stride * sizeof(float), cudaMemcpyHostToDevice, st));
-        PU_CUDA_TRY(cudaMemcpyAsync(dc, cfo_hz, B * sizeof(float), cudaMemcpyHostToDevice, st));
-        d_x = dx; d_cfo = dc;
-    }
-    (void)cudaGetLastError();
-    pu::channel_cfo_kernel<<<static_cast<unsigned>((B + 3) / 4), 128, 0, st>>>(d_x, stride, B, static_cast<int>(L), d_cfo, static_cast<double>(sample_rate),
-                                                                              static_cast<const float2*>(ctx->cfo_mix.ptr));
-    ctx->launches.fetch_add(1);
-    pu_status rs = PU_OK;
-    cudaError_t e = cudaGetLastError();
-    if (e == cudaSuccess && space == PU_MEM_HOST) {
-        e = cudaMemcpyAsync(samples, dx, B * stride * sizeof(float), cudaMemcpyDeviceToHost, st);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-    }
-    if (e != cudaSuccess) { pu::set_error("pu_channel_apply_cfo_batch: %s", cudaGetErrorString(e)); rs = PU_ERR_CUDA; }
-    if (dx) cudaFree(dx);
-    if (dc) cudaFree(dc);
-    return rs;
+    auto launch = [&](float* d_x, size_t d_stride, size_t nb, const float* d_cfo) -> pu_status {
+        (void)cudaGetLastError();
+        pu::channel_cfo_kernel<<<static_cast<unsigned>((nb + 3) / 4), 128, 0, st>>>(d_x, d_stride, nb, static_cast<int>(L), d_cfo,
+                                                                                   static_cast<double>(sample_rate), static_cast<const float2*>(ctx->cfo_mix.ptr));
+        ctx->launches.fetch_add(1);
+        PU_CUDA_TRY(cudaGetLastError());
+        return PU_OK;
+    };
+    if (space == PU_MEM_DEVICE) return launch(samples, stride, B, cfo_hz);
+    pu::HostStage hs(ctx, st, B);
+    float* d_x;
+    const float* d_cfo;
+    hs.inout(&d_x, samples, L, stride);
+    hs.in(&d_cfo, cfo_hz, 1);
+    return hs.run([&](size_t nb) { return launch(d_x, L, nb, d_cfo); });
 }
 
 pu_status pu_channel_apply_batch(pu_ctx* ctx, const pu_channel_config* cfg, const float* tx_pool, size_t pool_stride,
@@ -394,29 +385,19 @@ pu_status pu_channel_apply_batch(pu_ctx* ctx, const pu_channel_config* cfg, cons
     };
     if (space == PU_MEM_DEVICE) return launch(tx_pool, tx_index, noise_std, seed, B, rx);
 
-    // host buffers (tests, small batches): plain staging
-    float *d_pool = nullptr, *d_std = nullptr, *d_rx = nullptr;
-    uint32_t* d_idx = nullptr;
-    uint64_t* d_seed = nullptr;
-    std::vector<uint32_t> idx(B, 0);
-    if (tx_index) for (size_t b = 0; b < B; ++b) { idx[b] = tx_index[b]; PU_REQUIRE(idx[b] < pool_count, "pu_channel_apply_batch: tx_index out of range"); }
-    PU_CUDA_TRY(cudaMalloc(&d_pool, pool_count * pool_stride * sizeof(float)));
-    PU_CUDA_TRY(cudaMalloc(&d_std, B * sizeof(float)));
-    PU_CUDA_TRY(cudaMalloc(&d_rx, B * L * sizeof(float)));
-    PU_CUDA_TRY(cudaMalloc(&d_idx, B * sizeof(uint32_t)));
-    PU_CUDA_TRY(cudaMalloc(&d_seed, B * sizeof(uint64_t)));
-    PU_CUDA_TRY(cudaMemcpyAsync(d_pool, tx_pool, pool_count * pool_stride * sizeof(float), cudaMemcpyHostToDevice, st));
-    PU_CUDA_TRY(cudaMemcpyAsync(d_std, noise_std, B * sizeof(float), cudaMemcpyHostToDevice, st));
-    PU_CUDA_TRY(cudaMemcpyAsync(d_idx, idx.data(), B * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
-    PU_CUDA_TRY(cudaMemcpyAsync(d_seed, seed, B * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
-    pu_status s = launch(d_pool, d_idx, d_std, d_seed, B, d_rx);
-    if (s == PU_OK) {
-        cudaError_t e = cudaMemcpyAsync(rx, d_rx, B * L * sizeof(float), cudaMemcpyDeviceToHost, st);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-        if (e != cudaSuccess) { pu::set_error("pu_channel_apply_batch: %s", cudaGetErrorString(e)); s = PU_ERR_CUDA; }
-    }
-    cudaFree(d_pool); cudaFree(d_std); cudaFree(d_rx); cudaFree(d_idx); cudaFree(d_seed);
-    return s;
+    // host buffers: the indices come from outside the program, check them before any kernel reads the pool with them
+    if (tx_index) for (size_t b = 0; b < B; ++b) PU_REQUIRE(tx_index[b] < pool_count, "pu_channel_apply_batch: tx_index out of range");
+    pu::HostStage hs(ctx, st, B);
+    const float *d_pool, *d_std;
+    const uint32_t* d_idx;
+    const uint64_t* d_seed;
+    float* d_rx;
+    hs.whole(&d_pool, tx_pool, pool_count * pool_stride);
+    hs.in(&d_idx, tx_index, 1);
+    hs.in(&d_std, noise_std, 1);
+    hs.in(&d_seed, seed, 1);
+    hs.out(&d_rx, rx, L);
+    return hs.run([&](size_t nb) { return launch(d_pool, d_idx, d_std, d_seed, nb, d_rx); });
 }
 
 }  // extern "C"

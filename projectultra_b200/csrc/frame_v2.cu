@@ -117,36 +117,29 @@ pu_status pu_frame_decode_batch(pu_ctx* ctx, pu_ldpc* dec, const float* llr, siz
     PU_REQUIRE(num_codewords >= 1 && num_codewords <= 255 && frame_cap > 0 && B * num_codewords < (1u << 30), "pu_frame_decode_batch: bad size");
     PU_CUDA_TRY(cudaSetDevice(ctx->device));
     cudaStream_t st = pu::pick_stream(ctx, stream, space);
+    if (space == PU_MEM_HOST) {
+        pu::HostStage hs(ctx, st, B);
+        const float* d_llr;
+        uint8_t* d_frame;
+        int32_t *d_len, *d_info;
+        hs.in(&d_llr, llr, num_codewords * PU_LDPC_N);
+        hs.out(&d_frame, frame_out, frame_cap);
+        hs.out(&d_len, frame_len, 1);
+        hs.out(&d_info, info, 5);
+        return hs.run([&](size_t nb) {
+            return pu_frame_decode_batch(ctx, dec, d_llr, nb, num_codewords, d_frame, frame_cap, d_len, d_info, PU_MEM_DEVICE, st);
+        });
+    }
     const int kbytes = (pu_ldpc_info_bits(dec) + 7) / 8;
     const size_t ncw = B * num_codewords;
     // grow-only scratch on the context (the calling convention is one thread per context, as for the reference's objects)
     pu_status s;
-    const float* d_llr = llr;
-    uint8_t* d_out = frame_out;
-    int32_t* d_len = frame_len;
-    int32_t* d_info = info;
-    const size_t out_off_len = ((B * frame_cap + 15) / 16) * 16, out_off_info = out_off_len + B * sizeof(int32_t);
-    if (space == PU_MEM_HOST) {
-        if ((s = ctx->f_llr.reserve(ncw * PU_LDPC_N * sizeof(float))) != PU_OK) return s;
-        if ((s = ctx->f_out.reserve(out_off_info + B * 5 * sizeof(int32_t))) != PU_OK) return s;
-        PU_CUDA_TRY(cudaMemcpyAsync(ctx->f_llr.ptr, llr, ncw * PU_LDPC_N * sizeof(float), cudaMemcpyHostToDevice, st));
-        PU_CUDA_TRY(cudaMemsetAsync(ctx->f_out.ptr, 0, B * frame_cap, st));
-        d_llr = static_cast<const float*>(ctx->f_llr.ptr);
-        d_out = static_cast<uint8_t*>(ctx->f_out.ptr);
-        d_len = reinterpret_cast<int32_t*>(d_out + out_off_len);
-        d_info = reinterpret_cast<int32_t*>(d_out + out_off_info);
-    }
     if ((s = ctx->f_bytes.reserve(ncw * static_cast<size_t>(kbytes))) != PU_OK) return s;
     if ((s = ctx->f_ok.reserve(ncw)) != PU_OK) return s;
     if ((s = ctx->f_iters.reserve(ncw * sizeof(int32_t))) != PU_OK) return s;
-    s = pu::frame_decode_enqueue(ctx, dec, d_llr, B, static_cast<int>(num_codewords), nullptr, static_cast<uint8_t*>(ctx->f_bytes.ptr),
-                                 static_cast<uint8_t*>(ctx->f_ok.ptr), static_cast<int32_t*>(ctx->f_iters.ptr), d_out, frame_cap, d_len, d_info, st);
+    s = pu::frame_decode_enqueue(ctx, dec, llr, B, static_cast<int>(num_codewords), nullptr, static_cast<uint8_t*>(ctx->f_bytes.ptr),
+                                 static_cast<uint8_t*>(ctx->f_ok.ptr), static_cast<int32_t*>(ctx->f_iters.ptr), frame_out, frame_cap, frame_len, info, st);
     if (s != PU_OK) return s;
-    if (space == PU_MEM_HOST) {
-        PU_CUDA_TRY(cudaMemcpyAsync(frame_out, d_out, B * frame_cap, cudaMemcpyDeviceToHost, st));
-        PU_CUDA_TRY(cudaMemcpyAsync(frame_len, d_len, B * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-        PU_CUDA_TRY(cudaMemcpyAsync(info, d_info, B * 5 * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    }
     PU_CUDA_TRY(cudaStreamSynchronize(st));           // results are complete on return (the scratch is reused by the next call)
     return PU_OK;
 }

@@ -337,19 +337,6 @@ __global__ void __launch_bounds__(T, MINB) ldpc_flood_reg_kernel(LdpcRegDev t, c
     }
 }
 
-struct DevArray {
-    void* p = nullptr;
-    ~DevArray() { if (p) cudaFree(p); }
-    template <class T>
-    pu_status upload(const std::vector<T>& v) {
-        if (p) { cudaFree(p); p = nullptr; }
-        PU_CUDA_TRY(cudaMalloc(&p, std::max<size_t>(v.size() * sizeof(T), 16)));
-        PU_CUDA_TRY(cudaMemcpy(p, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice));
-        PU_CUDA_TRY(cudaStreamSynchronize(cudaStreamLegacy));   // pageable source: the DMA must have landed before a non-blocking stream reads it
-        return PU_OK;
-    }
-};
-
 }  // namespace pu
 
 struct pu_ldpc {
@@ -358,9 +345,9 @@ struct pu_ldpc {
     int max_iter = 50;
     pu::LdpcCode code;
     pu::LdpcHostTables host;
-    pu::DevArray d_ninfo, d_check, d_var, d_deg, d_slot;
+    pu::DevMem d_ninfo, d_check, d_var, d_deg, d_slot;
     pu::LdpcLayout layout;
-    pu::DevArray r_ninfo, r_check, r_rd, r_wr, r_vslot, r_svar;
+    pu::DevMem r_ninfo, r_check, r_rd, r_wr, r_vslot, r_svar;
     pu::LdpcRegDev reg{};
     pu::LdpcDevTables dev{};
     int threads = 128;
@@ -373,11 +360,11 @@ struct pu_ldpc {
         code = pu::build_ldpc_code(rate);
         host = pu::make_ldpc_tables(code);
         pu_status s;
-        if ((s = d_ninfo.upload(host.cn_ninfo)) != PU_OK) return s;
-        if ((s = d_check.upload(host.cn_check)) != PU_OK) return s;
-        if ((s = d_var.upload(host.cn_var)) != PU_OK) return s;
-        if ((s = d_deg.upload(host.vn_deg)) != PU_OK) return s;
-        if ((s = d_slot.upload(host.vn_slot)) != PU_OK) return s;
+        if ((s = d_ninfo.upload(host.cn_ninfo.data(), host.cn_ninfo.size())) != PU_OK) return s;
+        if ((s = d_check.upload(host.cn_check.data(), host.cn_check.size())) != PU_OK) return s;
+        if ((s = d_var.upload(host.cn_var.data(), host.cn_var.size())) != PU_OK) return s;
+        if ((s = d_deg.upload(host.vn_deg.data(), host.vn_deg.size())) != PU_OK) return s;
+        if ((s = d_slot.upload(host.vn_slot.data(), host.vn_slot.size())) != PU_OK) return s;
         dev.k = host.k;
         dev.m = host.m;
         dev.dv_max = host.dv_max;
@@ -391,12 +378,12 @@ struct pu_ldpc {
         threads = (per_round + 31) / 32 * 32;
         smem_bytes = sizeof(float) * (static_cast<size_t>(pu::kE + 2) * host.m + 2 * static_cast<size_t>(host.k));
         layout = pu::make_ldpc_layout(code);
-        if ((s = r_ninfo.upload(layout.cn_ninfo)) != PU_OK) return s;
-        if ((s = r_check.upload(layout.cn_check)) != PU_OK) return s;
-        if ((s = r_rd.upload(layout.cn_rd)) != PU_OK) return s;
-        if ((s = r_wr.upload(layout.cn_wr)) != PU_OK) return s;
-        if ((s = r_vslot.upload(layout.var_slot)) != PU_OK) return s;
-        if ((s = r_svar.upload(layout.slot_var)) != PU_OK) return s;
+        if ((s = r_ninfo.upload(layout.cn_ninfo.data(), layout.cn_ninfo.size())) != PU_OK) return s;
+        if ((s = r_check.upload(layout.cn_check.data(), layout.cn_check.size())) != PU_OK) return s;
+        if ((s = r_rd.upload(layout.cn_rd.data(), layout.cn_rd.size())) != PU_OK) return s;
+        if ((s = r_wr.upload(layout.cn_wr.data(), layout.cn_wr.size())) != PU_OK) return s;
+        if ((s = r_vslot.upload(layout.var_slot.data(), layout.var_slot.size())) != PU_OK) return s;
+        if ((s = r_svar.upload(layout.slot_var.data(), layout.slot_var.size())) != PU_OK) return s;
         reg.k = layout.k; reg.m = layout.m; reg.kpad = layout.kpad; reg.inf_slot = layout.inf_slot;
         reg.msg_words = layout.msg_words; reg.threads = layout.threads;
         reg.cn_ninfo = static_cast<const uint8_t*>(r_ninfo.p);
@@ -514,37 +501,15 @@ pu_status pu_ldpc_decode_batch(pu_ldpc* h, const float* llr, size_t llr_stride, 
     cudaStream_t st = pu::pick_stream(ctx, stream, space);
     if (space == PU_MEM_DEVICE) return launch_decode(h, llr, llr_stride, B, info_bytes, info_stride, ok, iters, st);
 
-    // host buffers: stage through pinned memory in slabs so that arbitrarily large batches fit
-    const size_t slab = std::min<size_t>(B, 1u << 16);
-    pu_status s;
-    if ((s = ctx->d_in.reserve(slab * PU_LDPC_N * sizeof(float))) != PU_OK) return s;
-    if ((s = ctx->h_in.reserve(slab * PU_LDPC_N * sizeof(float))) != PU_OK) return s;
-    const size_t out_row = kb + 1 + sizeof(int32_t);
-    if ((s = ctx->d_out.reserve(slab * out_row + 64)) != PU_OK) return s;
-    if ((s = ctx->h_out.reserve(slab * out_row + 64)) != PU_OK) return s;
-    for (size_t off = 0; off < B; off += slab) {
-        const size_t nb = std::min(slab, B - off);
-        float* hin = static_cast<float*>(ctx->h_in.ptr);
-        for (size_t b = 0; b < nb; ++b) std::memcpy(hin + b * PU_LDPC_N, llr + (off + b) * llr_stride, PU_LDPC_N * sizeof(float));
-        PU_CUDA_TRY(cudaMemcpyAsync(ctx->d_in.ptr, hin, nb * PU_LDPC_N * sizeof(float), cudaMemcpyHostToDevice, st));
-        uint8_t* d_info = static_cast<uint8_t*>(ctx->d_out.ptr);
-        int32_t* d_iters = reinterpret_cast<int32_t*>(d_info + ((slab * kb + 15) / 16) * 16);
-        uint8_t* d_ok = reinterpret_cast<uint8_t*>(d_iters + slab);
-        s = launch_decode(h, static_cast<const float*>(ctx->d_in.ptr), PU_LDPC_N, nb, d_info, kb, d_ok, d_iters, st);
-        if (s != PU_OK) return s;
-        uint8_t* hout = static_cast<uint8_t*>(ctx->h_out.ptr);
-        const size_t total = static_cast<size_t>(reinterpret_cast<uint8_t*>(d_ok + slab) - d_info);
-        PU_CUDA_TRY(cudaMemcpyAsync(hout, d_info, total, cudaMemcpyDeviceToHost, st));
-        PU_CUDA_TRY(cudaStreamSynchronize(st));
-        const int32_t* h_iters = reinterpret_cast<const int32_t*>(hout + ((slab * kb + 15) / 16) * 16);
-        const uint8_t* h_ok = reinterpret_cast<const uint8_t*>(h_iters + slab);
-        for (size_t b = 0; b < nb; ++b) {
-            std::memcpy(info_bytes + (off + b) * info_stride, hout + b * kb, kb);
-            if (ok) ok[off + b] = h_ok[b];
-            if (iters) iters[off + b] = h_iters[b];
-        }
-    }
-    return PU_OK;
+    pu::HostStage hs(ctx, st, B);
+    const float* d_llr;
+    uint8_t *d_info, *d_ok;
+    int32_t* d_iters;
+    hs.in(&d_llr, llr, PU_LDPC_N, llr_stride);
+    hs.out(&d_info, info_bytes, kb, info_stride);
+    hs.out(&d_ok, ok, 1);
+    hs.out(&d_iters, iters, 1);
+    return hs.run([&](size_t nb) { return launch_decode(h, d_llr, PU_LDPC_N, nb, d_info, kb, d_ok, d_iters, st); });
 }
 
 pu_status pu_ldpc_decode_soft(pu_ldpc* h, const float* llr, size_t n_llr, uint8_t* out, size_t out_cap,

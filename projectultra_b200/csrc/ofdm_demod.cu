@@ -1059,23 +1059,6 @@ __global__ void acquire_windows_kernel(const int4* __restrict__ acq, size_t B, i
     if (n_llr) n_llr[b] = min(n * llr_per_symbol, llr_stride);
 }
 
-struct DevMem {
-    void* p = nullptr;
-    ~DevMem() { if (p) cudaFree(p); }
-    template <class T>
-    pu_status upload(const T* src, size_t n) {
-        if (p) { cudaFree(p); p = nullptr; }
-        PU_CUDA_TRY(cudaMalloc(&p, std::max<size_t>(n * sizeof(T), 16)));
-        if (n) {
-            // A pageable H2D cudaMemcpy may return once the source is staged, before the DMA has landed, and the kernels that
-            // read these tables / samples run on NON-BLOCKING streams (no implicit ordering with the legacy stream): wait for it.
-            PU_CUDA_TRY(cudaMemcpy(p, src, n * sizeof(T), cudaMemcpyHostToDevice));
-            PU_CUDA_TRY(cudaStreamSynchronize(cudaStreamLegacy));
-        }
-        return PU_OK;
-    }
-};
-
 }  // namespace pu
 
 void pu_ldpc_encoder_view(const pu_ldpc* h, int* k, int* m, const uint8_t** cn_ninfo, const uint16_t** cn_check, const uint16_t** cn_var);   // ldpc_decode.cu
@@ -1393,40 +1376,18 @@ pu_status pu_ofdm_presynced_batch(pu_ofdm* h, const float* samples, size_t B, si
     if (space == PU_MEM_DEVICE)
         return launch_ofdm(h, samples, B, L, training_symbols, cfo_hz, cfo_phase, llr_out, llr_stride, snr_db, final_cfo_hz, nullptr, st);
 
-    const size_t slab = std::min<size_t>(B, 8192);
-    pu_status s;
-    const size_t in_floats = slab * (L + 2), out_floats = slab * (llr_stride + 2);
-    if ((s = ctx->d_in.reserve(in_floats * sizeof(float))) != PU_OK) return s;
-    if ((s = ctx->h_in.reserve(in_floats * sizeof(float))) != PU_OK) return s;
-    if ((s = ctx->d_out.reserve(out_floats * sizeof(float))) != PU_OK) return s;
-    if ((s = ctx->h_out.reserve(out_floats * sizeof(float))) != PU_OK) return s;
-    for (size_t off = 0; off < B; off += slab) {
-        const size_t nb = std::min(slab, B - off);
-        float* hin = static_cast<float*>(ctx->h_in.ptr);
-        std::memcpy(hin, samples + off * L, nb * L * sizeof(float));
-        float* hcfo = hin + slab * L;
-        float* hph = hcfo + slab;
-        for (size_t b = 0; b < nb; ++b) {
-            hcfo[b] = cfo_hz ? cfo_hz[off + b] : 0.0f;
-            hph[b] = cfo_phase ? cfo_phase[off + b] : 0.0f;
-        }
-        float* din = static_cast<float*>(ctx->d_in.ptr);
-        PU_CUDA_TRY(cudaMemcpyAsync(din, hin, in_floats * sizeof(float), cudaMemcpyHostToDevice, st));
-        float* dout = static_cast<float*>(ctx->d_out.ptr);
-        PU_CUDA_TRY(cudaMemsetAsync(dout, 0, out_floats * sizeof(float), st));
-        // without caller-supplied CFO / phase the launch sees NULL arrays and may take the differential fast kernels
-        const bool has_cfo = cfo_hz || cfo_phase;
-        s = launch_ofdm(h, din, nb, L, training_symbols, has_cfo ? din + slab * L : nullptr, has_cfo ? din + slab * L + slab : nullptr, dout,
-                        llr_stride, dout + slab * llr_stride, dout + slab * llr_stride + slab, nullptr, st);
-        if (s != PU_OK) return s;
-        float* hout = static_cast<float*>(ctx->h_out.ptr);
-        PU_CUDA_TRY(cudaMemcpyAsync(hout, dout, out_floats * sizeof(float), cudaMemcpyDeviceToHost, st));
-        PU_CUDA_TRY(cudaStreamSynchronize(st));
-        std::memcpy(llr_out + off * llr_stride, hout, nb * llr_stride * sizeof(float));
-        if (snr_db) std::memcpy(snr_db + off, hout + slab * llr_stride, nb * sizeof(float));
-        if (final_cfo_hz) std::memcpy(final_cfo_hz + off, hout + slab * llr_stride + slab, nb * sizeof(float));
-    }
-    return PU_OK;
+    pu::HostStage hs(ctx, st, B);
+    const float *d_x, *d_cfo, *d_ph;
+    float *d_llr, *d_snr, *d_fcfo;
+    hs.in(&d_x, samples, L);
+    hs.in(&d_cfo, cfo_hz, 1);
+    hs.in(&d_ph, cfo_phase, 1);
+    hs.out(&d_llr, llr_out, llr_stride);
+    hs.out(&d_snr, snr_db, 1);
+    hs.out(&d_fcfo, final_cfo_hz, 1);
+    return hs.run([&](size_t nb) {
+        return launch_ofdm(h, d_x, nb, L, training_symbols, d_cfo, d_ph, d_llr, llr_stride, d_snr, d_fcfo, nullptr, st);
+    });
 }
 
 pu_status pu_ofdm_chirp_receive_batch(pu_ofdm* h, const float* samples, size_t B, size_t L, float threshold, float* llr_out,
@@ -1444,53 +1405,40 @@ pu_status pu_ofdm_chirp_receive_batch(pu_ofdm* h, const float* samples, size_t B
     cudaStream_t st = pu::pick_stream(ctx, stream, space);
     const pu::OfdmPlan& p = h->plan;
     if (threshold <= 0.0f) threshold = 0.15f;        // the callers' value, tools/test_iwaveform.cpp:133
-    pu::DevMem dx, dl, dn, dsn, dinfo, dval, dstart, dnsym, dcfo, dph;
-    const float* d_x = samples;
-    float* d_llr = llr_out;
-    int32_t* d_n = n_llr;
-    float* d_snr = snr_db;
-    int32_t* d_info = sync_info;
-    float* d_val = sync_values;
-    std::vector<int32_t> zi(B * 4, 0);
     if (space == PU_MEM_HOST) {
-        if ((s = dx.upload(samples, B * L)) != PU_OK) return s;
-        if ((s = dinfo.upload(zi.data(), B * 4)) != PU_OK) return s;
-        if ((s = dval.upload(zi.data(), B * 4)) != PU_OK) return s;
-        d_x = static_cast<const float*>(dx.p); d_info = static_cast<int32_t*>(dinfo.p); d_val = static_cast<float*>(dval.p);
-        if (llr_out) {
-            std::vector<float> zl(B * llr_stride, 0.0f);
-            if ((s = dl.upload(zl.data(), zl.size())) != PU_OK) return s;
-            if ((s = dn.upload(zi.data(), B)) != PU_OK) return s;
-            if ((s = dsn.upload(zi.data(), B)) != PU_OK) return s;
-            d_llr = static_cast<float*>(dl.p); d_n = static_cast<int32_t*>(dn.p); d_snr = snr_db ? static_cast<float*>(dsn.p) : nullptr;
-        }
+        pu::HostStage hs(ctx, st, B);
+        const float* d_x;
+        float *d_val, *d_llr, *d_snr;
+        int32_t *d_info, *d_n;
+        hs.in(&d_x, samples, L);
+        hs.out(&d_info, sync_info, 4);
+        hs.out(&d_val, sync_values, 4);
+        hs.out(&d_llr, llr_out, llr_stride);
+        hs.out(&d_n, llr_out ? n_llr : nullptr, 1);
+        hs.out(&d_snr, llr_out ? snr_db : nullptr, 1);
+        return hs.run([&](size_t nb) {
+            return pu_ofdm_chirp_receive_batch(h, d_x, nb, L, threshold, d_llr, llr_stride, d_n, d_info, d_val, d_snr, PU_MEM_DEVICE, st);
+        });
     }
+    pu::DevMem dstart, dnsym, dcfo, dph;
+    std::vector<int32_t> zi(B, 0);
     if ((s = dstart.upload(zi.data(), B)) != PU_OK) return s;
     if ((s = dnsym.upload(zi.data(), B)) != PU_OK) return s;
     if ((s = dcfo.upload(zi.data(), B)) != PU_OK) return s;
     if ((s = dph.upload(zi.data(), B)) != PU_OK) return s;
     (void)cudaGetLastError();
-    PU_CUDA_TRY(pu::chirp_detect_launch(h->chirp, d_x, B, L, static_cast<int>(L), threshold, p.sym_len, reinterpret_cast<int4*>(d_info),
-                                        reinterpret_cast<float4*>(d_val), static_cast<int*>(dstart.p), static_cast<int*>(dnsym.p),
-                                        static_cast<float*>(dcfo.p), static_cast<float*>(dph.p), llr_out ? d_n : nullptr, p.n_data * p.bps,
+    PU_CUDA_TRY(pu::chirp_detect_launch(h->chirp, samples, B, L, static_cast<int>(L), threshold, p.sym_len, reinterpret_cast<int4*>(sync_info),
+                                        reinterpret_cast<float4*>(sync_values), static_cast<int*>(dstart.p), static_cast<int*>(dnsym.p),
+                                        static_cast<float*>(dcfo.p), static_cast<float*>(dph.p), llr_out ? n_llr : nullptr, p.n_data * p.bps,
                                         static_cast<int>(llr_stride), st));
     ctx->launches.fetch_add(1);
     if (llr_out) {
         // OFDMChirpWaveform::process (:170-199): setFrequencyOffsetWithPhase(cfo, accumulated phase); processPresynced(span, 2)
-        s = launch_ofdm(h, d_x, B, L, 2, static_cast<const float*>(dcfo.p), static_cast<const float*>(dph.p), d_llr, llr_stride, d_snr, nullptr,
+        s = launch_ofdm(h, samples, B, L, 2, static_cast<const float*>(dcfo.p), static_cast<const float*>(dph.p), llr_out, llr_stride, snr_db, nullptr,
                         nullptr, st, static_cast<const int*>(dstart.p), static_cast<const int*>(dnsym.p));
         if (s != PU_OK) return s;
     }
     PU_CUDA_TRY(cudaStreamSynchronize(st));           // the scratch buffers above are freed on return
-    if (space == PU_MEM_HOST) {
-        PU_CUDA_TRY(cudaMemcpy(sync_info, d_info, B * 4 * sizeof(int32_t), cudaMemcpyDeviceToHost));
-        PU_CUDA_TRY(cudaMemcpy(sync_values, d_val, B * 4 * sizeof(float), cudaMemcpyDeviceToHost));
-        if (llr_out) {
-            PU_CUDA_TRY(cudaMemcpy(llr_out, d_llr, B * llr_stride * sizeof(float), cudaMemcpyDeviceToHost));
-            PU_CUDA_TRY(cudaMemcpy(n_llr, d_n, B * sizeof(int32_t), cudaMemcpyDeviceToHost));
-            if (snr_db) PU_CUDA_TRY(cudaMemcpy(snr_db, d_snr, B * sizeof(float), cudaMemcpyDeviceToHost));
-        }
-    }
     return PU_OK;
 }
 
@@ -1592,20 +1540,19 @@ pu_status ofdm_tx_frames(pu_ofdm* h, const pu_ldpc* code, const uint8_t* frames,
     cudaStream_t st = pu::pick_stream(ctx, stream, space);
     (void)cudaGetLastError();
     const int fb = static_cast<int>(frame_bytes);
-    if (space == PU_MEM_DEVICE) {
-        PU_CUDA_TRY(pu::ofdm_tx_launch(t, frames, frame_stride, fb, n_cw, bpc, B, peak, out, out_stride, st));
+    auto launch = [&](const uint8_t* d_frames, size_t d_frame_stride, size_t nb, float* d_tx, size_t d_out_stride) -> pu_status {
+        PU_CUDA_TRY(pu::ofdm_tx_launch(t, d_frames, d_frame_stride, fb, n_cw, bpc, nb, peak, d_tx, d_out_stride, st));
         ctx->launches.fetch_add(1);
         return PU_OK;
-    }
-    // host memory: stage through the device; the padding of every output row beyond *frame_len comes back as it went in
-    pu::DevMem dp, dout;
-    if ((s = dp.upload(frames, (B - 1) * frame_stride + frame_bytes)) != PU_OK) return s;
-    if ((s = dout.upload(out, (B - 1) * out_stride + static_cast<size_t>(t.frame_len))) != PU_OK) return s;
-    PU_CUDA_TRY(pu::ofdm_tx_launch(t, static_cast<const uint8_t*>(dp.p), frame_stride, fb, n_cw, bpc, B, peak, static_cast<float*>(dout.p), out_stride, st));
-    ctx->launches.fetch_add(1);
-    PU_CUDA_TRY(cudaStreamSynchronize(st));
-    PU_CUDA_TRY(cudaMemcpy(out, dout.p, ((B - 1) * out_stride + static_cast<size_t>(t.frame_len)) * sizeof(float), cudaMemcpyDeviceToHost));
-    return PU_OK;
+    };
+    if (space == PU_MEM_DEVICE) return launch(frames, frame_stride, B, out, out_stride);
+    // host memory: the padding of every output row beyond *frame_len is not staged and stays as it was
+    pu::HostStage hs(ctx, st, B);
+    const uint8_t* d_frames;
+    float* d_tx;
+    hs.in(&d_frames, frames, frame_bytes, frame_stride);
+    hs.inout(&d_tx, out, static_cast<size_t>(t.frame_len), out_stride);
+    return hs.run([&](size_t nb) { return launch(d_frames, frame_bytes, nb, d_tx, static_cast<size_t>(t.frame_len)); });
 }
 }  // namespace
 }  // namespace pu
@@ -1658,19 +1605,14 @@ pu_status pu_ofdm_acquire_batch(pu_ofdm* h, const float* samples, size_t B, size
         ctx->launches.fetch_add(1);
         return PU_OK;
     }
-    pu::DevMem dx, di, dc;
-    if ((s = dx.upload(samples, B * L)) != PU_OK) return s;
-    std::vector<int32_t> zi(B * 4, 0);
-    std::vector<float> zc(B, 0.0f);
-    if ((s = di.upload(zi.data(), zi.size())) != PU_OK) return s;
-    if ((s = dc.upload(zc.data(), zc.size())) != PU_OK) return s;
-    PU_CUDA_TRY(pu::ofdm_acquire_launch(a, static_cast<const float*>(dx.p), B, L, static_cast<int>(L), static_cast<int>(std::min<size_t>(chunk, L)),
-                                        static_cast<int4*>(di.p), static_cast<float*>(dc.p), st));
-    ctx->launches.fetch_add(1);
-    PU_CUDA_TRY(cudaStreamSynchronize(st));
-    PU_CUDA_TRY(cudaMemcpy(sync_info, di.p, B * 4 * sizeof(int32_t), cudaMemcpyDeviceToHost));
-    PU_CUDA_TRY(cudaMemcpy(coarse_cfo_hz, dc.p, B * sizeof(float), cudaMemcpyDeviceToHost));
-    return PU_OK;
+    pu::HostStage hs(ctx, st, B);
+    const float* d_x;
+    int32_t* d_info;
+    float* d_cfo;
+    hs.in(&d_x, samples, L);
+    hs.out(&d_info, sync_info, 4);
+    hs.out(&d_cfo, coarse_cfo_hz, 1);
+    return hs.run([&](size_t nb) { return pu_ofdm_acquire_batch(h, d_x, nb, L, chunk, sync_threshold, d_info, d_cfo, PU_MEM_DEVICE, st); });
 }
 
 pu_status pu_ofdm_process_batch(pu_ofdm* h, const float* samples, size_t B, size_t L, size_t chunk, float sync_threshold,
@@ -1684,24 +1626,24 @@ pu_status pu_ofdm_process_batch(pu_ofdm* h, const float* samples, size_t B, size
     PU_CUDA_TRY(cudaSetDevice(ctx->device));
     cudaStream_t st = pu::pick_stream(ctx, stream, space);
     const pu::OfdmPlan& p = h->plan;
-    // device scratch: samples / llr (host callers), acquisition results, frame windows
-    pu::DevMem dx, dl, dn, dsn, dacq, dcfo, dstart, dnsym;
     pu_status s;
-    const float* d_x = samples;
-    float* d_llr = llr_out;
-    int32_t* d_n = n_llr;
-    float* d_snr = snr_db;
-    std::vector<float> zl;
     if (space == PU_MEM_HOST) {
-        if ((s = dx.upload(samples, B * L)) != PU_OK) return s;
-        zl.assign(B * llr_stride, 0.0f);
-        if ((s = dl.upload(zl.data(), zl.size())) != PU_OK) return s;
-        std::vector<int32_t> zn(B, 0);
-        if ((s = dn.upload(zn.data(), zn.size())) != PU_OK) return s;
-        if ((s = dsn.upload(zl.data(), B)) != PU_OK) return s;
-        d_x = static_cast<const float*>(dx.p); d_llr = static_cast<float*>(dl.p); d_n = static_cast<int32_t*>(dn.p);
-        d_snr = snr_db ? static_cast<float*>(dsn.p) : nullptr;
+        pu::HostStage hs(ctx, st, B);
+        const float* d_x;
+        float *d_llr, *d_snr, *d_cfo;
+        int32_t *d_n, *d_info;
+        hs.in(&d_x, samples, L);
+        hs.out(&d_llr, llr_out, llr_stride);
+        hs.out(&d_n, n_llr, 1);
+        hs.out(&d_snr, snr_db, 1);
+        hs.out(&d_info, sync_info, 4);
+        hs.out(&d_cfo, coarse_cfo_hz, 1);
+        return hs.run([&](size_t nb) {
+            return pu_ofdm_process_batch(h, d_x, nb, L, chunk, sync_threshold, d_llr, llr_stride, d_n, d_info, d_cfo, d_snr, PU_MEM_DEVICE, st);
+        });
     }
+    // device scratch: acquisition results, frame windows
+    pu::DevMem dacq, dcfo, dstart, dnsym;
     std::vector<int32_t> zi(B * 4, 0);
     if ((s = dacq.upload(zi.data(), zi.size())) != PU_OK) return s;
     if ((s = dcfo.upload(zi.data(), B)) != PU_OK) return s;
@@ -1716,30 +1658,22 @@ pu_status pu_ofdm_process_batch(pu_ofdm* h, const float* samples, size_t B, size
         if (sync_threshold > 0.0f) a.sync_threshold = sync_threshold;
         const size_t avail = std::min<size_t>(L, 40000);
         (void)cudaGetLastError();
-        PU_CUDA_TRY(pu::ofdm_acquire_launch(a, d_x, B, L, static_cast<int>(avail), static_cast<int>(std::min<size_t>(chunk, avail)),
+        PU_CUDA_TRY(pu::ofdm_acquire_launch(a, samples, B, L, static_cast<int>(avail), static_cast<int>(std::min<size_t>(chunk, avail)),
                                             static_cast<int4*>(dacq.p), static_cast<float*>(dcfo.p), st));
         ctx->launches.fetch_add(1);
     }
     pu::acquire_windows_kernel<<<static_cast<unsigned>((B + 255) / 256), 256, 0, st>>>(
         static_cast<const int4*>(dacq.p), B, static_cast<int>(L), p.sym_len, p.n_data * p.bps, static_cast<int>(llr_stride),
-        static_cast<int*>(dstart.p), static_cast<int*>(dnsym.p), d_n);
+        static_cast<int*>(dstart.p), static_cast<int*>(dnsym.p), n_llr);
     ctx->launches.fetch_add(1);
     // SYNCED state (demodulator.cpp:665-690): no LTS channel estimate, mixer restarted at the first data symbol, CFO = the
     // Schmidl-Cox estimate with zero rotator phase -- the presynced path with zero training symbols on the frame's window
-    s = launch_ofdm(h, d_x, B, L, 0, static_cast<const float*>(dcfo.p), nullptr, d_llr, llr_stride, d_snr, nullptr, nullptr, st,
+    s = launch_ofdm(h, samples, B, L, 0, static_cast<const float*>(dcfo.p), nullptr, llr_out, llr_stride, snr_db, nullptr, nullptr, st,
                     static_cast<const int*>(dstart.p), static_cast<const int*>(dnsym.p));
     if (s != PU_OK) return s;
+    if (sync_info) PU_CUDA_TRY(cudaMemcpyAsync(sync_info, dacq.p, B * 4 * sizeof(int32_t), cudaMemcpyDeviceToDevice, st));
+    if (coarse_cfo_hz) PU_CUDA_TRY(cudaMemcpyAsync(coarse_cfo_hz, dcfo.p, B * sizeof(float), cudaMemcpyDeviceToDevice, st));
     PU_CUDA_TRY(cudaStreamSynchronize(st));   // the scratch buffers above are freed on return
-    if (space == PU_MEM_HOST) {
-        PU_CUDA_TRY(cudaMemcpy(llr_out, d_llr, B * llr_stride * sizeof(float), cudaMemcpyDeviceToHost));
-        PU_CUDA_TRY(cudaMemcpy(n_llr, d_n, B * sizeof(int32_t), cudaMemcpyDeviceToHost));
-        if (snr_db) PU_CUDA_TRY(cudaMemcpy(snr_db, d_snr, B * sizeof(float), cudaMemcpyDeviceToHost));
-        if (sync_info) PU_CUDA_TRY(cudaMemcpy(sync_info, dacq.p, B * 4 * sizeof(int32_t), cudaMemcpyDeviceToHost));
-        if (coarse_cfo_hz) PU_CUDA_TRY(cudaMemcpy(coarse_cfo_hz, dcfo.p, B * sizeof(float), cudaMemcpyDeviceToHost));
-    } else {
-        if (sync_info) PU_CUDA_TRY(cudaMemcpy(sync_info, dacq.p, B * 4 * sizeof(int32_t), cudaMemcpyDeviceToDevice));
-        if (coarse_cfo_hz) PU_CUDA_TRY(cudaMemcpy(coarse_cfo_hz, dcfo.p, B * sizeof(float), cudaMemcpyDeviceToDevice));
-    }
     return PU_OK;
 }
 
@@ -1752,32 +1686,27 @@ pu_status pu_ofdm_training_cfo_batch(pu_ofdm* h, const float* samples, size_t B,
     PU_CUDA_TRY(cudaSetDevice(ctx->device));
     cudaStream_t st = pu::pick_stream(ctx, stream, space);
     const pu::OfdmPlan& p = h->plan;
-    pu::DevMem dx, dc;
-    const float* d_x = samples;
-    float* d_c = cfo_hz;
-    pu_status s;
     if (space == PU_MEM_HOST) {
-        std::vector<float> z(B, 0.0f);
-        if ((s = dx.upload(samples, B * L)) != PU_OK || (s = dc.upload(z.data(), B)) != PU_OK) return s;
-        d_x = static_cast<const float*>(dx.p);
-        d_c = static_cast<float*>(dc.p);
+        pu::HostStage hs(ctx, st, B);
+        const float* d_x;
+        float* d_c;
+        hs.in(&d_x, samples, L);
+        hs.out(&d_c, cfo_hz, 1);
+        return hs.run([&](size_t nb) { return pu_ofdm_training_cfo_batch(h, d_x, nb, L, training_symbols, d_c, PU_MEM_DEVICE, st); });
     }
     if (training_symbols < 2 || L < 2 * static_cast<size_t>(p.sym_len)) {          // ofdm_sync.cpp:279-282 (and nothing to correlate)
-        PU_CUDA_TRY(cudaMemsetAsync(d_c, 0, B * sizeof(float), st));
+        PU_CUDA_TRY(cudaMemsetAsync(cfo_hz, 0, B * sizeof(float), st));
     } else {
-        if ((s = h->ensure_nco(2)) != PU_OK) return s;
+        const pu_status s = h->ensure_nco(2);
+        if (s != PU_OK) return s;
         const int warps = 4;
         const size_t smem = static_cast<size_t>(warps) * 2 * p.nfft * sizeof(float2);
         static std::atomic<uint64_t> attr{0};
         PU_CUDA_TRY(pu::smem_optin(attr, pu::ofdm_training_cfo_kernel, 96 * 1024));
         (void)cudaGetLastError();
-        pu::ofdm_training_cfo_kernel<<<static_cast<unsigned>((B + warps - 1) / warps), warps * 32, smem, st>>>(h->dev, d_x, L, B, d_c);
+        pu::ofdm_training_cfo_kernel<<<static_cast<unsigned>((B + warps - 1) / warps), warps * 32, smem, st>>>(h->dev, samples, L, B, cfo_hz);
         ctx->launches.fetch_add(1);
         PU_CUDA_TRY(cudaGetLastError());
-    }
-    if (space == PU_MEM_HOST) {
-        PU_CUDA_TRY(cudaMemcpyAsync(cfo_hz, d_c, B * sizeof(float), cudaMemcpyDeviceToHost, st));
-        PU_CUDA_TRY(cudaStreamSynchronize(st));
     }
     return PU_OK;
 }
@@ -1796,22 +1725,16 @@ pu_status pu_ofdm_presynced_debug(pu_ofdm* h, const float* samples, size_t L, in
     const size_t rec = static_cast<size_t>(4 * nu + 3 * p.n_data + pu::kDbgScalars);
     PU_REQUIRE(records_cap >= rec * nds, "pu_ofdm_presynced_debug: records buffer too small");
     if (n_data_symbols) *n_data_symbols = nds;
-    pu::DevMem dx, dl, dr, dc;
-    pu_status s;
-    if ((s = dx.upload(samples, L)) != PU_OK) return s;
-    std::vector<float> zero(llr_cap, 0.0f), zr(rec * std::max(nds, 1), 0.0f);
-    if ((s = dl.upload(zero.data(), llr_cap)) != PU_OK) return s;
-    if ((s = dr.upload(zr.data(), zr.size())) != PU_OK) return s;
+    // one frame through the general presynced kernel, which records every symbol's intermediate values
+    pu::HostStage hs(ctx, st, 1);
     const float cp[2] = {cfo_hz, cfo_phase};
-    if ((s = dc.upload(cp, 2)) != PU_OK) return s;
-    s = launch_ofdm(h, static_cast<const float*>(dx.p), 1, L, training_symbols, static_cast<const float*>(dc.p),
-                    static_cast<const float*>(dc.p) + 1, static_cast<float*>(dl.p), llr_cap, nullptr, nullptr,
-                    static_cast<float*>(dr.p), st);
-    if (s != PU_OK) return s;
-    PU_CUDA_TRY(cudaStreamSynchronize(st));
-    PU_CUDA_TRY(cudaMemcpy(llr_out, dl.p, llr_cap * sizeof(float), cudaMemcpyDeviceToHost));
-    PU_CUDA_TRY(cudaMemcpy(records, dr.p, rec * nds * sizeof(float), cudaMemcpyDeviceToHost));
-    return PU_OK;
+    const float *d_x, *d_c;
+    float *d_llr, *d_rec;
+    hs.in(&d_x, samples, L);
+    hs.in(&d_c, cp, 2);
+    hs.out(&d_llr, llr_out, llr_cap);
+    hs.out(&d_rec, records, rec * nds);
+    return hs.run([&](size_t) { return launch_ofdm(h, d_x, 1, L, training_symbols, d_c, d_c + 1, d_llr, llr_cap, nullptr, nullptr, d_rec, st); });
 }
 
 }  // extern "C"

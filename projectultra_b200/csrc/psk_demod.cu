@@ -550,40 +550,6 @@ __global__ void __launch_bounds__(kCfoThreads) mcdpsk_cfo_correct_kernel(Hilbert
 
 #include "psk_handles.h"
 
-// Shared host-staging helper: samples (+ up to two per-frame float arrays) up, `out_floats` per frame (+ one per-frame
-// float array) back.
-template <class Launch>
-static pu_status psk_host_call(pu_ctx* ctx, cudaStream_t st, const float* samples, size_t B, size_t L, const float* a0, const float* a1,
-                               float* out, size_t out_stride, float* aux_out, Launch&& launch) {
-    const size_t slab = std::max<size_t>(1, std::min<size_t>(B, (64u << 20) / std::max<size_t>(L * sizeof(float), 1)));
-    pu_status s;
-    const size_t in_floats = slab * (L + 2), out_floats = slab * (out_stride + 1);
-    if ((s = ctx->d_in.reserve(in_floats * sizeof(float))) != PU_OK) return s;
-    if ((s = ctx->h_in.reserve(in_floats * sizeof(float))) != PU_OK) return s;
-    if ((s = ctx->d_out.reserve(out_floats * sizeof(float))) != PU_OK) return s;
-    if ((s = ctx->h_out.reserve(out_floats * sizeof(float))) != PU_OK) return s;
-    for (size_t off = 0; off < B; off += slab) {
-        const size_t nb = std::min(slab, B - off);
-        float* hin = static_cast<float*>(ctx->h_in.ptr);
-        std::memcpy(hin, samples + off * L, nb * L * sizeof(float));
-        for (size_t b = 0; b < nb; ++b) {
-            hin[slab * L + b] = a0 ? a0[off + b] : 0.0f;
-            hin[slab * L + slab + b] = a1 ? a1[off + b] : 0.0f;
-        }
-        float* din = static_cast<float*>(ctx->d_in.ptr);
-        float* dout = static_cast<float*>(ctx->d_out.ptr);
-        PU_CUDA_TRY(cudaMemcpyAsync(din, hin, in_floats * sizeof(float), cudaMemcpyHostToDevice, st));
-        PU_CUDA_TRY(cudaMemsetAsync(dout, 0, out_floats * sizeof(float), st));
-        if ((s = launch(din, nb, a0 ? din + slab * L : nullptr, a1 ? din + slab * L + slab : nullptr, dout, dout + slab * out_stride)) != PU_OK) return s;
-        float* hout = static_cast<float*>(ctx->h_out.ptr);
-        PU_CUDA_TRY(cudaMemcpyAsync(hout, dout, out_floats * sizeof(float), cudaMemcpyDeviceToHost, st));
-        PU_CUDA_TRY(cudaStreamSynchronize(st));
-        std::memcpy(out + off * out_stride, hout, nb * out_stride * sizeof(float));
-        if (aux_out) std::memcpy(aux_out + off, hout + slab * out_stride, nb * sizeof(float));
-    }
-    return PU_OK;
-}
-
 extern "C" {
 
 pu_status pu_dpsk_create(pu_ctx* ctx, const pu_dpsk_config* cfg, pu_dpsk** out) {
@@ -673,28 +639,19 @@ pu_status pu_dpsk_receive_batch(pu_dpsk* h, const float* samples, size_t B, size
         if (!llr_out || L <= static_cast<size_t>(39) * sps) return PU_OK;
         return dpsk_launch(h, samples, B, L, static_cast<size_t>(39) * sps, 1, est_cfo_hz, phase_offset, llr_out, llr_stride, st, data_start, n_llr);
     }
-    pu::PskDevMem dx, dst, dc, dp, dl, dn;
-    std::vector<float> zf(std::max<size_t>(B * std::max<size_t>(llr_stride, 1), B), 0.0f);
-    std::vector<int32_t> zi(B, 0);
-    if ((s = dx.upload(samples, B * L)) != PU_OK) return s;
-    if ((s = dst.upload(zi.data(), B)) != PU_OK) return s;
-    if ((s = dc.upload(zf.data(), B)) != PU_OK) return s;
-    if ((s = dp.upload(zf.data(), B)) != PU_OK) return s;
-    if ((s = dn.upload(zi.data(), B)) != PU_OK) return s;
-    if (llr_out && (s = dl.upload(zf.data(), B * llr_stride)) != PU_OK) return s;
-    s = pu_dpsk_receive_batch(h, static_cast<const float*>(dx.p), B, L, llr_out ? static_cast<float*>(dl.p) : nullptr, llr_stride,
-                              static_cast<int32_t*>(dn.p), static_cast<int32_t*>(dst.p), static_cast<float*>(dc.p), static_cast<float*>(dp.p),
-                              PU_MEM_DEVICE, st);
-    if (s != PU_OK) return s;
-    PU_CUDA_TRY(cudaStreamSynchronize(st));
-    PU_CUDA_TRY(cudaMemcpy(data_start, dst.p, B * sizeof(int32_t), cudaMemcpyDeviceToHost));
-    PU_CUDA_TRY(cudaMemcpy(est_cfo_hz, dc.p, B * sizeof(float), cudaMemcpyDeviceToHost));
-    PU_CUDA_TRY(cudaMemcpy(phase_offset, dp.p, B * sizeof(float), cudaMemcpyDeviceToHost));
-    if (llr_out) {
-        PU_CUDA_TRY(cudaMemcpy(llr_out, dl.p, B * llr_stride * sizeof(float), cudaMemcpyDeviceToHost));
-        PU_CUDA_TRY(cudaMemcpy(n_llr, dn.p, B * sizeof(int32_t), cudaMemcpyDeviceToHost));
-    }
-    return PU_OK;
+    pu::HostStage hs(ctx, st, B);
+    const float* d_x;
+    float *d_llr, *d_cfo, *d_phase;
+    int32_t *d_n, *d_start;
+    hs.in(&d_x, samples, L);
+    hs.out(&d_llr, llr_out, llr_stride);
+    hs.out(&d_n, llr_out ? n_llr : nullptr, 1);
+    hs.out(&d_start, data_start, 1);
+    hs.out(&d_cfo, est_cfo_hz, 1);
+    hs.out(&d_phase, phase_offset, 1);
+    return hs.run([&](size_t nb) {
+        return pu_dpsk_receive_batch(h, d_x, nb, L, d_llr, llr_stride, d_n, d_start, d_cfo, d_phase, PU_MEM_DEVICE, st);
+    });
 }
 
 void pu_dpsk_destroy(pu_dpsk* h) {
@@ -753,10 +710,14 @@ pu_status pu_dpsk_demod_soft_batch(pu_dpsk* h, const float* samples, size_t B, s
     PU_CUDA_TRY(cudaSetDevice(ctx->device));
     cudaStream_t st = pu::pick_stream(ctx, stream, space);
     if (space == PU_MEM_DEVICE) return dpsk_launch(h, samples, B, L, data_start, ref_mode, est_cfo_hz, phase_offset, llr_out, llr_stride, st, nullptr, nullptr);
-    return psk_host_call(ctx, st, samples, B, L, est_cfo_hz, phase_offset, llr_out, llr_stride, nullptr,
-                         [&](const float* din, size_t nb, const float* c, const float* p, float* dout, float*) {
-                             return dpsk_launch(h, din, nb, L, data_start, ref_mode, c, p, dout, llr_stride, st, nullptr, nullptr);
-                         });
+    pu::HostStage hs(ctx, st, B);
+    const float *d_x, *d_cfo, *d_phase;
+    float* d_llr;
+    hs.in(&d_x, samples, L);
+    hs.in(&d_cfo, est_cfo_hz, 1);
+    hs.in(&d_phase, phase_offset, 1);
+    hs.out(&d_llr, llr_out, llr_stride);
+    return hs.run([&](size_t nb) { return dpsk_launch(h, d_x, nb, L, data_start, ref_mode, d_cfo, d_phase, d_llr, llr_stride, st, nullptr, nullptr); });
 }
 
 pu_status pu_mcdpsk_create(pu_ctx* ctx, const pu_mcdpsk_config* cfg, pu_mcdpsk** out) {
@@ -843,10 +804,13 @@ pu_status pu_mcdpsk_demod_soft_batch(pu_mcdpsk* h, const float* samples, size_t 
     PU_CUDA_TRY(cudaSetDevice(ctx->device));
     cudaStream_t st = pu::pick_stream(ctx, stream, space);
     if (space == PU_MEM_DEVICE) return mcdpsk_launch(h, samples, B, L, llr_out, llr_stride, residual_cfo_hz, st);
-    return psk_host_call(ctx, st, samples, B, L, nullptr, nullptr, llr_out, llr_stride, residual_cfo_hz,
-                         [&](const float* din, size_t nb, const float*, const float*, float* dout, float* daux) {
-                             return mcdpsk_launch(h, din, nb, L, dout, llr_stride, residual_cfo_hz ? daux : nullptr, st);
-                         });
+    pu::HostStage hs(ctx, st, B);
+    const float* d_x;
+    float *d_llr, *d_res;
+    hs.in(&d_x, samples, L);
+    hs.out(&d_llr, llr_out, llr_stride);
+    hs.out(&d_res, residual_cfo_hz, 1);
+    return hs.run([&](size_t nb) { return mcdpsk_launch(h, d_x, nb, L, d_llr, llr_stride, d_res, st); });
 }
 
 // MultiCarrierDPSKDemodulator behind an externally detected chirp (MCDPSKWaveform::process, src/waveform/mc_dpsk_waveform.cpp:144-170:
@@ -856,7 +820,7 @@ static pu_status mcdpsk_got_chirp(pu_mcdpsk* h, const float* d_x, size_t B, size
                                   std::vector<float>& after_h, cudaStream_t st) {
     pu_ctx* ctx = h->ctx;
     const size_t pre = static_cast<size_t>(h->cfg.training_symbols + 1) * h->cfg.samples_per_symbol;
-    pu::PskDevMem dres;
+    pu::DevMem dres;
     pu_status s;
     std::vector<float> res(B, 0.0f), cfo_h(B);
     size_t Lmax = 0;                                     // longest per-frame span
@@ -885,10 +849,10 @@ static pu_status mcdpsk_got_chirp(pu_mcdpsk* h, const float* d_x, size_t B, size
         ctx->launches.fetch_add(1);
         PU_CUDA_TRY(cudaGetLastError());
         if ((s = mcdpsk_launch(h, dy, B, L, d_llr, llr_stride, static_cast<float*>(dres.p), st)) != PU_OK) return s;
-        PU_CUDA_TRY(cudaStreamSynchronize(st));
-        PU_CUDA_TRY(cudaMemcpy(res.data(), dres.p, B * sizeof(float), cudaMemcpyDeviceToHost));
+        PU_CUDA_TRY(cudaMemcpyAsync(res.data(), dres.p, B * sizeof(float), cudaMemcpyDeviceToHost, st));
     }
-    PU_CUDA_TRY(cudaMemcpy(cfo_h.data(), d_cfo, B * sizeof(float), cudaMemcpyDeviceToHost));
+    PU_CUDA_TRY(cudaMemcpyAsync(cfo_h.data(), d_cfo, B * sizeof(float), cudaMemcpyDeviceToHost, st));
+    PU_CUDA_TRY(cudaStreamSynchronize(st));
     // processTraining's cfo update and the false-positive rule (:572-607), per frame on the host: a handful of scalar operations
     const int nc = static_cast<int>(h->cfg.num_carriers), bits = static_cast<int>(h->cfg.bits_per_symbol), sps = static_cast<int>(h->cfg.samples_per_symbol);
     n_h.assign(B, 0);
@@ -918,29 +882,26 @@ pu_status pu_mcdpsk_got_chirp_batch(pu_mcdpsk* h, const float* samples, size_t B
     pu_ctx* ctx = h->ctx;
     PU_CUDA_TRY(cudaSetDevice(ctx->device));
     cudaStream_t st = pu::pick_stream(ctx, stream, space);
-    pu::PskDevMem dx, dcfo, dl;
-    pu_status s;
-    const float* d_x = samples;
-    const float* d_cfo = chirp_cfo_hz;
-    float* d_llr = llr_out;
     if (space == PU_MEM_HOST) {
-        std::vector<float> zf(B * llr_stride, 0.0f);
-        if ((s = dx.upload(samples, B * L)) != PU_OK) return s;
-        if ((s = dcfo.upload(chirp_cfo_hz, B)) != PU_OK) return s;
-        if ((s = dl.upload(zf.data(), zf.size())) != PU_OK) return s;
-        d_x = static_cast<const float*>(dx.p); d_cfo = static_cast<const float*>(dcfo.p); d_llr = static_cast<float*>(dl.p);
+        pu::HostStage hs(ctx, st, B);
+        const float *d_x, *d_cfo;
+        float *d_llr, *d_after;
+        int32_t* d_n;
+        hs.in(&d_x, samples, L);
+        hs.in(&d_cfo, chirp_cfo_hz, 1);
+        hs.out(&d_llr, llr_out, llr_stride);
+        hs.out(&d_n, n_llr, 1);
+        hs.out(&d_after, cfo_after_hz, 1);
+        return hs.run([&](size_t nb) {
+            return pu_mcdpsk_got_chirp_batch(h, d_x, nb, L, d_cfo, d_llr, llr_stride, d_n, d_after, PU_MEM_DEVICE, st);
+        });
     }
     std::vector<int32_t> n_h;
     std::vector<float> after_h;
-    if ((s = mcdpsk_got_chirp(h, d_x, B, L, d_cfo, nullptr, nullptr, d_llr, llr_stride, n_h, after_h, st)) != PU_OK) return s;
-    if (space == PU_MEM_HOST) {
-        PU_CUDA_TRY(cudaMemcpy(llr_out, d_llr, B * llr_stride * sizeof(float), cudaMemcpyDeviceToHost));
-        std::memcpy(n_llr, n_h.data(), B * sizeof(int32_t));
-        std::memcpy(cfo_after_hz, after_h.data(), B * sizeof(float));
-    } else {
-        PU_CUDA_TRY(cudaMemcpy(n_llr, n_h.data(), B * sizeof(int32_t), cudaMemcpyHostToDevice));
-        PU_CUDA_TRY(cudaMemcpy(cfo_after_hz, after_h.data(), B * sizeof(float), cudaMemcpyHostToDevice));
-    }
+    const pu_status s = mcdpsk_got_chirp(h, samples, B, L, chirp_cfo_hz, nullptr, nullptr, llr_out, llr_stride, n_h, after_h, st);
+    if (s != PU_OK) return s;
+    PU_CUDA_TRY(cudaMemcpyAsync(n_llr, n_h.data(), B * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    PU_CUDA_TRY(cudaMemcpyAsync(cfo_after_hz, after_h.data(), B * sizeof(float), cudaMemcpyHostToDevice, st));
     return PU_OK;
 }
 
@@ -966,25 +927,29 @@ pu_status pu_mcdpsk_chirp_receive_batch(pu_mcdpsk* h, const float* samples, size
     }
     cudaStream_t st = pu::pick_stream(ctx, stream, space);
     if (threshold <= 0.0f) threshold = 0.15f;        // the callers' value, tools/test_iwaveform.cpp:133
-    pu::PskDevMem dx, dl, dinfo, dval, dcfo, dstart;
-    const float* d_x = samples;
-    float* d_llr = llr_out;
+    if (space == PU_MEM_HOST) {
+        pu::HostStage hs(ctx, st, B);
+        const float* d_x;
+        float *d_val, *d_llr, *d_after;
+        int32_t *d_info, *d_n;
+        hs.in(&d_x, samples, L);
+        hs.out(&d_info, sync_info, 4);
+        hs.out(&d_val, sync_values, 4);
+        hs.out(&d_llr, llr_out, llr_stride);
+        hs.out(&d_n, llr_out ? n_llr : nullptr, 1);
+        hs.out(&d_after, llr_out ? cfo_after_hz : nullptr, 1);
+        return hs.run([&](size_t nb) {
+            return pu_mcdpsk_chirp_receive_batch(h, d_x, nb, L, threshold, d_llr, llr_stride, d_n, d_info, d_val, d_after, PU_MEM_DEVICE, st);
+        });
+    }
+    pu::DevMem dinfo, dval, dcfo, dstart;
     std::vector<int32_t> info_h(B * 4, 0);
     std::vector<float> val_h(B * 4, 0.0f);
-    if (space == PU_MEM_HOST) {
-        if ((s = dx.upload(samples, B * L)) != PU_OK) return s;
-        d_x = static_cast<const float*>(dx.p);
-        if (llr_out) {
-            std::vector<float> zf(B * llr_stride, 0.0f);
-            if ((s = dl.upload(zf.data(), zf.size())) != PU_OK) return s;
-            d_llr = static_cast<float*>(dl.p);
-        }
-    }
     if ((s = dinfo.upload(info_h.data(), info_h.size())) != PU_OK) return s;
     if ((s = dval.upload(val_h.data(), val_h.size())) != PU_OK) return s;
     if ((s = dcfo.upload(val_h.data(), B)) != PU_OK) return s;
     (void)cudaGetLastError();
-    PU_CUDA_TRY(pu::chirp_detect_launch(h->chirp, d_x, B, L, static_cast<int>(L), threshold, static_cast<int>(h->cfg.samples_per_symbol),
+    PU_CUDA_TRY(pu::chirp_detect_launch(h->chirp, samples, B, L, static_cast<int>(L), threshold, static_cast<int>(h->cfg.samples_per_symbol),
                                         static_cast<int4*>(dinfo.p), static_cast<float4*>(dval.p), nullptr, nullptr, static_cast<float*>(dcfo.p),
                                         nullptr, nullptr, 0, 0, st));
     ctx->launches.fetch_add(1);
@@ -1001,27 +966,16 @@ pu_status pu_mcdpsk_chirp_receive_batch(pu_mcdpsk* h, const float* samples, size
         val_h[4 * b + 3] = 0.0f;                       // no rotator phase on this path (the CFO is removed by the Hilbert-FIR shift)
         start_h[b] = (start >= 0 && static_cast<size_t>(start) < L) ? start : -1;
     }
-    if (space == PU_MEM_HOST) {
-        std::memcpy(sync_info, info_h.data(), info_h.size() * sizeof(int32_t));
-        std::memcpy(sync_values, val_h.data(), val_h.size() * sizeof(float));
-    } else {
-        PU_CUDA_TRY(cudaMemcpy(sync_info, info_h.data(), info_h.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
-        PU_CUDA_TRY(cudaMemcpy(sync_values, val_h.data(), val_h.size() * sizeof(float), cudaMemcpyHostToDevice));
-    }
+    PU_CUDA_TRY(cudaMemcpyAsync(sync_info, info_h.data(), info_h.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    PU_CUDA_TRY(cudaMemcpyAsync(sync_values, val_h.data(), val_h.size() * sizeof(float), cudaMemcpyHostToDevice, st));
     if (!llr_out) return PU_OK;                        // detection only (IWaveform::detectSync)
     if ((s = dstart.upload(start_h.data(), B)) != PU_OK) return s;
     std::vector<int32_t> n_h;
     std::vector<float> after_h;
-    if ((s = mcdpsk_got_chirp(h, d_x, B, L, static_cast<const float*>(dcfo.p), static_cast<const int*>(dstart.p), &start_h, d_llr, llr_stride,
+    if ((s = mcdpsk_got_chirp(h, samples, B, L, static_cast<const float*>(dcfo.p), static_cast<const int*>(dstart.p), &start_h, llr_out, llr_stride,
                               n_h, after_h, st)) != PU_OK) return s;
-    if (space == PU_MEM_HOST) {
-        PU_CUDA_TRY(cudaMemcpy(llr_out, d_llr, B * llr_stride * sizeof(float), cudaMemcpyDeviceToHost));
-        std::memcpy(n_llr, n_h.data(), B * sizeof(int32_t));
-        std::memcpy(cfo_after_hz, after_h.data(), B * sizeof(float));
-    } else {
-        PU_CUDA_TRY(cudaMemcpy(n_llr, n_h.data(), B * sizeof(int32_t), cudaMemcpyHostToDevice));
-        PU_CUDA_TRY(cudaMemcpy(cfo_after_hz, after_h.data(), B * sizeof(float), cudaMemcpyHostToDevice));
-    }
+    PU_CUDA_TRY(cudaMemcpyAsync(n_llr, n_h.data(), B * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    PU_CUDA_TRY(cudaMemcpyAsync(cfo_after_hz, after_h.data(), B * sizeof(float), cudaMemcpyHostToDevice, st));
     return PU_OK;
 }
 

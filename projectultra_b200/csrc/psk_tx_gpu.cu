@@ -242,22 +242,20 @@ pu_status pu_dpsk_tx_batch(pu_dpsk* h, const pu_ldpc* code, const uint8_t* paylo
     t.pulse = static_cast<const float*>(h->d_tx_pulse.p);
     cudaStream_t st = pu::pick_stream(ctx, stream, space);
     (void)cudaGetLastError();
-    if (space == PU_MEM_DEVICE) {
-        pu::dpsk_tx_kernel<<<static_cast<unsigned>(B), 256, 0, st>>>(t, payload, payload_stride, static_cast<int>(payload_bytes), peak, out, out_stride);
-        ctx->launches.fetch_add(1);
-        PU_CUDA_TRY(cudaGetLastError());
-        return PU_OK;
+    if (space == PU_MEM_HOST) {
+        // host memory: every output row comes back whole, zeros beyond *frame_len
+        pu::HostStage hs(ctx, st, B);
+        const uint8_t* d_payload;
+        float* d_tx;
+        hs.in(&d_payload, payload, payload_stride);
+        hs.out(&d_tx, out, out_stride);
+        return hs.run([&](size_t nb) {
+            return pu_dpsk_tx_batch(h, code, d_payload, payload_stride, payload_bytes, nb, peak, d_tx, out_stride, frame_len, PU_MEM_DEVICE, st);
+        });
     }
-    pu::PskDevMem dp, dout;
-    if ((s = dp.upload(payload, B * payload_stride)) != PU_OK) return s;
-    std::vector<float> z(B * out_stride, 0.0f);
-    if ((s = dout.upload(z.data(), z.size())) != PU_OK) return s;
-    pu::dpsk_tx_kernel<<<static_cast<unsigned>(B), 256, 0, st>>>(t, static_cast<const uint8_t*>(dp.p), payload_stride, static_cast<int>(payload_bytes), peak,
-                                                                 static_cast<float*>(dout.p), out_stride);
+    pu::dpsk_tx_kernel<<<static_cast<unsigned>(B), 256, 0, st>>>(t, payload, payload_stride, static_cast<int>(payload_bytes), peak, out, out_stride);
     ctx->launches.fetch_add(1);
     PU_CUDA_TRY(cudaGetLastError());
-    PU_CUDA_TRY(cudaStreamSynchronize(st));
-    PU_CUDA_TRY(cudaMemcpy(out, dout.p, B * out_stride * sizeof(float), cudaMemcpyDeviceToHost));
     return PU_OK;
 }
 
@@ -306,22 +304,20 @@ pu_status pu_mcdpsk_tx_batch(pu_mcdpsk* h, const pu_ldpc* code, const uint8_t* p
     const size_t smem = static_cast<size_t>(t.nsym) * t.nc * sizeof(float2);
     cudaStream_t st = pu::pick_stream(ctx, stream, space);
     (void)cudaGetLastError();
-    if (space == PU_MEM_DEVICE) {
-        pu::mcdpsk_tx_kernel<<<static_cast<unsigned>(B), 256, smem, st>>>(t, payload, payload_stride, static_cast<int>(payload_bytes), peak, out, out_stride);
-        ctx->launches.fetch_add(1);
-        PU_CUDA_TRY(cudaGetLastError());
-        return PU_OK;
+    if (space == PU_MEM_HOST) {
+        // host memory: every output row comes back whole, zeros beyond *frame_len
+        pu::HostStage hs(ctx, st, B);
+        const uint8_t* d_payload;
+        float* d_tx;
+        hs.in(&d_payload, payload, payload_stride);
+        hs.out(&d_tx, out, out_stride);
+        return hs.run([&](size_t nb) {
+            return pu_mcdpsk_tx_batch(h, code, d_payload, payload_stride, payload_bytes, nb, peak, d_tx, out_stride, frame_len, PU_MEM_DEVICE, st);
+        });
     }
-    pu::PskDevMem dp, dout;
-    if ((s = dp.upload(payload, B * payload_stride)) != PU_OK) return s;
-    std::vector<float> z(B * out_stride, 0.0f);
-    if ((s = dout.upload(z.data(), z.size())) != PU_OK) return s;
-    pu::mcdpsk_tx_kernel<<<static_cast<unsigned>(B), 256, smem, st>>>(t, static_cast<const uint8_t*>(dp.p), payload_stride, static_cast<int>(payload_bytes), peak,
-                                                                      static_cast<float*>(dout.p), out_stride);
+    pu::mcdpsk_tx_kernel<<<static_cast<unsigned>(B), 256, smem, st>>>(t, payload, payload_stride, static_cast<int>(payload_bytes), peak, out, out_stride);
     ctx->launches.fetch_add(1);
     PU_CUDA_TRY(cudaGetLastError());
-    PU_CUDA_TRY(cudaStreamSynchronize(st));
-    PU_CUDA_TRY(cudaMemcpy(out, dout.p, B * out_stride * sizeof(float), cudaMemcpyDeviceToHost));
     return PU_OK;
 }
 

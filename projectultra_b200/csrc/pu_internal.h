@@ -8,7 +8,9 @@
 #include <cstdint>
 #include <cstdio>
 #include <cstring>
+#include <functional>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "pu/pu_capi.h"
@@ -43,6 +45,64 @@ struct Buffer {
     void release();
 };
 
+// Device copy of a host table, owned by a handle and freed with it.
+struct DevMem {
+    void* p = nullptr;
+    DevMem() = default;
+    DevMem(const DevMem&) = delete;
+    DevMem& operator=(const DevMem&) = delete;
+    ~DevMem() { if (p) cudaFree(p); }
+    template <class T>
+    pu_status upload(const T* src, size_t n) {
+        if (p) { cudaFree(p); p = nullptr; }
+        PU_CUDA_TRY(cudaMalloc(&p, n * sizeof(T) > 16 ? n * sizeof(T) : 16));
+        if (n) {
+            // A pageable H2D cudaMemcpy may return once the source is staged, before the DMA has landed, and the kernels that
+            // read these tables run on NON-BLOCKING streams (no implicit ordering with the legacy stream): wait for it.
+            PU_CUDA_TRY(cudaMemcpy(p, src, n * sizeof(T), cudaMemcpyHostToDevice));
+            PU_CUDA_TRY(cudaStreamSynchronize(cudaStreamLegacy));
+        }
+        return PU_OK;
+    }
+};
+
+// The PU_MEM_HOST side of a batch entry point: the call declares its host arrays, each with the device pointer its body reads,
+// then run() moves the batch through the context's pinned and device staging buffers in slabs of whole rows.  Per slab: one packed
+// H2D copy, the body on device pointers (the entry point's PU_MEM_DEVICE path on `st`), one packed D2H copy, a synchronise of `st`.
+// Every staged array starts on a 256-byte boundary (the TMA paths check sample addresses); a NULL host array stays NULL.
+class HostStage {
+public:
+    HostStage(pu_ctx* ctx, cudaStream_t st, size_t B) : ctx_(ctx), st_(st), B_(B) {}
+    // per-row arrays: `row` elements of row b are read from / written to host + b * host_stride and packed on the device
+    template <class T> void in(const T** dev, const T* host, size_t row, size_t host_stride = 0) { add(kIn, dev, host, row, host_stride); }
+    // output rows come back as the body left them, zero-filled before it runs
+    template <class T> void out(T** dev, T* host, size_t row, size_t host_stride = 0) { add(kOut, dev, host, row, host_stride); }
+    // the caller's bytes go down and come back: in-place rows, or rows the body writes only in part
+    template <class T> void inout(T** dev, T* host, size_t row, size_t host_stride = 0) { add(kInOut, dev, host, row, host_stride); }
+    // one array of n elements for the whole call
+    template <class T> void whole(const T** dev, const T* host, size_t n) { add(kWhole, dev, host, n, n); }
+    // body(nb) runs on nb rows at the declared device pointers; B == 0 runs nothing
+    pu_status run(const std::function<pu_status(size_t nb)>& body);
+
+private:
+    enum Kind { kWhole, kIn, kInOut, kOut };   // the order of the staged layout: H2D covers [whole, inout], D2H [inout, out]
+    struct Array {
+        Kind kind;
+        std::function<void(void*)> bind;
+        char* host;
+        size_t row, stride, off;   // bytes
+    };
+    template <class P, class T>
+    void add(Kind k, P** dev, T* host, size_t row, size_t host_stride) {
+        arrays_.push_back({k, [dev](void* d) { *dev = static_cast<P*>(d); }, reinterpret_cast<char*>(const_cast<std::remove_const_t<T>*>(host)),
+                           row * sizeof(T), (host_stride ? host_stride : row) * sizeof(T), 0});
+    }
+    pu_ctx* ctx_;
+    cudaStream_t st_;
+    size_t B_;
+    std::vector<Array> arrays_;
+};
+
 }  // namespace pu
 
 namespace pu {
@@ -62,9 +122,9 @@ struct pu_ctx {
     cudaStream_t stream = nullptr;  // context-owned stream used when the caller passes NULL
     std::atomic<uint64_t> launches{0};
     std::atomic<uint64_t> h2d_bytes{0}, d2h_bytes{0};   // bytes moved by the host-buffer pipeline (pu_receive_decode_batch, PU_MEM_HOST)
-    // staging for PU_MEM_HOST calls
-    pu::Buffer d_in, d_out, d_aux, h_in, h_out;
-    pu::Buffer f_llr, f_bytes, f_ok, f_iters, f_out;   // scratch of pu_frame_decode_batch (grow-only, reused across calls)
+    pu::Buffer stage_dev, stage_host;                   // pu::HostStage: staging of PU_MEM_HOST calls
+    pu::Buffer d_aux;                                   // LLR scratch of pu_receive_decode_batch
+    pu::Buffer f_bytes, f_ok, f_iters;                  // scratch of pu_frame_decode_batch (grow-only, reused across calls)
     pu::PipeSlot pipe[2];
     cudaEvent_t pipe_ev = nullptr;
     // scratch of pu_linksim_run (sweep.cu), grow-only and reused across calls: [0..6] batch buffers (rx, llr, info, ok, iters, n_llr, sync),

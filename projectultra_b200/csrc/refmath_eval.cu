@@ -29,18 +29,16 @@ extern "C" pu_status pu_refmath_eval(pu_ctx* ctx, int op, const float* a, const 
         return PU_OK;
     }
     PU_CUDA_TRY(cudaSetDevice(ctx->device));
-    float *da = nullptr, *db = nullptr, *dout = nullptr;
-    PU_CUDA_TRY(cudaMalloc(&da, n * sizeof(float)));
-    PU_CUDA_TRY(cudaMalloc(&db, n * sizeof(float)));
-    PU_CUDA_TRY(cudaMalloc(&dout, n * sizeof(float)));
-    PU_CUDA_TRY(cudaMemcpy(da, a, n * sizeof(float), cudaMemcpyHostToDevice));
-    if (b) PU_CUDA_TRY(cudaMemcpy(db, b, n * sizeof(float), cudaMemcpyHostToDevice));
-    PU_CUDA_TRY(cudaStreamSynchronize(cudaStreamLegacy));   // pageable H2D: wait for the DMA before the non-blocking stream's kernel
-    pu::refmath_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, ctx->stream>>>(op, da, b ? db : nullptr, dout, n);
-    ctx->launches.fetch_add(1);
-    PU_CUDA_TRY(cudaGetLastError());
-    PU_CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-    PU_CUDA_TRY(cudaMemcpy(out, dout, n * sizeof(float), cudaMemcpyDeviceToHost));
-    cudaFree(da); cudaFree(db); cudaFree(dout);
-    return PU_OK;
+    pu::HostStage hs(ctx, ctx->stream, n);
+    const float *da, *db;
+    float* dout;
+    hs.in(&da, a, 1);
+    hs.in(&db, b, 1);
+    hs.out(&dout, out, 1);
+    return hs.run([&](size_t nb) -> pu_status {
+        pu::refmath_kernel<<<static_cast<unsigned>((nb + 255) / 256), 256, 0, ctx->stream>>>(op, da, db, dout, nb);
+        ctx->launches.fetch_add(1);
+        PU_CUDA_TRY(cudaGetLastError());
+        return PU_OK;
+    });
 }

@@ -886,23 +886,19 @@ pu_status pu_counters_allreduce(pu_ctx* ctx, uint64_t* counters, size_t n, void*
     PU_CUDA_TRY(cudaSetDevice(ctx->device));
     cudaStream_t st = pu::pick_stream(ctx, stream, space);
     constexpr int kNcclUint64 = 5, kNcclSum = 0;
-    uint64_t* dbuf = counters;
-    if (space == PU_MEM_HOST) {
-        pu_status s = ctx->d_aux.reserve(n * sizeof(uint64_t));
-        if (s != PU_OK) return s;
-        dbuf = static_cast<uint64_t*>(ctx->d_aux.ptr);
-        PU_CUDA_TRY(cudaMemcpyAsync(dbuf, counters, n * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
-    }
-    const int r = fn(dbuf, dbuf, n, kNcclUint64, kNcclSum, nccl_comm, st);
-    if (r != 0) {
-        pu::set_error("pu_counters_allreduce: ncclAllReduce failed with ncclResult_t %d", r);
-        return PU_ERR_CUDA;
-    }
-    if (space == PU_MEM_HOST) {
-        PU_CUDA_TRY(cudaMemcpyAsync(counters, dbuf, n * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-        PU_CUDA_TRY(cudaStreamSynchronize(st));
-    }
-    return PU_OK;
+    auto allreduce = [&](uint64_t* dbuf) -> pu_status {
+        const int r = fn(dbuf, dbuf, n, kNcclUint64, kNcclSum, nccl_comm, st);
+        if (r != 0) {
+            pu::set_error("pu_counters_allreduce: ncclAllReduce failed with ncclResult_t %d", r);
+            return PU_ERR_CUDA;
+        }
+        return PU_OK;
+    };
+    if (space == PU_MEM_DEVICE) return allreduce(counters);
+    pu::HostStage hs(ctx, st, 1);
+    uint64_t* dbuf;
+    hs.inout(&dbuf, counters, n);
+    return hs.run([&](size_t) { return allreduce(dbuf); });
 }
 
 }  // extern "C"

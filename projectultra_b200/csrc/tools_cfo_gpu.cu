@@ -159,8 +159,8 @@ struct pu_tools_cfo {
     int p = 0;                    // log2 of the transform size; 0: the call leaves rows untouched
     float scale = 0.0f;           // 1.0f / P, as the host evaluates it
     size_t chunk = 0;             // rows per pass of the two-pass schedule (scratch bound)
-    pu::Buffer tw, rot, s1, s2, staging;
-    ~pu_tools_cfo() { tw.release(); rot.release(); s1.release(); s2.release(); staging.release(); }
+    pu::Buffer tw, rot, s1, s2;
+    ~pu_tools_cfo() { tw.release(); rot.release(); s1.release(); s2.release(); }
 };
 
 namespace pu {
@@ -265,20 +265,11 @@ pu_status pu_tools_cfo_apply_batch(pu_tools_cfo* h, float* samples, size_t B, si
     PU_CUDA_TRY(cudaSetDevice(h->ctx->device));
     cudaStream_t st = pu::pick_stream(h->ctx, stream, space);
     if (space == PU_MEM_DEVICE) return pu::tools_cfo_rows(h, samples, B, stride, st);
-    // host rows: staged through the handle in pieces of at most 64 MiB; only the n samples of each row travel
-    const size_t n = h->n, rows = std::max<size_t>(1, pu::kScratchBytes / (n * sizeof(float)));
-    pu_status s = h->staging.reserve(std::min(rows, B) * n * sizeof(float));
-    if (s != PU_OK) return s;
-    float* d = static_cast<float*>(h->staging.ptr);
-    for (size_t b0 = 0; b0 < B; b0 += rows) {
-        const size_t nb = std::min(rows, B - b0);
-        float* hx = samples + b0 * stride;
-        PU_CUDA_TRY(cudaMemcpy2DAsync(d, n * sizeof(float), hx, stride * sizeof(float), n * sizeof(float), nb, cudaMemcpyHostToDevice, st));
-        if ((s = pu::tools_cfo_rows(h, d, nb, n, st)) != PU_OK) return s;
-        PU_CUDA_TRY(cudaMemcpy2DAsync(hx, stride * sizeof(float), d, n * sizeof(float), n * sizeof(float), nb, cudaMemcpyDeviceToHost, st));
-        PU_CUDA_TRY(cudaStreamSynchronize(st));
-    }
-    return PU_OK;
+    // host rows: only the n samples of each row travel
+    pu::HostStage hs(h->ctx, st, B);
+    float* d;
+    hs.inout(&d, samples, h->n, stride);
+    return hs.run([&](size_t nb) { return pu::tools_cfo_rows(h, d, nb, h->n, st); });
 }
 
 }  // extern "C"
