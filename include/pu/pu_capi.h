@@ -117,6 +117,12 @@ PU_API pu_status pu_channel_interleaver_perm(size_t bits_per_symbol, size_t tota
                                              uint32_t* inverse_perm, size_t* step);
 /* ultra::Interleaver (fec.hpp:85-107; ldpc_decoder.cpp:454-464): perm[i] = (i%cols)*rows + i/cols */
 PU_API pu_status pu_block_interleaver_perm(size_t rows, size_t cols, uint32_t* perm);
+/* ChannelInterleaver(bits_per_symbol, 648)::deinterleave on the soft bits of any receiver, the step RxPipeline takes between getSoftBits
+ * and decodeSoft, 648 soft bits at a time: IN PLACE on llr[b*llr_stride + c*648 .. + 648) for b < B and c < n_blocks, every block on
+ * its own (out[k] = in[k * step mod 648]).  n_blocks * 648 <= llr_stride; the columns beyond n_blocks * 648 are not written.  A block
+ * of zeros (an erasure) stays zeros.  PU_MEM_HOST stages the first n_blocks * 648 soft bits of every row (csrc/interleave.cu). */
+PU_API pu_status pu_llr_deinterleave_batch(pu_ctx* ctx, float* llr, size_t B, size_t llr_stride, size_t n_blocks,
+                                           size_t bits_per_symbol, pu_memspace space, void* stream);
 
 /* ---------------------------------------------------------------- OFDM demodulator (presynced path)
  * Replaces ultra::OFDMDemodulator (include/ultra/ofdm.hpp:58-127) on the externally-timed path that
@@ -155,6 +161,12 @@ PU_API int pu_ofdm_carrier_bins(const pu_ofdm* h, int32_t* bins, int cap);
 /* Fuse ChannelInterleaver(bits_per_symbol, total_bits)::deinterleave (ldpc_decoder.cpp:612-620) into the LLR
  * write address for the first total_bits LLRs of every frame; bits_per_symbol = 0 switches it off. */
 PU_API pu_status pu_ofdm_set_deinterleave(pu_ofdm* h, size_t bits_per_symbol, size_t total_bits);
+/* ChannelInterleaver(bits_per_symbol, 648)::interleave of every codeword in the transmitters of this handle: while it is set,
+ * pu_ofdm_tx_batch and pu_frame_tx_batch interleave each 648-bit codeword on its own after LDPC encoding and before mapping, i.e.
+ * transmitted bit j of a codeword is coded bit j * step^-1 mod 648 -- the waveform of pu_ofdm_tx on the interleaved bytes.
+ * bits_per_symbol = 0 (the default) switches it off.  The receivers of the handle are unaffected: deinterleave with
+ * pu_ofdm_set_deinterleave (first codeword, fused) or pu_llr_deinterleave_batch (any codeword), never both. */
+PU_API pu_status pu_ofdm_set_tx_interleave(pu_ofdm* h, size_t bits_per_symbol);
 /* B independent frames, each L samples starting at the first training symbol:
  *   samples [B][L]; cfo_hz[B] / cfo_phase[B] = arguments of setFrequencyOffsetWithPhase (demodulator.cpp:816-825),
  *   NULL meaning setFrequencyOffset(0) (:805-814);
@@ -352,6 +364,9 @@ PU_API pu_status pu_mcdpsk_tx(const pu_mcdpsk_config* cfg, const uint8_t* data, 
  * (multi_carrier_dpsk.hpp:118-243); bit-identical to pu_ldpc_encode + pu_mcdpsk_tx.  Arguments as pu_dpsk_tx_batch. */
 PU_API pu_status pu_mcdpsk_tx_batch(pu_mcdpsk* h, const pu_ldpc* code, const uint8_t* payload, size_t payload_stride, size_t payload_bytes,
                                     size_t B, float peak, float* out, size_t out_stride, size_t* frame_len, pu_memspace space, void* stream);
+/* As pu_ofdm_set_tx_interleave for pu_mcdpsk_tx_batch: the 648 coded bits are interleaved before the differential encoding; the zero
+ * padding of the last symbol is unchanged.  0 (the default) switches it off.  Deinterleave with pu_llr_deinterleave_batch. */
+PU_API pu_status pu_mcdpsk_set_tx_interleave(pu_mcdpsk* h, size_t bits_per_symbol);
 
 /* ---------------------------------------------------------------- channel simulator
  * Replaces sim::WattersonChannel (src/sim/hf_channel.hpp:34-299) for batches of frames.  POD mirror of
@@ -498,6 +513,12 @@ typedef struct {
                                  * src 0x123456, dst 0xABCDEF}: pool waveform i carries pu_sweep_payload(base_seed, mode, i) with seq i + 1,
                                  * a fresh frame the fresh payload bytes with seq = trial & 0xFFFF.  Acquired frames deliver
                                  * min(n_cw, soft bits / 648) codewords to the decoder.  payload_bytes is unused (0 allowed); 0 = codeword mode */
+    uint32_t interleave_bps;    /* > 0: ChannelInterleaver(interleave_bps, 648) on every codeword, as the reference's IWaveform path does
+                                 * (getSoftBits -> ChannelInterleaver::deinterleave -> decodeSoft): the pool interleaves each codeword's bytes
+                                 * before modulating them, fresh frames through pu_*_set_tx_interleave; the receiver deinterleaves
+                                 * (PU_WF_OFDM codewords: pu_ofdm_set_deinterleave, fused; everything else: pu_llr_deinterleave_batch on
+                                 * every codeword).  OFDM and MC-DPSK waveforms, codeword and frame modes; a nonzero value on PU_WF_DPSK /
+                                 * PU_WF_DPSK_ACQ makes the table invalid.  0 = no interleaving */
 } pu_sweep_mode;
 
 typedef struct {

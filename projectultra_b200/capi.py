@@ -330,6 +330,23 @@ def channel_interleaver_perm(bps, total=648):
     return perm, inv, step.value
 
 
+def llr_deinterleave_batch(ctx, llr, n_blocks, bps):
+    """pu_llr_deinterleave_batch: ChannelInterleaver(bps, 648)::deinterleave IN PLACE on the first n_blocks * 648 soft bits of every row
+    of llr [B, stride] (float32, rows contiguous; numpy => host, torch.cuda => device on torch's current stream), each 648-bit block on
+    its own.  Returns llr."""
+    if _is_torch(llr):
+        import torch
+        assert llr.dtype == torch.float32 and llr.dim() == 2 and llr.stride(1) == 1
+        B, stride = llr.shape[0], llr.stride(0)
+    else:
+        assert llr.dtype == np.float32 and llr.ndim == 2 and llr.strides[1] == 4 and llr.strides[0] % 4 == 0
+        B, stride = llr.shape[0], llr.strides[0] // 4
+    sp = _space(llr)
+    check(lib().pu_llr_deinterleave_batch(ctx._h, _ptr(llr), C.c_size_t(B), C.c_size_t(stride), C.c_size_t(n_blocks), C.c_size_t(bps),
+                                          sp, _stream(sp)))
+    return llr
+
+
 def block_interleaver_perm(rows, cols):
     perm = np.zeros(rows * cols, np.uint32)
     check(lib().pu_block_interleaver_perm(C.c_size_t(rows), C.c_size_t(cols), _ptr(perm)))
@@ -385,6 +402,10 @@ class OfdmDemodulator:
 
     def set_deinterleave(self, bits_per_symbol, total_bits=648):
         check(lib().pu_ofdm_set_deinterleave(self._h, C.c_size_t(bits_per_symbol), C.c_size_t(total_bits)))
+
+    def set_tx_interleave(self, bits_per_symbol):
+        """pu_ofdm_set_tx_interleave: ChannelInterleaver(bits_per_symbol, 648) on every codeword of tx_batch / frame_tx_batch; 0 = off."""
+        check(lib().pu_ofdm_set_tx_interleave(self._h, C.c_size_t(bits_per_symbol)))
 
     def n_llr(self, L, training=2):
         return max(0, L // self.symbol_samples - training) * self.bits_per_symbol
@@ -771,6 +792,10 @@ class McDpskDemodulator:
         """pu_mcdpsk_tx_batch: LDPC encode + training + reference + MC-DPSK modulate for every row of payload [B, bytes] on the GPU."""
         return _psk_tx_batch(lib().pu_mcdpsk_tx_batch, self._h, ldpc, payload, peak, out)
 
+    def set_tx_interleave(self, bits_per_symbol):
+        """pu_mcdpsk_set_tx_interleave: ChannelInterleaver(bits_per_symbol, 648) on the codeword of tx_batch; 0 = off."""
+        check(lib().pu_mcdpsk_set_tx_interleave(self._h, C.c_size_t(bits_per_symbol)))
+
     def n_llr(self, L):
         c = self.cfg
         return max(0, L // c.samples_per_symbol - c.training_symbols - 1) * c.num_carriers * c.bits_per_symbol
@@ -844,7 +869,7 @@ class SweepMode(C.Structure):
                 ("code_rate", C.c_uint32), ("payload_bytes", C.c_uint32), ("channel", C.c_uint32), ("n_snr", C.c_uint32),
                 ("snr_first_db", C.c_float), ("snr_step_db", C.c_float), ("peak", C.c_float), ("precision", C.c_uint32),
                 ("chunk", C.c_uint32), ("cost", C.c_float), ("lead_samples", C.c_uint32), ("tail_samples", C.c_uint32),
-                ("cfo_hz", C.c_float), ("fresh_payloads", C.c_uint32), ("frame_payload_bytes", C.c_uint32)]
+                ("cfo_hz", C.c_float), ("fresh_payloads", C.c_uint32), ("frame_payload_bytes", C.c_uint32), ("interleave_bps", C.c_uint32)]
 
     @property
     def snr_points(self):
@@ -865,9 +890,10 @@ class SweepStats(C.Structure):
 
 
 def sweep_mode(waveform, cfg, code_rate, payload_bytes, channel, snr_first, snr_step, n_snr, peak=0.0, precision="exact", chunk=0, cost=0.0,
-               lead_samples=0, tail_samples=0, cfo_hz=0.0, fresh_payloads=False, frame_payload_bytes=0):
+               lead_samples=0, tail_samples=0, cfo_hz=0.0, fresh_payloads=False, frame_payload_bytes=0, interleave_bps=0):
     """One pu_sweep_mode.  frame_payload_bytes > 0 makes every trial a protocol-v2 DATA frame of that many payload bytes (OFDM waveforms;
-    payload_bytes is then unused) with whole-frame counters (linksim.FRAME_COUNTER_NAMES)."""
+    payload_bytes is then unused) with whole-frame counters (linksim.FRAME_COUNTER_NAMES).  interleave_bps > 0 passes every codeword
+    through ChannelInterleaver(interleave_bps, 648) (OFDM and MC-DPSK waveforms)."""
     m = SweepMode()
     m.waveform = waveform
     if isinstance(cfg, ModemConfig):
@@ -881,6 +907,7 @@ def sweep_mode(waveform, cfg, code_rate, payload_bytes, channel, snr_first, snr_
     m.precision, m.chunk, m.cost = {"exact": 0, "fast": 1}[precision], int(chunk), float(cost)
     m.lead_samples, m.tail_samples, m.cfo_hz, m.fresh_payloads = int(lead_samples), int(tail_samples), float(cfo_hz), int(bool(fresh_payloads))
     m.frame_payload_bytes = int(frame_payload_bytes)
+    m.interleave_bps = int(interleave_bps)
     return m
 
 

@@ -608,6 +608,36 @@ pu_status pu_channel_interleaver_perm(size_t bps, size_t total, uint32_t* perm, 
     return PU_OK;
 }
 
+}  // extern "C"
+
+namespace pu {
+
+uint32_t channel_interleaver_inverse_step(size_t bits_per_symbol) {
+    size_t step = 0;
+    pu_channel_interleaver_perm(bits_per_symbol, PU_LDPC_N, nullptr, nullptr, &step);
+    for (uint32_t x = 1; x < PU_LDPC_N; ++x)
+        if (step * x % PU_LDPC_N == 1) return x;
+    return 0;      // unreachable: the step is coprime with 648
+}
+
+void channel_interleave_codewords(size_t bits_per_symbol, uint8_t* coded, size_t n_cw) {
+    const uint32_t inv = channel_interleaver_inverse_step(bits_per_symbol);
+    uint8_t cw[PU_LDPC_N / 8];
+    for (size_t c = 0; c < n_cw; ++c) {
+        uint8_t* in = coded + c * (PU_LDPC_N / 8);
+        std::memset(cw, 0, sizeof cw);
+        for (uint32_t j = 0; j < PU_LDPC_N; ++j) {      // out[perm[i]] = in[i]: bit j is coded bit j * step^-1
+            const uint32_t i = j * inv % PU_LDPC_N;
+            cw[j >> 3] |= static_cast<uint8_t>(((in[i >> 3] >> (7 - (i & 7))) & 1u) << (7 - (j & 7)));
+        }
+        std::memcpy(in, cw, sizeof cw);
+    }
+}
+
+}  // namespace pu
+
+extern "C" {
+
 pu_status pu_block_interleaver_perm(size_t rows, size_t cols, uint32_t* perm) {
     PU_REQUIRE(perm && rows && cols, "pu_block_interleaver_perm: bad argument");
     for (size_t i = 0; i < rows * cols; ++i) perm[i] = static_cast<uint32_t>((i % cols) * rows + i / cols);

@@ -991,6 +991,7 @@ struct TxDev {
     int pre_len, n_sym, frame_len;
     int osc_start;
     float scale;
+    int il_inv;
     const uint8_t* cn_ninfo;
     const uint16_t* cn_check;
     const uint16_t* cn_var;
@@ -1089,6 +1090,7 @@ struct pu_ofdm {
     pu::DevMem d_tx_osc, d_tx_pre[2], d_tx_points;   // transmitter tables (built on first use; preamble per layout)
     int tx_pre_len[2] = {-1, -1};
     size_t tx_osc_len = 0;
+    int tx_il_inv = 0;                               // pu_ofdm_set_tx_interleave (TxDev::il_inv)
     pu::AcqDev acq{};
     bool acq_ready = false;
 
@@ -1261,6 +1263,12 @@ pu_status pu_ofdm_set_deinterleave(pu_ofdm* h, size_t bits_per_symbol, size_t to
     if ((s = h->d_perm.upload(dst.data(), dst.size())) != PU_OK) return s;
     h->dev.llr_perm = static_cast<const int*>(h->d_perm.p);
     h->dev.perm_len = static_cast<int>(total_bits);
+    return PU_OK;
+}
+
+pu_status pu_ofdm_set_tx_interleave(pu_ofdm* h, size_t bits_per_symbol) {
+    PU_REQUIRE(h, "pu_ofdm_set_tx_interleave: NULL handle");
+    h->tx_il_inv = bits_per_symbol ? static_cast<int>(pu::channel_interleaver_inverse_step(bits_per_symbol)) : 0;
     return PU_OK;
 }
 
@@ -1533,6 +1541,7 @@ pu_status ofdm_tx_frames(pu_ofdm* h, const pu_ldpc* code, const uint8_t* frames,
     t.nfft = p.nfft; t.cp = p.cp; t.sym_len = p.sym_len; t.guard = static_cast<int>(p.cfg.symbol_guard);
     t.n_data = p.n_data; t.n_pilot = p.n_pilot; t.bps = p.bps; t.differential = pu::is_differential(p.cfg.modulation) ? 1 : 0;
     t.scale = p.cfg.output_scale;
+    t.il_inv = h->tx_il_inv;
     t.data_bin = static_cast<const int*>(h->d_dbin.p); t.pilot_bin = static_cast<const int*>(h->d_pbin.p);
     t.pilot_sign = static_cast<const float*>(h->d_psign.p); t.twiddle = static_cast<const float2*>(h->d_tw.p);
     t.osc = static_cast<const float2*>(h->d_tx_osc.p); t.preamble = static_cast<const float*>(h->d_tx_pre[layout].p);

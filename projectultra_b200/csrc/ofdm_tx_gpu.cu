@@ -28,6 +28,8 @@ struct TxDev {
     int osc_start;                     // mixer position of the first data symbol (the Schmidl-Cox preamble repeats one STS and one
                                        // LTS waveform, so the mixer has only advanced by two symbols there: modulator.cpp:479-532)
     float scale;                       // ModemConfig::output_scale
+    int il_inv;                        // pu_ofdm_set_tx_interleave: step^-1 mod 648 of ChannelInterleaver (bit j of a codeword is coded
+                                       // bit j * il_inv mod 648), 0 = no interleaving
     const uint8_t* cn_ninfo;           // LDPC tables in slot order (ldpc_code.h: LdpcHostTables)
     const uint16_t* cn_check;
     const uint16_t* cn_var;
@@ -109,7 +111,11 @@ __global__ void __launch_bounds__(128) ofdm_tx_kernel(TxDev t, const uint8_t* __
             if (b0 < total_bits) {                        // a carrier exists while data remains at its first bit (:418-436)
                 unsigned v = 0;
                 for (int b = 0; b < t.bps; ++b) {
-                    const int bit = b0 + b;
+                    int bit = b0 + b;
+                    if (t.il_inv && bit < total_bits) {   // the codeword's own ChannelInterleaver: the coded bytes stay as encoded
+                        const int c = bit / PU_LDPC_N;
+                        bit = c * PU_LDPC_N + (bit - c * PU_LDPC_N) * t.il_inv % PU_LDPC_N;
+                    }
                     v = (v << 1) | ((bit < total_bits) ? ((coded[bit >> 3] >> (7 - (bit & 7))) & 1u) : 0u);
                 }
                 float2 sym = __ldg(&t.points[v]);

@@ -30,5 +30,6 @@ struct pu_mcdpsk {
     // batched transmitter (psk_tx_gpu.cu), built on first use: training + reference symbols, polar(1, i * inc_c) per (carrier, sample)
     pu::DevMem d_tx_pre, d_tx_polar;
     size_t tx_pre_len = 0;
+    int tx_il_inv = 0;         // pu_mcdpsk_set_tx_interleave: step^-1 mod 648 of ChannelInterleaver, 0 = no interleaving
 };
 

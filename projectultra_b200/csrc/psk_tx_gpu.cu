@@ -113,6 +113,7 @@ __global__ void __launch_bounds__(256) dpsk_tx_kernel(DpskTxDev t, const uint8_t
 struct McTxDev {
     LdpcEncDev enc;
     int nc, sps, bits_c, nsym, pre_len, frame_len;
+    int il_inv;                  // pu_mcdpsk_set_tx_interleave: coded bit j * il_inv mod 648 goes out as bit j; 0 = no interleaving
     float2 change[4];            // std::polar(1.0f, phase change of symbol value v), multi_carrier_dpsk.hpp:198-214
     const float* preamble;       // [pre_len] training sequence + reference symbol
     const float2* polar;         // [nc][sps] std::polar(1.0f, i * inc_c)
@@ -140,7 +141,7 @@ __global__ void __launch_bounds__(256) mcdpsk_tx_kernel(McTxDev t, const uint8_t
             int v = 0;
             for (int b = 0; b < t.bits_c; ++b) {
                 const int pos = (s * t.nc + tid) * t.bits_c + b;
-                v = (v << 1) | (pos < PU_LDPC_N ? bits[pos] : 0);     // zero padding of the last symbol (:186-188)
+                v = (v << 1) | (pos < PU_LDPC_N ? bits[t.il_inv ? pos * t.il_inv % PU_LDPC_N : pos] : 0);   // zero padding of the last symbol (:186-188)
             }
             float2 c = cmul(prev, t.change[v]);
             c = cdivs(c, cabs_ref(c));
@@ -301,6 +302,7 @@ pu_status pu_mcdpsk_tx_batch(pu_mcdpsk* h, const pu_ldpc* code, const uint8_t* p
     }
     t.preamble = static_cast<const float*>(h->d_tx_pre.p);
     t.polar = static_cast<const float2*>(h->d_tx_polar.p);
+    t.il_inv = h->tx_il_inv;
     const size_t smem = static_cast<size_t>(t.nsym) * t.nc * sizeof(float2);
     cudaStream_t st = pu::pick_stream(ctx, stream, space);
     (void)cudaGetLastError();
@@ -318,6 +320,12 @@ pu_status pu_mcdpsk_tx_batch(pu_mcdpsk* h, const pu_ldpc* code, const uint8_t* p
     pu::mcdpsk_tx_kernel<<<static_cast<unsigned>(B), 256, smem, st>>>(t, payload, payload_stride, static_cast<int>(payload_bytes), peak, out, out_stride);
     ctx->launches.fetch_add(1);
     PU_CUDA_TRY(cudaGetLastError());
+    return PU_OK;
+}
+
+pu_status pu_mcdpsk_set_tx_interleave(pu_mcdpsk* h, size_t bits_per_symbol) {
+    PU_REQUIRE(h, "pu_mcdpsk_set_tx_interleave: NULL handle");
+    h->tx_il_inv = bits_per_symbol ? static_cast<int>(pu::channel_interleaver_inverse_step(bits_per_symbol)) : 0;
     return PU_OK;
 }
 

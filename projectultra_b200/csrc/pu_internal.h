@@ -184,6 +184,13 @@ pu_status frame_decode_enqueue(pu_ctx* ctx, pu_ldpc* dec, const float* llr, size
 pu_status count_frame_errors(pu_ctx* ctx, const uint8_t* frame_out, size_t frame_cap, const int32_t* frame_len, const int32_t* info,
                              const uint8_t* sent, size_t sent_stride, const uint32_t* tx_index, const uint32_t* bin, size_t sent_len, int n_cw,
                              size_t B, uint64_t* counters, cudaStream_t st);
+// ldpc_decode.cu: ChannelInterleaver(bits_per_symbol, 648) of pu_channel_interleaver_perm, perm[i] = i * step mod 648.  The inverse of
+// step mod 648 (transmitted bit j of a codeword is coded bit j * step^-1 mod 648), and ChannelInterleaver::interleave of n_cw packed
+// 81-byte codewords in place, each on its own.
+uint32_t channel_interleaver_inverse_step(size_t bits_per_symbol);
+void channel_interleave_codewords(size_t bits_per_symbol, uint8_t* coded, size_t n_cw);
+// interleave.cu: the body of pu_llr_deinterleave_batch on device pointers, enqueue only
+pu_status llr_deinterleave_enqueue(pu_ctx* ctx, float* llr, size_t B, size_t llr_stride, size_t n_blocks, size_t bits_per_symbol, cudaStream_t st);
 float channel_power_sum(const float* tx, size_t L);                                   // channel.cu: the two halves of pu_channel_noise_std
 float channel_noise_std_from_sum(float acc, size_t L, float snr_db, int convention);
 cudaError_t chirp_search_stats(unsigned long long* out);

@@ -17,6 +17,7 @@
 #include <algorithm>
 #include <chrono>
 #include <cmath>
+#include <cstddef>
 #include <cstdio>
 #include <cstdlib>
 #include <memory>
@@ -76,6 +77,8 @@ bool make_plan(const pu_sweep_desc* d, SweepPlan* p) {
     for (uint32_t m = 0; m < d->n_modes; ++m) {
         const pu_sweep_mode& md = d->modes[m];
         if (md.n_snr == 0 || md.n_snr > 255 || md.waveform > PU_WF_MCDPSK_CHIRP || md.channel > PU_CH_ITU_FLUTTER) return false;
+        // ChannelInterleaver rides on the IWaveform path (OFDM, MC-DPSK); single-carrier DPSK has no interleaver in the reference
+        if (md.interleave_bps && (md.waveform == PU_WF_DPSK || md.waveform == PU_WF_DPSK_ACQ)) return false;
         uint32_t ncw;
         double scale;
         if (!frame_mode_shape(md, &ncw, &scale)) return false;
@@ -144,7 +147,9 @@ uint64_t desc_key(const pu_sweep_desc* d, const SweepPlan& p) {      // FNV-1a o
     for (uint32_t m = 0; m < d->n_modes; ++m) {
         pu_sweep_mode md = d->modes[m];
         md.cost = 0;             // the partitioner's weights do not change what a unit computes
-        mix(&md, sizeof md);
+        // fields appended to the mode enter the key only when set: a table without them keeps the key -- and the manifests -- it had
+        mix(&md, offsetof(pu_sweep_mode, interleave_bps));
+        if (md.interleave_bps) mix(&md.interleave_bps, sizeof md.interleave_bps);
     }
     mix(&p.pool, sizeof p.pool); mix(&p.block, sizeof p.block); mix(&p.max_iter, sizeof p.max_iter);
     mix(&p.base_seed, sizeof p.base_seed); mix(&p.trials, sizeof p.trials);
@@ -243,6 +248,7 @@ struct ModeEngine {
     uint32_t n_cw = 1;                   // codewords per trial
     size_t frame_bytes = 0;              // frame modes: bytes of the DATA frame (payload + 19)
     size_t pay_stride = 0;               // bytes per row of d_payload / the fresh payload rows: kb, or frame_bytes in frame modes
+    bool deinterleave = false;           // pu_sweep_mode.interleave_bps on a receiver without the fused table: pu_llr_deinterleave_batch
 
     ~ModeEngine() {
         if (ofdm) pu_ofdm_destroy(ofdm);
@@ -283,6 +289,12 @@ struct ModeEngine {
             if ((s = pu_dpsk_create(c, &m->dpsk, &dpsk)) != PU_OK) return s;
         } else {
             if ((s = pu_mcdpsk_create(c, &m->mcdpsk, &mcd)) != PU_OK) return s;
+        }
+        if (m->interleave_bps) {
+            // one deinterleaver per handle: the fused table of the presynced receiver only holds the first codeword of a row
+            if (m->waveform != PU_WF_OFDM || frames) deinterleave = true;
+            else if ((s = pu_ofdm_set_deinterleave(ofdm, m->interleave_bps, PU_LDPC_N)) != PU_OK) return s;
+            if ((s = ofdm ? pu_ofdm_set_tx_interleave(ofdm, m->interleave_bps) : pu_mcdpsk_set_tx_interleave(mcd, m->interleave_bps)) != PU_OK) return s;
         }
         const auto t1 = now();
         const float fs = is_ofdm ? static_cast<float>(m->ofdm.sample_rate) : is_dpsk ? m->dpsk.sample_rate : m->mcdpsk.sample_rate;
@@ -330,6 +342,7 @@ struct ModeEngine {
                 pu_sweep_payload(p.base_seed, mode_index, i, pay, m->payload_bytes);
                 if ((s = pu_ldpc_encode(static_cast<int>(m->code_rate), pay, m->payload_bytes, coded.data(), coded.size(), &nc)) != PU_OK) return s;
             }
+            if (m->interleave_bps) channel_interleave_codewords(m->interleave_bps, coded.data(), nc / (PU_LDPC_N / 8));
             size_t n = 0;
             std::vector<float> w;
             auto tx = [&](float* out, size_t cap, size_t* len) -> pu_status {
@@ -425,6 +438,7 @@ struct ModeEngine {
             ctx->launches.fetch_add(1);
             PU_CUDA_TRY(cudaGetLastError());
         }
+        if (deinterleave && (s = llr_deinterleave_enqueue(ctx, llr, B, stride, n_cw, md->interleave_bps, st)) != PU_OK) return s;
         return frame_decode_enqueue(ctx, ldpc, llr, B, static_cast<int>(n_cw), ncw, cw_bytes, cw_ok, cw_iters, frame_out, frame_bytes, frame_len, info, st);
     }
 
@@ -458,6 +472,7 @@ struct ModeEngine {
                 mask = true; break;
         }
         if (s != PU_OK) return s;
+        if (deinterleave && (s = llr_deinterleave_enqueue(ctx, llr, B, PU_LDPC_N, 1, md->interleave_bps, st)) != PU_OK) return s;
         if ((s = pu_ldpc_decode_batch(ldpc, llr, PU_LDPC_N, B, info, kb, ok, iters, PU_MEM_DEVICE, st)) != PU_OK) return s;
         if (mask) {
             mask_short_kernel<<<static_cast<unsigned>((B + 255) / 256), 256, 0, st>>>(ok, n_llr, B);

@@ -111,6 +111,16 @@ def count_errors(ctx, info, ok, iters, payload_pool, tx_index, bins, payload_byt
     return counters
 
 
+def interleave_codewords(coded, bps):
+    """ChannelInterleaver(bps, 648)::interleave (out[perm[i]] = in[i], bits MSB first) of every 81-byte codeword of `coded`, each on its own,
+    as the reference's IWaveform transmitters do before modulating."""
+    perm = capi.channel_interleaver_perm(bps)[0]
+    bits = np.unpackbits(np.ascontiguousarray(coded, np.uint8).reshape(-1, 81), axis=1)
+    out = np.zeros_like(bits)
+    out[:, perm] = bits
+    return np.packbits(out, axis=1).reshape(-1)
+
+
 def wilson_interval(errors, n, z=1.96):
     """Wilson score interval for an error rate (the Monte-Carlo confidence interval of the north star)."""
     if n == 0:
@@ -132,6 +142,9 @@ class LinkSim:
     (tools/test_iwaveform.cpp:501-506) to every clean TX waveform after it: capi.tools_apply_cfo on the pool, capi.ToolsCfo on fresh frames.
     lead_samples / tail_samples (layout 'chirp') surround every frame with silence before both, as the tools do (test_iwaveform.cpp:396-459):
     a positive tuning error moves the up chirp's apparent start in front of the frame, so without a lead the chirp's timing is lost.
+    interleave_bps > 0 (OFDM and MC-DPSK) passes every codeword through ChannelInterleaver(interleave_bps, 648) as the sweep driver does
+    (pu_sweep_mode.interleave_bps): the pool interleaves the coded bytes, fresh frames the transmitter (set_tx_interleave); the presynced
+    OFDM receiver deinterleaves in its LLR write (set_deinterleave), every other receiver through capi.llr_deinterleave_batch.
 
     Frames are identified by (snr index, trial index); frame -> (tx waveform, seed) is a pure function, so any
     frame can be regenerated, and ranks take disjoint trial ranges with no data exchange (SURVEY §8e)."""
@@ -139,7 +152,7 @@ class LinkSim:
     def __init__(self, ctx, cfg, channel="awgn", payload_bytes=40, pool=64, snr_convention=None, pool_seed=12345,
                  max_iter=50, device=None, code_rate=None, peak=None, layout="presynced", chunk=960, fresh_payload=False,
                  acquire=False, precision="exact", payloads=None, tools_cfo_hz=0.0,
-                 lead_samples=0, tail_samples=0):
+                 lead_samples=0, tail_samples=0, interleave_bps=0):
         import torch
         self.ctx, self.cfg = ctx, cfg
         self.precision = precision
@@ -198,6 +211,12 @@ class LinkSim:
         self.acquire = bool(acquire)
         assert not self.acquire or self.kind == "dpsk", "acquire=True is the DPSK Barker path; OFDM uses layout='sc'"
         self.fresh_payload = bool(fresh_payload)
+        self.interleave_bps = int(interleave_bps)
+        assert not self.interleave_bps or self.kind != "dpsk", "single-carrier DPSK has no ChannelInterleaver in the reference"
+        if self.interleave_bps:
+            self.demod.set_tx_interleave(self.interleave_bps)
+            if self.kind == "ofdm" and self.layout == "presynced":
+                self.ofdm.set_deinterleave(self.interleave_bps, 648)
         self.peak = peak
         self.chirp = None if chirp is None else torch.from_numpy(chirp).to(self.device)
         self.sample_rate = float(cfg.sample_rate)
@@ -210,7 +229,10 @@ class LinkSim:
         # payloads: explicit [pool, payload_bytes] array (e.g. the splitmix64 pool of the C++ sweep driver, capi.Sweep.payload)
         self.payloads = (rng.integers(0, 256, (pool, payload_bytes), dtype=np.uint8) if payloads is None
                          else np.ascontiguousarray(payloads, dtype=np.uint8).reshape(pool, payload_bytes))
-        waves = [np.pad(build(capi.ldpc_encode(rate, p)), (self.lead, self.tail)) for p in self.payloads]
+        coded = [capi.ldpc_encode(rate, p) for p in self.payloads]
+        if self.interleave_bps:
+            coded = [interleave_codewords(c, self.interleave_bps) for c in coded]
+        waves = [np.pad(build(c), (self.lead, self.tail)) for c in coded]
         if peak is not None:
             waves = [(w * (np.float32(peak) / np.abs(w).max())).astype(np.float32) for w in waves]
         if self.tools_cfo_hz != 0.0:
@@ -225,7 +247,13 @@ class LinkSim:
         self.pool = pool
 
     def demod_llr(self, rx, llr=None):
-        """First 648 soft bits of every frame (device tensors), as the tools consume them."""
+        """First 648 soft bits of every frame (device tensors), as the tools consume them, in the decoder's order."""
+        out = self._receiver_llr(rx, llr)
+        if self.interleave_bps and not (self.kind == "ofdm" and self.layout == "presynced"):     # that one deinterleaves in its kernel
+            capi.llr_deinterleave_batch(self.ctx, out, 1, self.interleave_bps)
+        return out
+
+    def _receiver_llr(self, rx, llr=None):
         if self.kind == "ofdm" and self.layout == "sc":
             out = self.demod.process_batch(rx, chunk=self.chunk, llr_stride=648)
             self.last_n_llr, self.last_sync = out[1], out[2]
@@ -422,12 +450,18 @@ class FrameLinkSim:
         codewords of the frame, llr_stride = n_cw * 648) -> pu_frame_decode_batch -> compare with the frame sent -> counters
 
     counters [n_snr, 6] = FRAME_COUNTER_NAMES.  payloads: explicit [pool, payload_bytes] array (e.g. the sweep driver's pool,
-    capi.Sweep.payload; frame i then carries seq i + 1 as there); peak: the tools' peak normalisation of every TX waveform."""
+    capi.Sweep.payload; frame i then carries seq i + 1 as there); peak: the tools' peak normalisation of every TX waveform; interleave_bps > 0:
+    ChannelInterleaver(interleave_bps, 648) on every codeword (interleave_codewords before modulating, capi.llr_deinterleave_batch on the
+    soft bits of all codewords before decodeFrame), as the sweep driver's frame modes do."""
 
     def __init__(self, ctx, cfg, channel="awgn", payload_bytes=200, pool=16, pool_seed=12345, max_iter=50, precision="exact", code_rate=None,
-                 payloads=None, peak=None):
+                 payloads=None, peak=None, interleave_bps=0, layout="presynced", lead_samples=0, tail_samples=0):
         import torch
         assert isinstance(cfg, capi.ModemConfig), "whole frames ride on the OFDM waveforms"
+        # layout "chirp": ChirpSync::generate() + training + data behind lead_samples of silence and ahead of tail_samples, received through
+        # pu_ofdm_chirp_receive_batch; decodeFrame gets the whole codewords of soft bits the receiver delivered (the sweep driver's rule)
+        assert layout in ("presynced", "chirp") and (layout == "chirp" or not (lead_samples or tail_samples))
+        self.layout = layout
         self.ctx, self.cfg = ctx, cfg
         self.device = torch.device("cuda", ctx.device)
         self.ch = channel_preset(channel) if isinstance(channel, str) else channel
@@ -443,14 +477,20 @@ class FrameLinkSim:
             payloads = np.ascontiguousarray(payloads, dtype=np.uint8).reshape(pool, payload_bytes)
         self.frames_host = [v2_data_frame(payloads[i], self.rate, seq=i + 1) for i in range(pool)]
         cws = [capi.frame_encode(self.rate, f) for f in self.frames_host]
+        self.interleave_bps = int(interleave_bps)
+        if self.interleave_bps:
+            cws = [interleave_codewords(c, self.interleave_bps).reshape(c.shape) for c in cws]
         self.n_cw = len(cws[0])
         assert all(len(c) == self.n_cw for c in cws)
         waves = [ofdm_tx(cfg, c.reshape(-1), 0) for c in cws]
+        if layout == "chirp":
+            chirp = capi.chirp_generate(float(cfg.sample_rate), float(cfg.tx_cfo_hz))
+            waves = [np.pad(np.concatenate([chirp, w]), (int(lead_samples), int(tail_samples))) for w in waves]
         if peak is not None:
             waves = [(w * (np.float32(peak) / np.abs(w).max())).astype(np.float32) for w in waves]
         self.tx_host = np.stack(waves)
         self.L = self.tx_host.shape[1]
-        assert self.ofdm.n_llr(self.L) >= self.n_cw * 648
+        assert layout == "chirp" or self.ofdm.n_llr(self.L) >= self.n_cw * 648
         self.tx_pool = torch.from_numpy(self.tx_host).to(self.device)
         self.frame_len = len(self.frames_host[0])
         self.frame_pool = torch.from_numpy(np.stack(self.frames_host)).to(self.device)
@@ -472,10 +512,25 @@ class FrameLinkSim:
         """channel -> demod (every codeword of the frame) -> decodeFrame -> counters, on the current stream."""
         import torch
         rx = channel_apply(self.ctx, self.ch, self.tx_pool, batch["tx_index"], batch["noise_std"], batch["seed"])
-        llr = self.ofdm.presynced_batch(rx, 2, llr_stride=self.n_cw * 648, want_aux=False)[0]
+        if self.layout == "chirp":
+            llr, n_llr = self.ofdm.chirp_receive_batch(rx, llr_stride=self.n_cw * 648)[:2]
+        else:
+            llr = self.ofdm.presynced_batch(rx, 2, llr_stride=self.n_cw * 648, want_aux=False)[0]
+        if self.interleave_bps:
+            capi.llr_deinterleave_batch(self.ctx, llr, self.n_cw, self.interleave_bps)
         frames, flen, info = self.ldpc.frame_decode_batch(llr, self.n_cw, frame_cap=self.frame_len)
         want = self.frame_pool[batch["tx_index"].long()]
         good = (info[:, 0] == 1) & (flen == self.frame_len) & (frames == want).all(dim=1)
+        if self.layout == "chirp":
+            # decodeFrame(soft_bits, num_codewords) with fewer codewords than the header expects: no codeword after CW0 is decoded and the
+            # frame waits (rx_pipeline.cpp:394-401); without one whole codeword nothing is decoded at all (:352-354)
+            short = n_llr < self.n_cw * 648
+            none = n_llr < 648
+            good = good & ~short
+            info = info.clone()
+            info[:, 3] = torch.where(short & (info[:, 2] > 0), 0, info[:, 3])
+            info[:, 3] = torch.where(none, 0, info[:, 3])
+            info[:, 4] = torch.where(none, 0, info[:, 4])
         upd = torch.stack([torch.ones_like(flen, dtype=torch.int64), (~good).to(torch.int64), info[:, 3].to(torch.int64),
                            torch.full_like(flen, self.n_cw, dtype=torch.int64), (info[:, 4] == 0).to(torch.int64),
                            torch.zeros_like(flen, dtype=torch.int64)], dim=1)

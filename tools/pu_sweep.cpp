@@ -5,8 +5,12 @@
 //
 //   torchrun-style launch (RANK / WORLD_SIZE / LOCAL_RANK in the environment), or a single process:
 //     projectultra_b200/pu_sweep --table reduced --trials 16384 [--block 2048] [--manifest DIR] [--out rows.jsonl] [--fresh] [--frame-bytes N]
+//                                [--interleave]
 //   tables: smoke (4 modes, seconds), reduced (one mode per waveform family and channel + the chirp-acquired CFO rows of the regression matrix), config5 (105 modes x 40 SNR points),
 //   frames (whole-frame FER of protocol-v2 DATA frames of 200 and 1000 payload bytes, or N with --frame-bytes, over AWGN / good / poor)
+//   --interleave: every OFDM and MC-DPSK codeword through ChannelInterleaver(bits per symbol, 648) as the reference's IWaveform path
+//   does (OFDM: data carriers x bits per carrier = ChannelInterleaver(60) for the M1 DQPSK modes; MC-DPSK: carriers x bits per carrier);
+//   single-carrier DPSK rows stay without
 //
 // Rank 0 prints one JSON object per (mode, SNR point) with the Wilson 95 % interval of the FER, then one summary line with the
 // per-rank run times (scaling efficiency = mean / max of the ranks' times: ranks never wait for each other before the final sum).
@@ -222,6 +226,17 @@ int main(int argc, char** argv) {
     std::vector<pu_sweep_mode> modes = make_table(table, fast, frame_bytes);
     if (fresh)
         for (auto& m : modes) m.fresh_payloads = 1;
+    if (flag(argc, argv, "--interleave"))
+        for (auto& m : modes) {
+            if (m.waveform <= PU_WF_OFDM_CHIRP) {
+                pu_ofdm* h = nullptr;
+                if (pu_ofdm_create(ctx, &m.ofdm, &h) != PU_OK) { fprintf(stderr, "pu_sweep[%d]: %s\n", rank, pu_last_error()); return 2; }
+                m.interleave_bps = static_cast<uint32_t>(pu_ofdm_bits_per_symbol(h));
+                pu_ofdm_destroy(h);
+            } else if (m.waveform >= PU_WF_MCDPSK) {
+                m.interleave_bps = m.mcdpsk.num_carriers * m.mcdpsk.bits_per_symbol;
+            }
+        }
     pu_sweep_desc d{};
     d.modes = modes.data();
     d.n_modes = static_cast<uint32_t>(modes.size());
@@ -262,6 +277,8 @@ int main(int argc, char** argv) {
             if (is_ofdm) snprintf(desc, sizeof desc, "%u-FFT %s%s", md.ofdm.fft_size, mod_name(md.ofdm.modulation), md.ofdm.use_pilots ? " pilots" : "");
             else if (is_dpsk) snprintf(desc, sizeof desc, "%s 125 baud", md.dpsk.modulation == 0 ? "DBPSK" : md.dpsk.modulation == 1 ? "DQPSK" : "D8PSK");
             else snprintf(desc, sizeof desc, "%u carriers DQPSK", md.mcdpsk.num_carriers);
+            char il[40] = "";
+            if (md.interleave_bps) snprintf(il, sizeof il, ", \"interleave_bps\": %u", md.interleave_bps);
             for (uint32_t s = 0; s < md.n_snr; ++s, ++at) {
                 const uint64_t* c = &counters[static_cast<size_t>(at) * 6];
                 double lo, hi;
@@ -270,18 +287,18 @@ int main(int argc, char** argv) {
                 if (md.frame_payload_bytes) {     // whole-frame counters {frames, frame_errors, codewords_failed, codewords, header_failures, 0}
                     fprintf(out, "{\"mode\": %u, \"waveform\": \"%s\", \"modem\": \"%s\", \"code_rate\": \"%s\", \"channel\": \"%s\", \"cfo_hz\": %.1f, \"snr_db\": %.2f, "
                                  "\"frame_payload_bytes\": %u, \"codewords\": %llu, \"frames\": %llu, \"frame_errors\": %llu, \"fer\": %.6g, \"fer_ci95\": [%.6g, %.6g], "
-                                 "\"codeword_fail_rate\": %.6g, \"header_fail_rate\": %.6g}\n",
+                                 "\"codeword_fail_rate\": %.6g, \"header_fail_rate\": %.6g%s}\n",
                             m, kWaveform[md.waveform], desc, kRate[md.code_rate], kChannel[md.channel], md.cfo_hz, md.snr_first_db + s * md.snr_step_db,
                             md.frame_payload_bytes, (unsigned long long)(c[0] ? c[3] / c[0] : 0), (unsigned long long)c[0], (unsigned long long)c[1],
-                            c[0] ? double(c[1]) / c[0] : 0.0, lo, hi, c[3] ? double(c[2]) / c[3] : 0.0, c[0] ? double(c[4]) / c[0] : 0.0);
+                            c[0] ? double(c[1]) / c[0] : 0.0, lo, hi, c[3] ? double(c[2]) / c[3] : 0.0, c[0] ? double(c[4]) / c[0] : 0.0, il);
                     continue;
                 }
                 fprintf(out, "{\"mode\": %u, \"waveform\": \"%s\", \"modem\": \"%s\", \"code_rate\": \"%s\", \"channel\": \"%s\", \"cfo_hz\": %.1f, \"snr_db\": %.2f, "
                              "\"frames\": %llu, \"frame_errors\": %llu, \"fer\": %.6g, \"fer_ci95\": [%.6g, %.6g], \"ber\": %.6g, \"decode_fail\": %.6g, "
-                             "\"avg_iters\": %.4g}\n",
+                             "\"avg_iters\": %.4g%s}\n",
                         m, kWaveform[md.waveform], desc, kRate[md.code_rate], kChannel[md.channel], md.cfo_hz, md.snr_first_db + s * md.snr_step_db,
                         (unsigned long long)c[0], (unsigned long long)c[1], c[0] ? double(c[1]) / c[0] : 0.0, lo, hi, c[3] ? double(c[2]) / c[3] : 0.0,
-                        c[0] ? double(c[4]) / c[0] : 0.0, c[0] ? double(c[5]) / c[0] : 0.0);
+                        c[0] ? double(c[4]) / c[0] : 0.0, c[0] ? double(c[5]) / c[0] : 0.0, il);
             }
         }
         double tmax = 0, tsum = 0;
