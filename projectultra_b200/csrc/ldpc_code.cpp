@@ -329,6 +329,8 @@ LdpcLayout make_ldpc_layout(const LdpcCode& code) {
         rank[chk].resize(row.size() - 1);
         for (size_t e = 0; e + 1 < row.size(); ++e) rank[chk][e] = seen[row[e]]++;
     }
+    L.slot_deg.assign(L.kpad, 0);
+    for (int j = 0; j < k; ++j) L.slot_deg[L.var_slot[j]] = static_cast<uint8_t>(seen[j]);
 
     L.inf_slot = L.kpad;
     L.tot_words = L.kpad + 32;    // + one +INF word per bank

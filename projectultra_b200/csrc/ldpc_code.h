@@ -57,6 +57,8 @@ struct LdpcLayout {
     std::vector<uint16_t> cn_wr;      // [6][threads] msg[] index written by edge e of slot p
     std::vector<uint16_t> var_slot;   // [k]    a(j)
     std::vector<int16_t> slot_var;    // [kpad] j or -1
+    std::vector<uint8_t> slot_deg;    // [kpad] checks of the bit in slot a (0 for an empty slot): msg[d * kpad + a] is written
+                                      //        by a check exactly for d < slot_deg[a]
     int conflicts = 0;                // extra shared-memory wavefronts per iteration that the layout could not remove
 };
 LdpcLayout make_ldpc_layout(const LdpcCode& code);

@@ -165,9 +165,10 @@ __global__ void __launch_bounds__(512) ldpc_flood_kernel(LdpcDevTables t, const 
 //    (minimum of the other edges' magnitudes) (:185-201): both are FMNMX.XORSIGN combines (minxs below), so signs are
 //    never separated from magnitudes.  Ties between magnitudes need no care: every edge sees the minimum over the
 //    OTHER edges, which is what the reference's scan yields.
-//  * absent edges: variable-side slots point at a word holding +0.0f (x + 0 == x for x != -0); check-side edges of
-//    rows shorter than their warp's longest row read a total of +INF: no sign, and a magnitude of exactly the clamp
-//    limit, which cannot lower the first or second minimum of a row that has two real edges (every row does).
+//  * absent edges: variable-side message words that no check writes (degree <= d < DV, and every word of an empty slot) are
+//    zeroed once and hold +0.0f (x + 0 == x for x != -0); check-side edges of rows shorter than their warp's longest row read a
+//    total of +INF: no sign, and a magnitude that is never below the clamp limit, which cannot lower the first or second
+//    minimum of a row that has two real edges (every row does).
 struct LdpcRegDev {   // device view of LdpcLayout (ldpc_code.h)
     int k, m, kpad, inf_slot, msg_words, threads;
     const uint8_t* cn_ninfo;
@@ -176,6 +177,7 @@ struct LdpcRegDev {   // device view of LdpcLayout (ldpc_code.h)
     const uint16_t* cn_wr;     // [kE][threads]
     const uint16_t* var_slot;  // [k]
     const int16_t* slot_var;   // [kpad]
+    const uint8_t* slot_deg;   // [kpad]
 };
 
 // sign(a) XOR sign(b) on min(|a|, |b|): one FMNMX.XORSIGN.  It is the min-sum combine of two messages (:185-197: the
@@ -186,49 +188,81 @@ __device__ __forceinline__ float minxs(float a, float b) {
     return d;
 }
 
-template <int NE>
-__device__ __forceinline__ void cn_update(const float* __restrict__ tot, float* __restrict__ msg, const int (&rd)[kE], const int (&wr)[kE],
-                                          float (&prev)[kE], float par_llr, float& pc, float lim, bool last, unsigned& syn_bits) {
-    const float ptot = __fadd_rn(par_llr, pc);        // total of the parity bit (:206-213)
-    const float vp = __fsub_rn(ptot, pc);             // its v2c before the clamp (:219-222)
-    unsigned px = __float_as_uint(ptot);              // XOR of the totals' sign bits = parity of the hard decisions
-    // c[0] = parity edge, c[1..NE] = info edges: the clamped v2c messages, sign and magnitude together
+// One check pass of a row with NE info edges: new messages to every edge, and the XOR of the sign bits of the totals it read
+// (bit 31 = the row's parity of the previous iteration's hard decisions).  FIRST = iteration 0: no message has been sent yet
+// (prev = pc = 0, so the v2c messages are the totals themselves) and the channel LLRs are not clamped (:169-173).
+template <int NE, bool FIRST>
+__device__ __forceinline__ unsigned cn_update(const float* __restrict__ tot, float* __restrict__ msg, const int (&rd)[kE],
+                                              const int (&wr)[kE], float (&prev)[kE], float par_llr, float& pc) {
+    const float ptot = FIRST ? par_llr : __fadd_rn(par_llr, pc);   // total of the parity bit (:206-213)
+    const float vp = FIRST ? ptot : __fsub_rn(ptot, pc);           // its v2c before the clamp (:219-222)
+    unsigned px = __float_as_uint(ptot);                            // XOR of the totals' sign bits = parity of the hard decisions
+    // c[0] = parity edge, c[1..NE] = info edges: the v2c messages, sign and magnitude together.  The clamp to +-50 (:222) is
+    // applied to the two heads of the scans below only, c[0] (first term of every prefix) and c[NE] (first term of every
+    // suffix): every output oth[e] combines a prefix and a suffix, or is one of them, so its operand set holds at least one
+    // clamped head.  A combine takes the XOR of the signs, which a clamp does not touch, and the minimum of the magnitudes;
+    // min(|v|, 50) commutes with the minimum, so one clamped operand gives min(50, minimum of all operands): each output is
+    // exactly what clamping every operand gives.  The +INF totals of absent edges are covered too: unclamped they only add
+    // an operand of magnitude >= 50.
     float c[NE + 1];
-    c[0] = minxs(vp, lim);
+    c[0] = FIRST ? vp : minxs(vp, 50.0f);
 #pragma unroll
     for (int e = 0; e < NE; ++e) {
         const float te = tot[rd[e]];
         px ^= __float_as_uint(te);
-        c[e + 1] = minxs(__fsub_rn(te, prev[e]), lim);
+        const float v = FIRST ? te : __fsub_rn(te, prev[e]);
+        c[e + 1] = (FIRST || e + 1 < NE) ? v : minxs(v, 50.0f);
     }
-    syn_bits = px;
-    if (!last) {
-        // sign product and minimum magnitude over the OTHER edges of the row (:185-197) from prefix and suffix combines:
-        // 3(n-2) FMNMX.XORSIGN for n edges, exact (neither a minimum nor an XOR depends on the order it is taken in)
-        float oth[NE + 1];
-        if (NE == 0) {
-            oth[0] = FLT_MAX;
-        } else {
-            float pre[NE + 1], suf[NE + 1];
-            pre[0] = c[0];
+    // sign product and minimum magnitude over the OTHER edges of the row (:185-197) from prefix and suffix combines:
+    // 3(n-2) FMNMX.XORSIGN for n edges, exact (neither a minimum nor an XOR depends on the order it is taken in)
+    float oth[NE + 1];
+    if (NE == 0) {
+        oth[0] = FLT_MAX;
+    } else {
+        float pre[NE + 1], suf[NE + 1];
+        pre[0] = c[0];
 #pragma unroll
-            for (int i = 1; i < NE; ++i) pre[i] = minxs(pre[i - 1], c[i]);
-            suf[NE] = c[NE];
+        for (int i = 1; i < NE; ++i) pre[i] = minxs(pre[i - 1], c[i]);
+        suf[NE] = c[NE];
 #pragma unroll
-            for (int i = NE - 1; i >= 1; --i) suf[i] = minxs(suf[i + 1], c[i]);
-            oth[0] = suf[1];
-            oth[NE] = pre[NE - 1];
+        for (int i = NE - 1; i >= 1; --i) suf[i] = minxs(suf[i + 1], c[i]);
+        oth[0] = suf[1];
+        oth[NE] = pre[NE - 1];
 #pragma unroll
-            for (int i = 1; i < NE; ++i) oth[i] = minxs(pre[i - 1], suf[i + 1]);
+        for (int i = 1; i < NE; ++i) oth[i] = minxs(pre[i - 1], suf[i + 1]);
+    }
+    // sign * min_abs * 0.75f (:200)
+#pragma unroll
+    for (int e = 0; e < NE; ++e) {
+        const float out = __fmul_rn(oth[e + 1], 0.75f);
+        prev[e] = out;
+        msg[wr[e]] = out;
+    }
+    pc = __fmul_rn(oth[0], 0.75f);
+    return px;
+}
+
+// The syndrome part of a check pass alone (the pass after the last iteration sends no messages).
+template <int NE>
+__device__ __forceinline__ unsigned cn_syndrome(const float* __restrict__ tot, const int (&rd)[kE], float par_llr, float pc) {
+    unsigned px = __float_as_uint(__fadd_rn(par_llr, pc));
+#pragma unroll
+    for (int e = 0; e < NE; ++e) px ^= __float_as_uint(tot[rd[e]]);
+    return px;
+}
+
+// Variable pass: the total of every information bit this thread owns, messages summed in ascending check order (:208-213).
+template <int VR, int DV, int T, int KP>
+__device__ __forceinline__ void vn_update(const float* __restrict__ msg, float* __restrict__ tot, const float (&lin)[VR], int tid) {
+#pragma unroll
+    for (int r = 0; r < VR; ++r) {
+        const int a = tid + r * T;
+        if ((r + 1) * T <= KP || a < KP) {
+            float s = lin[r];
+#pragma unroll
+            for (int d = 0; d < DV; ++d) s = __fadd_rn(s, msg[d * KP + a]);
+            tot[a] = s;
         }
-        // sign * min_abs * 0.75f (:200)
-#pragma unroll
-        for (int e = 0; e < NE; ++e) {
-            const float out = __fmul_rn(oth[e + 1], 0.75f);
-            prev[e] = out;
-            msg[wr[e]] = out;
-        }
-        pc = __fmul_rn(oth[0], 0.75f);
     }
 }
 
@@ -237,42 +271,38 @@ __device__ __forceinline__ void cn_update(const float* __restrict__ tot, float* 
 // construction.  The check pass gathers tot[a] and scatters msg[rank * KP + a]; both hit bank a mod 32, and the
 // layout (ldpc_code.cpp: make_ldpc_layout) makes the 32 lanes of a warp use 32 different banks on every edge.
 //
-// The whole iteration loop is specialised on NE = the longest row of the warp (check slots are sorted by degree, so
-// warps are nearly uniform): every warp runs its own copy of the loop, and all copies execute the same sequence of
-// CTA-wide barriers (barrier 0 counts arriving threads, not program counters).  KP, T and DV are compile-time, so every
-// shared-memory access of the variable pass is base + immediate.  Threads past the last check slot run a dummy row
-// (table defaults: reads of the +INF word, writes to the scratch words, a parity LLR of +0) whose total is never
-// negative, so there is no per-thread predicate in the loop.
+// The whole decode is specialised on NE = the longest row of the warp (check slots are sorted by degree, so warps are
+// nearly uniform): every warp runs its own copy, and all copies execute the same sequence of CTA-wide barriers (barrier 0
+// counts arriving threads, not program counters; max_iter and the voted syndrome are uniform over the CTA).  KP, T and DV
+// are compile-time, so every shared-memory access of the variable pass is base + immediate.  Threads past the last check
+// slot run a dummy row (table defaults: reads of the +INF word, writes to the scratch words, a parity LLR of +0) whose total
+// is never negative, so there is no per-thread predicate in the loop.
+//
+// Iteration 0 (unclamped, no syndrome to test) and the syndrome-only pass after the last iteration are peeled off, so the
+// loop body is one check pass, the vote and one variable pass.  The syndrome voted in iteration it is that of the totals
+// of iteration it-1 (:227-235): a zero syndrome there means it-1 iterations were run, and converged.
 template <int NE, int VR, int DV, int T, int KP>
 __device__ __forceinline__ void decode_loop(float* __restrict__ msg, float* __restrict__ tot, const int (&rd)[kE], const int (&wr)[kE],
                                             const float (&lin)[VR], float par_llr, int tid, int max_iter, int& it_out, int& converged) {
-    float prev[kE];
-#pragma unroll
-    for (int e = 0; e < kE; ++e) prev[e] = 0.0f;
-    float pc = 0.0f;
-    int it = 0;
+    it_out = 0;
     converged = 0;
-    for (;; ++it) {
-        const bool last = (it == max_iter);
-        const float lim = (it == 0) ? INFINITY : 50.0f;   // iteration 0 consumes the raw channel LLRs (:169-173)
-        unsigned syn_bits = 0;
-        cn_update<NE>(tot, msg, rd, wr, prev, par_llr, pc, lim, last, syn_bits);
-        const int any = __syncthreads_or(static_cast<int>(syn_bits >> 31));   // syndrome of iteration it-1's totals (:227-235)
-        if (it > 0 && !any) { converged = 1; --it; break; }
-        if (last) break;
-#pragma unroll
-        for (int r = 0; r < VR; ++r) {
-            const int a = tid + r * T;
-            if ((r + 1) * T <= KP || a < KP) {
-                float s = lin[r];
-#pragma unroll
-                for (int d = 0; d < DV; ++d) s = __fadd_rn(s, msg[d * KP + a]);   // ascending check order (:208-213)
-                tot[a] = s;
-            }
-        }
+    if (max_iter == 0) return;   // no iteration: the hard decisions of the channel LLRs, not converged
+    float prev[kE];
+    float pc = 0.0f;
+    cn_update<NE, true>(tot, msg, rd, wr, prev, par_llr, pc);
+    __syncthreads();
+    vn_update<VR, DV, T, KP>(msg, tot, lin, tid);
+    __syncthreads();
+    int it = 1, any = 1;
+    for (; it < max_iter; ++it) {
+        any = __syncthreads_or(static_cast<int>(cn_update<NE, false>(tot, msg, rd, wr, prev, par_llr, pc)) < 0);   // sign bit
+        if (!any) break;
+        vn_update<VR, DV, T, KP>(msg, tot, lin, tid);
         __syncthreads();
     }
-    it_out = it;
+    if (any) any = __syncthreads_or(static_cast<int>(cn_syndrome<NE>(tot, rd, par_llr, pc)) < 0);   // it == max_iter
+    converged = !any;
+    it_out = any ? it : it - 1;
 }
 
 template <int VR, int DV, int T, int MINB, int KP>
@@ -294,21 +324,30 @@ __global__ void __launch_bounds__(T, MINB) ldpc_flood_reg_kernel(LdpcRegDev t, c
         wr[e] = t.cn_wr[e * T + tid];
     }
     const int ninfo = t.cn_ninfo[tid];                       // 0 past the last check slot
-    const float par_llr = tid < M ? __fadd_rn(x[K + t.cn_check[tid]], 0.0f) : 0.0f;
+    const int chk = t.cn_check[tid];
+    int sv[VR];
+#pragma unroll
+    for (int r = 0; r < VR; ++r) {
+        const int a = tid + r * T;
+        sv[r] = a < KP ? t.slot_var[a] : -1;
+        if (a < KP) {   // the message words of slot a that no check writes; the others are written by the first check pass
+            const int deg = t.slot_deg[a];
+#pragma unroll
+            for (int d = 0; d < DV; ++d)
+                if (d >= deg) msg[d * KP + a] = 0.0f;
+        }
+    }
     const int nw = __reduce_max_sync(0xffffffffu, ninfo);   // longest row of this warp (slots are sorted by degree)
+    if (tid < 32) tot[KP + tid] = INFINITY;                    // LdpcLayout::inf_slot: one +INF word per bank
+    // channel LLRs canonicalised on load (+0.0f)
+    const float par_llr = tid < M ? __fadd_rn(x[K + chk], 0.0f) : 0.0f;
     float lin[VR];
 #pragma unroll
     for (int r = 0; r < VR; ++r) {
         const int a = tid + r * T;
-        lin[r] = 0.0f;
-        if (a < KP) {
-            const int j = t.slot_var[a];
-            if (j >= 0) lin[r] = __fadd_rn(x[j], 0.0f);
-            tot[a] = lin[r];
-        }
+        lin[r] = sv[r] >= 0 ? __fadd_rn(x[sv[r]], 0.0f) : 0.0f;
+        if (a < KP) tot[a] = lin[r];
     }
-    for (int i = tid; i < kMsgWords; i += T) msg[i] = 0.0f;   // absent variable-side edges stay +0 forever
-    if (tid < 32) tot[KP + tid] = INFINITY;                    // LdpcLayout::inf_slot: one +INF word per bank
     __syncthreads();
 
     int it = 0, converged = 0;
@@ -323,13 +362,21 @@ __global__ void __launch_bounds__(T, MINB) ldpc_flood_reg_kernel(LdpcRegDev t, c
     }
     __syncthreads();   // every warp has left its loop: the totals are final
 
+    // k information bits MSB-first, last byte left-justified (:242-256): warp w packs bits r*T + 32w .. +31 into 4 bytes
     uint8_t* out = info + static_cast<size_t>(blockIdx.x) * info_stride;
-    const int nbytes = (K + 7) >> 3;
-    for (int b = tid; b < nbytes; b += T) {   // k information bits MSB-first, last byte left-justified (:242-256)
-        unsigned byte = 0;
-        int cnt = 0;
-        for (int j = b * 8; j < b * 8 + 8 && j < K; ++j, ++cnt) byte = (byte << 1) | (tot[t.var_slot[j]] < 0.0f ? 1u : 0u);
-        out[b] = static_cast<uint8_t>(byte << (8 - cnt));
+    // (the slots are loaded here and not in the prologue: kept in registers through the loop, they would cost the R2/3 .. R5/6
+    // instances registers and occupancy)
+    const int nbytes = (K + 7) >> 3, lane = tid & 31;
+    int vs[VR];   // slot of information bit j = tid + r*T (the +INF word past k)
+#pragma unroll
+    for (int r = 0; r < VR; ++r) vs[r] = tid + r * T < K ? t.var_slot[tid + r * T] : KP;
+#pragma unroll
+    for (int r = 0; r < VR; ++r) {
+        if (r * T < K) {
+            const unsigned bits = __brev(__ballot_sync(0xffffffffu, tot[vs[r]] < 0.0f));   // bit 31 = lowest j of the warp
+            const int b = ((r * T + (tid & ~31)) >> 3) + lane;
+            if (lane < 4 && b < nbytes) out[b] = static_cast<uint8_t>(bits >> (24 - 8 * lane));
+        }
     }
     if (tid == 0) {
         if (ok) ok[blockIdx.x] = static_cast<uint8_t>(converged);
@@ -347,7 +394,7 @@ struct pu_ldpc {
     pu::LdpcHostTables host;
     pu::DevMem d_ninfo, d_check, d_var, d_deg, d_slot;
     pu::LdpcLayout layout;
-    pu::DevMem r_ninfo, r_check, r_rd, r_wr, r_vslot, r_svar;
+    pu::DevMem r_ninfo, r_check, r_rd, r_wr, r_vslot, r_svar, r_sdeg;
     pu::LdpcRegDev reg{};
     pu::LdpcDevTables dev{};
     int threads = 128;
@@ -384,6 +431,7 @@ struct pu_ldpc {
         if ((s = r_wr.upload(layout.cn_wr.data(), layout.cn_wr.size())) != PU_OK) return s;
         if ((s = r_vslot.upload(layout.var_slot.data(), layout.var_slot.size())) != PU_OK) return s;
         if ((s = r_svar.upload(layout.slot_var.data(), layout.slot_var.size())) != PU_OK) return s;
+        if ((s = r_sdeg.upload(layout.slot_deg.data(), layout.slot_deg.size())) != PU_OK) return s;
         reg.k = layout.k; reg.m = layout.m; reg.kpad = layout.kpad; reg.inf_slot = layout.inf_slot;
         reg.msg_words = layout.msg_words; reg.threads = layout.threads;
         reg.cn_ninfo = static_cast<const uint8_t*>(r_ninfo.p);
@@ -392,6 +440,7 @@ struct pu_ldpc {
         reg.cn_wr = static_cast<const uint16_t*>(r_wr.p);
         reg.var_slot = static_cast<const uint16_t*>(r_vslot.p);
         reg.slot_var = static_cast<const int16_t*>(r_svar.p);
+        reg.slot_deg = static_cast<const uint8_t*>(r_sdeg.p);
         reg_threads = layout.threads;
         reg_vr = layout.vr;
         reg_dv = layout.dv;
