@@ -449,6 +449,16 @@ PU_API pu_status pu_frame_decode_batch(pu_ctx* ctx, pu_ldpc* dec, const float* l
  * the codeword count. */
 PU_API pu_status pu_frame_encode(int code_rate, const uint8_t* frame, size_t n_bytes, uint8_t* out, size_t out_cap,
                                  size_t* n_codewords);
+/* LDPCEncoder::encode of one block per row on the GPU: payload[b * payload_stride ..+ payload_bytes) (payload_bytes <= k / 8, zero padded
+ * to k bits) -> coded[b * coded_stride ..+ 81).  Bit-identical to pu_ldpc_encode.  One CTA per row, the encoder of pu_ofdm_tx_batch.
+ * PU_MEM_HOST stages through the context; bytes beyond 81 in a row are not written. */
+PU_API pu_status pu_ldpc_encode_batch(const pu_ldpc* code, const uint8_t* payload, size_t payload_stride, size_t payload_bytes, size_t B,
+                                      uint8_t* coded, size_t coded_stride, pu_memspace space, void* stream);
+/* v2::encodeFrameWithLDPC (frame_v2.cpp:1079-1127) per row on the GPU at the code's rate: frames[b * frame_stride ..+ frame_bytes) ->
+ * coded[b * coded_stride ..+ n_codewords * 81).  Bit-identical to pu_frame_encode; at most 255 codewords, as pu_frame_tx_batch (whose
+ * encoder it is).  B == 0 or coded == NULL only sets *n_codewords.  Bytes beyond n_codewords * 81 in a row are not written. */
+PU_API pu_status pu_frame_encode_batch(const pu_ldpc* code, const uint8_t* frames, size_t frame_stride, size_t frame_bytes, size_t B,
+                                       uint8_t* coded, size_t coded_stride, size_t* n_codewords, pu_memspace space, void* stream);
 
 /* Frame-error rule of the tools (tools/test_mode_snr.cpp:98-104): success iff lastDecodeSuccess() and the first
  * payload_bytes decoded bytes equal the payload.  DEVICE pointers.  counters[bin[b]][6] (uint64, atomically
@@ -458,6 +468,17 @@ PU_API pu_status pu_count_errors(pu_ctx* ctx, const uint8_t* info_bytes, size_t 
                                  const int32_t* iters, const uint8_t* payload_pool, size_t payload_stride,
                                  const uint32_t* tx_index, const uint32_t* bin, size_t payload_bytes, size_t B,
                                  uint64_t* counters, void* stream);
+/* Pre-decoder (raw) bit errors: soft bits against the coded bits sent, DEVICE pointers.  For b < B and j < n_bits, soft bit
+ * llr[b * llr_stride + j] (decoder order, i.e. after any deinterleaving) against bit j (MSB first) of coded[coded_index[b] *
+ * coded_stride ...] (coded_index NULL = row b).  Positions j >= n_valid[b] (n_valid NULL = all valid) and soft bits equal to +-0 are
+ * erasures; otherwise the hard decision is 1 iff llr < 0 (the decoder's rule).  counters[bin[b]][4] (uint64, accumulated with integer
+ * atomics, so a table does not depend on the launch order) = {soft_bits (n_bits per row), erasures, bit_errors (erasures excluded),
+ * strong_errors (bit errors with |llr| >= strong)}; bin NULL = row 0.  The sweep passes strong = 10, the clipLLR bound of the OFDM
+ * demappers and the clamp of the MC-DPSK demapper; single-carrier DPSK soft bits stop at 5, so that column is 0 for its rows (and
+ * MC-DPSK's errors were not seen to reach 10 in the reduced sweep table either). */
+PU_API pu_status pu_count_raw_errors(pu_ctx* ctx, const float* llr, size_t llr_stride, size_t n_bits, const int32_t* n_valid,
+                                     const uint8_t* coded, size_t coded_stride, const uint32_t* coded_index, const uint32_t* bin,
+                                     size_t B, float strong, uint64_t* counters, void* stream);
 
 /* ---------------------------------------------------------------- Monte-Carlo sweep driver (BASELINE.json config 5)
  * The reference runs its FER/BER waterfalls as a shell matrix over one-process-per-cell tools (tests/regression_matrix.sh:139-243 over
@@ -562,6 +583,14 @@ PU_API void pu_sweep_payload(uint64_t base_seed, uint32_t mode, uint32_t index, 
  * iteration_sum} per (mode, SNR point) -- whole-frame counters for frame modes (pu_sweep_mode.frame_payload_bytes) --, rank 0
  * additionally holding the resumed units; stats may be NULL. */
 PU_API pu_status pu_linksim_run(pu_ctx* ctx, const pu_sweep_desc* d, uint64_t* counters, pu_sweep_stats* stats);
+/* pu_linksim_run with a second table: raw[pu_sweep_point_count][4] (HOST, uint64) = the pu_count_raw_errors counters {soft_bits, erasures,
+ * bit_errors, strong_errors} (strong = 10) over every soft bit the decoder is given (648 per codeword trial, n_cw x 648 per frame trial;
+ * the soft bits an acquiring receiver did not deliver are erasures, located through the deinterleaver's permutation when the mode
+ * interleaves), or raw == NULL = exactly pu_linksim_run.  counters is the same table
+ * pu_linksim_run returns: PU_WF_OFDM codewords leave the fused demodulate + decode call for its two halves, which decode the same.  A raw
+ * run keys its manifest apart from a plain run of the same table (neither resumes from the other's shards) and records the 4 raw
+ * counters of every unit behind its 6 counters; rank 0 returns the resumed raw counters too. */
+PU_API pu_status pu_linksim_run_raw(pu_ctx* ctx, const pu_sweep_desc* d, uint64_t* counters, uint64_t* raw, pu_sweep_stats* stats);
 /* Sum n uint64 counters over the ranks of an NCCL communicator (ncclComm_t passed as void*; libnccl is resolved at run time with
  * dlopen, the library does not link it).  PU_MEM_HOST stages through the context; comm == NULL is a no-op (single rank). */
 PU_API pu_status pu_counters_allreduce(pu_ctx* ctx, uint64_t* counters, size_t n, void* nccl_comm, pu_memspace space, void* stream);

@@ -189,6 +189,42 @@ class LdpcDecoder:
                                           C.c_size_t(frame_cap), _ptr(flen), _ptr(info), sp, _stream(sp)))
         return frames, flen, info
 
+    def encode_batch(self, payload, out=None):
+        """pu_ldpc_encode_batch: LDPCEncoder::encode of every row of payload [B, payload_bytes <= k / 8] uint8 (numpy => host, torch.cuda =>
+        device) at this decoder's rate -> coded [B, 81] uint8.  `out` may have rows wider than 81 bytes (their padding is left as it is)."""
+        B, nbytes = payload.shape
+        payload, stride = _byte_rows(payload)
+        out = _like(payload, (B, 81), np.uint8, "uint8") if out is None else out
+        out, ostride = _byte_rows(out)
+        assert out.shape[0] == B and out.shape[1] >= 81
+        sp = _space(payload, out)
+        check(lib().pu_ldpc_encode_batch(self._h, _ptr(payload), C.c_size_t(stride), C.c_size_t(nbytes), C.c_size_t(B), _ptr(out),
+                                         C.c_size_t(ostride), sp, _stream(sp)))
+        return out
+
+    def frame_codewords(self, frame_bytes):
+        """Codewords of a frame of frame_bytes bytes at this decoder's rate (pu_frame_encode_batch's query)."""
+        n = C.c_size_t(0)
+        check(lib().pu_frame_encode_batch(self._h, None, C.c_size_t(frame_bytes), C.c_size_t(frame_bytes), C.c_size_t(0), None, C.c_size_t(0),
+                                          C.byref(n), 0, None))
+        return int(n.value)
+
+    def frame_encode_batch(self, frames, out=None):
+        """pu_frame_encode_batch: v2::encodeFrameWithLDPC of every row of frames [B, frame_bytes] uint8 (numpy => host, torch.cuda => device)
+        at this decoder's rate -> coded [B, n_codewords * 81] uint8.  `out` may have wider rows (their padding is left as it is).
+        Returns (out, n_codewords)."""
+        B, nbytes = frames.shape
+        ncw = self.frame_codewords(nbytes)
+        frames, stride = _byte_rows(frames)
+        out = _like(frames, (B, ncw * 81), np.uint8, "uint8") if out is None else out
+        out, ostride = _byte_rows(out)
+        assert out.shape[0] == B and out.shape[1] >= ncw * 81
+        n = C.c_size_t(0)
+        sp = _space(frames, out)
+        check(lib().pu_frame_encode_batch(self._h, _ptr(frames), C.c_size_t(stride), C.c_size_t(nbytes), C.c_size_t(B), _ptr(out),
+                                          C.c_size_t(ostride), C.byref(n), sp, _stream(sp)))
+        return out, int(n.value)
+
     def decode_batch(self, llr, info=None, ok=None, iters=None):
         """llr: [B, >=648] float32 (numpy => host, torch.cuda => device).  Returns (info_bytes, ok, iters)."""
         if _is_torch(llr):
@@ -320,6 +356,33 @@ def frame_encode(rate, frame):
     out = np.zeros((n.value, 81), np.uint8)
     check(lib().pu_frame_encode(int(rate), _ptr(f), C.c_size_t(len(f)), _ptr(out), C.c_size_t(out.size), C.byref(n)))
     return out
+
+
+def _byte_rows(x):
+    """(x, row stride in bytes) of a 2-D uint8 array whose rows are contiguous (numpy arrays are made so)."""
+    if _is_torch(x):
+        import torch
+        assert x.dtype == torch.uint8 and x.dim() == 2 and x.stride(1) == 1
+        return x, x.stride(0)
+    if not (x.dtype == np.uint8 and x.ndim == 2 and x.strides[1] == 1):
+        x = np.ascontiguousarray(x, dtype=np.uint8)
+    return x, x.strides[0]
+
+
+def count_raw_errors(ctx, llr, coded, counters, n_bits=None, n_valid=None, coded_index=None, bins=None, strong=10.0):
+    """pu_count_raw_errors on device tensors, torch's current stream: soft bits llr [B, >= n_bits] float32 (decoder order) against the
+    coded bytes sent, row coded_index[b] of coded [P, >= n_bits / 8] uint8 (None = row b); positions >= n_valid[b] (int32 [B], None = all)
+    and soft bits equal to +-0 are erasures.  counters: torch.int64 [n_bins, 4] (RAW_COUNTER_NAMES of linksim) accumulated in place at
+    row bins[b] (None = row 0).  n_bits defaults to the width of llr."""
+    import torch
+    assert llr.dtype == torch.float32 and llr.dim() == 2 and llr.stride(1) == 1 and coded.dtype == torch.uint8 and coded.stride(-1) == 1
+    assert counters.dtype == torch.int64 and counters.is_contiguous() and counters.shape[-1] == 4
+    B = llr.shape[0]
+    n = llr.shape[1] if n_bits is None else int(n_bits)
+    check(lib().pu_count_raw_errors(ctx._h, _ptr(llr), C.c_size_t(llr.stride(0)), C.c_size_t(n), _ptr(n_valid), _ptr(coded),
+                                    C.c_size_t(coded.stride(0)), _ptr(coded_index), _ptr(bins), C.c_size_t(B), C.c_float(strong),
+                                    _ptr(counters), C.c_void_p(torch.cuda.current_stream().cuda_stream)))
+    return counters
 
 
 def channel_interleaver_perm(bps, total=648):
@@ -948,12 +1011,17 @@ class Sweep:
         lib().pu_sweep_payload(C.c_uint64(self.desc.base_seed), C.c_uint32(mode), C.c_uint32(index), _ptr(out), C.c_size_t(len(out)))
         return out
 
-    def run(self, ctx):
-        """pu_linksim_run -> (counters [n_points, 6] uint64 on the host, SweepStats)."""
+    def run(self, ctx, raw=False):
+        """pu_linksim_run -> (counters [n_points, 6] uint64 on the host, SweepStats); raw=True: pu_linksim_run_raw -> (counters, stats,
+        raw [n_points, 4] uint64 = linksim.RAW_COUNTER_NAMES of the soft bits the decoder was given)."""
         counters = np.zeros((self.n_points, 6), np.uint64)
         st = SweepStats()
-        check(lib().pu_linksim_run(ctx._h, C.byref(self.desc), _ptr(counters), C.byref(st)))
-        return counters, st
+        if not raw:
+            check(lib().pu_linksim_run(ctx._h, C.byref(self.desc), _ptr(counters), C.byref(st)))
+            return counters, st
+        table = np.zeros((self.n_points, 4), np.uint64)
+        check(lib().pu_linksim_run_raw(ctx._h, C.byref(self.desc), _ptr(counters), _ptr(table), C.byref(st)))
+        return counters, st, table
 
     def point_rows(self, counters):
         """[(mode index, snr_db, counter row)] in counter-table order."""

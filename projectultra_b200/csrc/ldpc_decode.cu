@@ -488,6 +488,7 @@ void pu_ldpc_encoder_view(const pu_ldpc* h, int* k, int* m, const uint8_t** cn_n
     *k = h->dev.k; *m = h->dev.m;
     *cn_ninfo = h->dev.cn_ninfo; *cn_check = h->dev.cn_check; *cn_var = h->dev.cn_var;
 }
+pu_ctx* pu_ldpc_context(const pu_ldpc* h) { return h->ctx; }
 
 extern "C" {
 

@@ -5,6 +5,7 @@
 // tools/test_ofdm_chirp_pilots.cpp:166-260: per trial  channel.process -> demodulator.processPresynced ->
 // getSoftBits (first 648) -> LDPCDecoder::decodeSoft -> success iff lastDecodeSuccess() AND decoded bytes == payload
 // (test_mode_snr.cpp:98-104).  Trials are independent, so here they are the batch dimension.
+#include <algorithm>
 #include <memory>
 #include <new>
 
@@ -103,9 +104,93 @@ pu_status count_frame_errors(pu_ctx* ctx, const uint8_t* frame_out, size_t frame
     return PU_OK;
 }
 
+// Pre-decoder counters (pu_count_raw_errors): counters[bin][4] = {soft_bits, erasures, bit_errors, strong_errors}.  Each warp takes a
+// contiguous range of rows; neighbouring rows of a sweep batch share their bin (one work unit), so a lane keeps its counts in registers
+// while the bin stays the same and the warp sums them into the global table only when it changes: a few atomics per (warp, unit) instead
+// of per soft bit or per row.  Soft bits past n_valid are not read.  il_step != 0: the row was deinterleaved codeword by codeword with
+// ChannelInterleaver(step = il_step, 648), so n_valid counts soft bits in DELIVERED order: decoder bit c * 648 + i came from delivered
+// position c * 648 + (i * il_step mod 648), and it is an erasure when that position is >= n_valid.
+__global__ void __launch_bounds__(256) count_raw_errors_kernel(const float* __restrict__ llr, size_t llr_stride, int n_bits, int il_step,
+                                                               const int32_t* __restrict__ n_valid, const uint8_t* __restrict__ coded,
+                                                               size_t coded_stride, const uint32_t* __restrict__ coded_index,
+                                                               const uint32_t* __restrict__ bin, size_t B, size_t rows_per_warp, float strong,
+                                                               unsigned long long* __restrict__ counters) {
+    const int lane = threadIdx.x & 31;
+    const size_t b0 = ((blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x) >> 5) * rows_per_warp;
+    const size_t b1 = min(B, b0 + rows_per_warp);
+    if (b0 >= b1) return;
+    unsigned long long c[4] = {0ull, 0ull, 0ull, 0ull};
+    uint32_t cur = bin ? bin[b0] : 0u;
+    auto flush = [&]() {
+        for (int i = 0; i < 4; ++i)
+            for (int o = 16; o > 0; o >>= 1) c[i] += __shfl_xor_sync(0xffffffffu, c[i], o);
+        if (lane == 0)
+            for (int i = 0; i < 4; ++i)
+                if (c[i]) atomicAdd(&counters[static_cast<size_t>(cur) * 4 + i], c[i]);
+        c[0] = c[1] = c[2] = c[3] = 0ull;
+    };
+    for (size_t b = b0; b < b1; ++b) {
+        const uint32_t bb = bin ? bin[b] : 0u;
+        if (bb != cur) {
+            flush();
+            cur = bb;
+        }
+        const float* x = llr + b * llr_stride;
+        const uint8_t* want = coded + static_cast<size_t>(coded_index ? coded_index[b] : b) * coded_stride;
+        const int nv = n_valid ? min(max(n_valid[b], 0), n_bits) : n_bits;
+        const bool permuted = il_step && nv < n_bits;
+        if (lane == 0) {
+            c[0] += static_cast<unsigned long long>(n_bits);
+            if (!permuted) c[1] += static_cast<unsigned long long>(n_bits - nv);
+        }
+        for (int j = lane; j < (permuted ? n_bits : nv); j += 32) {
+            if (permuted) {
+                const int cw = j / PU_LDPC_N, i = j - cw * PU_LDPC_N;
+                if (cw * PU_LDPC_N + i * il_step % PU_LDPC_N >= nv) { ++c[1]; continue; }
+            }
+            const float v = x[j];
+            if (v == 0.0f) { ++c[1]; continue; }                      // +0 and -0
+            const unsigned sent = (want[j >> 3] >> (7 - (j & 7))) & 1u;
+            if ((v < 0.0f ? 1u : 0u) != sent) {
+                ++c[2];
+                if (fabsf(v) >= strong) ++c[3];
+            }
+        }
+    }
+    flush();
+}
+
+pu_status count_raw_errors(pu_ctx* ctx, const float* llr, size_t llr_stride, size_t n_bits, const int32_t* n_valid, const uint8_t* coded,
+                           size_t coded_stride, const uint32_t* coded_index, const uint32_t* bin, size_t B, float strong, uint64_t* counters,
+                           cudaStream_t st, uint32_t il_step) {
+    PU_REQUIRE(n_bits <= llr_stride && (n_bits + 7) / 8 <= coded_stride && n_bits < (size_t(1) << 30),
+               "pu_count_raw_errors: rows shorter than n_bits soft / coded bits");
+    if (B == 0 || n_bits == 0) return PU_OK;
+    const size_t warps = std::min<size_t>(B, static_cast<size_t>(std::max(ctx->sm_count, 1)) * 64);
+    const size_t per = (B + warps - 1) / warps;
+    const size_t blocks = ((B + per - 1) / per + 7) / 8;
+    (void)cudaGetLastError();
+    count_raw_errors_kernel<<<static_cast<unsigned>(blocks), 256, 0, st>>>(llr, llr_stride, static_cast<int>(n_bits), static_cast<int>(il_step), n_valid,
+                                                                          coded, coded_stride,
+                                                                          coded_index, bin, B, per, strong,
+                                                                          reinterpret_cast<unsigned long long*>(counters));
+    ctx->launches.fetch_add(1);
+    PU_CUDA_TRY(cudaGetLastError());
+    return PU_OK;
+}
+
 }  // namespace pu
 
 extern "C" {
+
+pu_status pu_count_raw_errors(pu_ctx* ctx, const float* llr, size_t llr_stride, size_t n_bits, const int32_t* n_valid, const uint8_t* coded,
+                              size_t coded_stride, const uint32_t* coded_index, const uint32_t* bin, size_t B, float strong, uint64_t* counters,
+                              void* stream) {
+    PU_REQUIRE(ctx && counters && (B == 0 || (llr && coded)), "pu_count_raw_errors: NULL argument");
+    PU_CUDA_TRY(cudaSetDevice(ctx->device));
+    return pu::count_raw_errors(ctx, llr, llr_stride, n_bits, n_valid, coded, coded_stride, coded_index, bin, B, strong, counters,
+                                reinterpret_cast<cudaStream_t>(stream));
+}
 
 pu_status pu_count_errors(pu_ctx* ctx, const uint8_t* info_bytes, size_t info_stride, const uint8_t* ok,
                           const int32_t* iters, const uint8_t* payload_pool, size_t payload_stride,

@@ -30,6 +30,7 @@
 #include "ofdm_plan.h"
 #include "pu_async.cuh"
 #include "frame_v2.cuh"
+#include "ldpc_encode.cuh"
 #include "pu_internal.h"
 #include "ref_math.cuh"
 #include "ofdm_dev.cuh"
@@ -987,14 +988,11 @@ cudaError_t ofdm_acquire_launch(const AcqDev& a, const float* samples, size_t B,
 // ofdm_tx_gpu.cu
 struct TxDev {
     int nfft, cp, sym_len, guard, n_data, n_pilot, bps, differential;
-    int k, m;
     int pre_len, n_sym, frame_len;
     int osc_start;
     float scale;
     int il_inv;
-    const uint8_t* cn_ninfo;
-    const uint16_t* cn_check;
-    const uint16_t* cn_var;
+    LdpcEncDev enc;
     const int* data_bin;
     const int* pilot_bin;
     const float* pilot_sign;
@@ -1504,7 +1502,7 @@ pu_status ofdm_tx_frames(pu_ofdm* h, const pu_ldpc* code, const uint8_t* frames,
     pu_ctx* ctx = h->ctx;
     PU_CUDA_TRY(cudaSetDevice(ctx->device));
     pu::TxDev t{};
-    pu_ldpc_encoder_view(code, &t.k, &t.m, &t.cn_ninfo, &t.cn_check, &t.cn_var);
+    pu_ldpc_encoder_view(code, &t.enc.k, &t.enc.m, &t.enc.cn_ninfo, &t.enc.cn_check, &t.enc.cn_var);
     pu_status s;
     if (h->tx_pre_len[layout] < 0) {                 // generateTrainingSymbols / generatePreamble: payload independent
         std::vector<float> pre = pu::ofdm_modulate_frame(p, layout, nullptr, 0);

@@ -16,6 +16,7 @@
 // The inverse FFT is the reference's radix-2 DIT with conjugated twiddles and 1/N scaling on a shared-memory buffer
 // (fft_smem.cuh); constellation points / differential steps come from host-built tables, so no libm call is involved.
 #include "fft_smem.cuh"
+#include "ldpc_encode.cuh"
 #include "ofdm_dev.cuh"
 #include "pu_internal.h"
 
@@ -23,16 +24,13 @@ namespace pu {
 
 struct TxDev {
     int nfft, cp, sym_len, guard, n_data, n_pilot, bps, differential;
-    int k, m;                          // LDPC dimensions
     int pre_len, n_sym, frame_len;     // preamble samples, data symbols, total samples
     int osc_start;                     // mixer position of the first data symbol (the Schmidl-Cox preamble repeats one STS and one
                                        // LTS waveform, so the mixer has only advanced by two symbols there: modulator.cpp:479-532)
     float scale;                       // ModemConfig::output_scale
     int il_inv;                        // pu_ofdm_set_tx_interleave: step^-1 mod 648 of ChannelInterleaver (bit j of a codeword is coded
                                        // bit j * il_inv mod 648), 0 = no interleaving
-    const uint8_t* cn_ninfo;           // LDPC tables in slot order (ldpc_code.h: LdpcHostTables)
-    const uint16_t* cn_check;
-    const uint16_t* cn_var;
+    LdpcEncDev enc;                    // LDPC dimensions and tables (ldpc_encode.cuh)
     const int* data_bin;
     const int* pilot_bin;
     const float* pilot_sign;
@@ -42,60 +40,20 @@ struct TxDev {
     const float2* points;              // [1 << bps] constellation points (coherent) or differential steps
 };
 
-// Shared memory of one CTA: the n_cw * 81 coded bytes packed MSB first (255 codewords: 20.7 KB), then the inverse of the parity
-// placement (parity bit r of a codeword = check p with cn_check[p] == r).
-inline size_t ofdm_tx_smem(int n_cw, int m) { return static_cast<size_t>(n_cw) * (PU_LDPC_N / 8) + static_cast<size_t>(m) * sizeof(uint16_t) + 16; }
-
+// Shared memory of one CTA: the encoder's coded frame and parity table (ldpc_encode_smem; 255 codewords take 20.7 KB of coded bytes)
 template <int NFFT>
 __global__ void __launch_bounds__(128) ofdm_tx_kernel(TxDev t, const uint8_t* __restrict__ frames, size_t frame_stride, int frame_bytes, int n_cw,
                                                       int bpc, float peak, float* __restrict__ out, size_t out_stride) {
     __shared__ float2 buf[NFFT];
     __shared__ float red[4];
     extern __shared__ __align__(16) uint8_t tx_smem[];
-    constexpr int kCwBytes = PU_LDPC_N / 8;               // 648 = 81 bytes exactly: codewords stay byte aligned back to back
     uint8_t* coded = tx_smem;
-    uint16_t* parity_of = reinterpret_cast<uint16_t*>(tx_smem + ((static_cast<size_t>(n_cw) * kCwBytes + 1) & ~size_t(1)));
     const int tid = threadIdx.x, T = blockDim.x;
     const uint8_t* fr = frames + static_cast<size_t>(blockIdx.x) * frame_stride;
     float* w = out + static_cast<size_t>(blockIdx.x) * out_stride;
 
-    // ---- v2::encodeFrameWithLDPC chunking: CW0 = frame bytes [0, bpc), CWi = {0xD5, i, bytes [bpc + (i-1)(bpc-2), ...)}, zero padded
-    // to the codeword's k information bits (bpc * 8 <= k; the bits from bpc * 8 to k are zero)
-    for (int j = tid; j < n_cw * bpc; j += T) {
-        const int i = j / bpc, q = j - i * bpc;
-        int src = q;
-        uint8_t v;
-        if (i == 0) v = q < frame_bytes ? fr[q] : 0;
-        else if (q < 2) v = q == 0 ? 0xD5 : static_cast<uint8_t>(i);
-        else { src = bpc + (i - 1) * (bpc - 2) + q - 2; v = src < frame_bytes ? fr[src] : 0; }
-        coded[i * kCwBytes + q] = v;
-    }
-    for (int p = tid; p < t.m; p += T) parity_of[t.cn_check[p]] = static_cast<uint16_t>(p);
     for (int i = tid; i < t.pre_len; i += T) w[i] = __ldg(&t.preamble[i]);
-    __syncthreads();
-    // ---- LDPCEncoder::encode of every codeword: k information bits, then parity bit r = XOR of H_data row parity_of[r]; one thread per
-    // output byte from byte bpc on (whole bytes, so no two threads write one byte)
-    const int info_bits = bpc * 8;
-    for (int j = tid; j < n_cw * (kCwBytes - bpc); j += T) {
-        const int i = j / (kCwBytes - bpc), q = bpc + (j - i * (kCwBytes - bpc));
-        const uint8_t* cw = coded + i * kCwBytes;
-        unsigned byte = 0;
-        for (int e = 0; e < 8; ++e) {
-            const int bit = q * 8 + e;
-            unsigned acc = 0;
-            if (bit >= t.k) {
-                const int p = parity_of[bit - t.k];
-                const int ninfo = t.cn_ninfo[p];
-                for (int x = 0; x < ninfo; ++x) {
-                    const int v = t.cn_var[x * t.m + p];
-                    if (v < info_bits) acc ^= (cw[v >> 3] >> (7 - (v & 7))) & 1u;
-                }
-            }
-            byte = (byte << 1) | acc;
-        }
-        coded[i * kCwBytes + q] = static_cast<uint8_t>(byte);
-    }
-    __syncthreads();
+    ldpc_encode_frame_cta(t.enc, fr, frame_bytes, n_cw, bpc, coded, ldpc_encode_parity_of(tx_smem, n_cw));
 
     const int total_bits = n_cw * PU_LDPC_N;
     const int per_sym = t.n_data * t.bps;
@@ -154,7 +112,7 @@ __global__ void __launch_bounds__(128) ofdm_tx_kernel(TxDev t, const uint8_t* __
 cudaError_t ofdm_tx_launch(const TxDev& t, const uint8_t* frames, size_t frame_stride, int frame_bytes, int n_cw, int bpc, size_t B, float peak,
                            float* out, size_t out_stride, cudaStream_t st) {
     if (B == 0) return cudaSuccess;
-    const size_t smem = ofdm_tx_smem(n_cw, t.m);
+    const size_t smem = ldpc_encode_smem(n_cw, t.enc.m);
     if (t.nfft == 512)
         ofdm_tx_kernel<512><<<static_cast<unsigned>(B), 128, smem, st>>>(t, frames, frame_stride, frame_bytes, n_cw, bpc, peak, out, out_stride);
     else

@@ -15,6 +15,7 @@
 #include <complex>
 #include <vector>
 
+#include "ldpc_encode.cuh"
 #include "ofdm_dev.cuh"
 #include "psk_handles.h"
 #include "ref_math.cuh"
@@ -25,13 +26,6 @@ namespace pu { std::vector<float> mcdpsk_carrier_freqs(const pu_mcdpsk_config& c
 namespace pu {
 
 constexpr double kTxPi = 3.14159265358979323846;   // M_PI
-
-struct LdpcEncDev {
-    int k, m;
-    const uint8_t* cn_ninfo;
-    const uint16_t* cn_check;
-    const uint16_t* cn_var;
-};
 
 // LDPCEncoder::encode of one block into bits[648]: k information bits (payload, zero padded), then the m parity bits
 __device__ __forceinline__ void encode_block(const LdpcEncDev& e, const uint8_t* __restrict__ pl, int payload_bytes, uint8_t* bits) {

@@ -129,11 +129,12 @@ struct pu_ctx {
     cudaEvent_t pipe_ev = nullptr;
     // scratch of pu_linksim_run (sweep.cu), grow-only and reused across calls: [0..6] batch buffers (rx, llr, info, ok, iters, n_llr, sync),
     // [7 + 4 s .. 10 + 4 s] slot s = {pinned descriptors, device descriptors, device counters, pinned counters},
-    // [15..17] fresh payloads {TX rows, payload rows, noise levels}, [18..19] frame modes {reassembled frames, frame_len + info + ncw}
+    // [15..17] fresh payloads {TX rows, payload rows, noise levels}, [18..19] frame modes {reassembled frames, frame_len + info + ncw},
+    // [20] coded bytes of fresh payloads (pu_linksim_run_raw)
     pu::Buffer cfo_mix;            // pu_channel_apply_cfo_batch: (cos, sin)(2 pi 1500 i / fs) per sample index, host libm
     size_t cfo_mix_len = 0;
     uint32_t cfo_mix_fs = 0;
-    pu::Buffer sweep[20];
+    pu::Buffer sweep[21];
     cudaEvent_t sweep_ev[2] = {nullptr, nullptr};
 };
 
@@ -184,6 +185,12 @@ pu_status frame_decode_enqueue(pu_ctx* ctx, pu_ldpc* dec, const float* llr, size
 pu_status count_frame_errors(pu_ctx* ctx, const uint8_t* frame_out, size_t frame_cap, const int32_t* frame_len, const int32_t* info,
                              const uint8_t* sent, size_t sent_stride, const uint32_t* tx_index, const uint32_t* bin, size_t sent_len, int n_cw,
                              size_t B, uint64_t* counters, cudaStream_t st);
+// linksim.cu: the body of pu_count_raw_errors on the caller's stream (pre-decoder counters {soft_bits, erasures, bit_errors, strong_errors}).
+// il_step != 0: the rows were deinterleaved by ChannelInterleaver(step = il_step, 648) codeword by codeword after the receiver wrote them,
+// and n_valid[b] counts soft bits in the receiver's (delivered) order, so the erasures past it are found through the permutation.
+pu_status count_raw_errors(pu_ctx* ctx, const float* llr, size_t llr_stride, size_t n_bits, const int32_t* n_valid, const uint8_t* coded,
+                           size_t coded_stride, const uint32_t* coded_index, const uint32_t* bin, size_t B, float strong, uint64_t* counters,
+                           cudaStream_t st, uint32_t il_step = 0);
 // ldpc_decode.cu: ChannelInterleaver(bits_per_symbol, 648) of pu_channel_interleaver_perm, perm[i] = i * step mod 648.  The inverse of
 // step mod 648 (transmitted bit j of a codeword is coded bit j * step^-1 mod 648), and ChannelInterleaver::interleave of n_cw packed
 // 81-byte codewords in place, each on its own.

@@ -137,7 +137,9 @@ uint64_t splitmix64(uint64_t& x) {
     return z ^ (z >> 31);
 }
 
-uint64_t desc_key(const pu_sweep_desc* d, const SweepPlan& p) {      // FNV-1a over everything that defines the frames of a unit
+// FNV-1a over everything that defines the frames of a unit, and the record format: a raw run (pu_linksim_run_raw) mixes in one more tag,
+// so that it and a plain run of the same table never resume from each other's shards; a plain run keeps the key its manifests have
+uint64_t desc_key(const pu_sweep_desc* d, const SweepPlan& p, bool raw) {
     uint64_t h = 0xcbf29ce484222325ull;
     auto mix = [&h](const void* ptr, size_t n) {
         const unsigned char* b = static_cast<const unsigned char*>(ptr);
@@ -153,6 +155,7 @@ uint64_t desc_key(const pu_sweep_desc* d, const SweepPlan& p) {      // FNV-1a o
     }
     mix(&p.pool, sizeof p.pool); mix(&p.block, sizeof p.block); mix(&p.max_iter, sizeof p.max_iter);
     mix(&p.base_seed, sizeof p.base_seed); mix(&p.trials, sizeof p.trials);
+    if (raw) mix("raw counters", 12);
     return h;
 }
 
@@ -239,6 +242,7 @@ struct ModeEngine {
     int convention = 0;
     std::vector<float> noise_std;        // [n_snr][pool]; fresh payloads: [n_snr] SNR factors of pu_channel_noise_std_batch
     Buffer d_tx, d_payload;              // [pool][L] floats, [pool][kb] bytes
+    Buffer d_coded;                      // raw counts: [pool][n_cw * 81] coded bytes of the pool, before interleaving
     bool fresh = false;                  // pu_sweep_mode.fresh_payloads: TX inside the batch
     size_t body_len = 0;                 // samples the transmitter writes per frame (L = lead + chirp + body + tail)
     size_t chirp_len = 0;                // fresh payloads of the chirp waveforms: the pair in d_chirp, written in front of every body
@@ -256,10 +260,10 @@ struct ModeEngine {
         if (mcd) pu_mcdpsk_destroy(mcd);
         if (ldpc && own_ldpc) pu_ldpc_destroy(ldpc);
         if (tools_cfo) pu_tools_cfo_destroy(tools_cfo);
-        d_tx.release(); d_payload.release(); d_chirp.release();
+        d_tx.release(); d_payload.release(); d_chirp.release(); d_coded.release();
     }
 
-    pu_status build(pu_ctx* c, const pu_sweep_mode* m, uint32_t mode_index, const SweepPlan& p, cudaStream_t st, pu_ldpc* shared_ldpc = nullptr) {
+    pu_status build(pu_ctx* c, const pu_sweep_mode* m, uint32_t mode_index, const SweepPlan& p, cudaStream_t st, pu_ldpc* shared_ldpc, bool raw) {
         ctx = c; md = m; pool = p.pool;
         pu_status s;
         const bool trace = std::getenv("PU_SWEEP_TRACE") != nullptr;
@@ -329,6 +333,7 @@ struct ModeEngine {
         // (frame modes: the payload inside DataFrame::serialize, seq i + 1 -> v2::encodeFrameWithLDPC -> all codewords modulated)
         std::vector<uint8_t> payloads(static_cast<size_t>(pool) * pay_stride, 0);
         std::vector<uint8_t> coded(static_cast<size_t>(n_cw) * (PU_LDPC_N / 8));
+        std::vector<uint8_t> coded_pool(raw ? static_cast<size_t>(pool) * coded.size() : 0);
         for (uint32_t i = 0; i < pool; ++i) {
             uint8_t* pay = payloads.data() + static_cast<size_t>(i) * pay_stride;
             size_t nc = 0;
@@ -342,6 +347,7 @@ struct ModeEngine {
                 pu_sweep_payload(p.base_seed, mode_index, i, pay, m->payload_bytes);
                 if ((s = pu_ldpc_encode(static_cast<int>(m->code_rate), pay, m->payload_bytes, coded.data(), coded.size(), &nc)) != PU_OK) return s;
             }
+            if (raw) std::copy(coded.begin(), coded.end(), coded_pool.begin() + static_cast<size_t>(i) * coded.size());
             if (m->interleave_bps) channel_interleave_codewords(m->interleave_bps, coded.data(), nc / (PU_LDPC_N / 8));
             size_t n = 0;
             std::vector<float> w;
@@ -382,7 +388,11 @@ struct ModeEngine {
         for (uint32_t i = 0; i < pool; ++i) std::copy(waves[i].begin(), waves[i].end(), flat.begin() + static_cast<size_t>(i) * L);
         PU_CUDA_TRY(cudaMemcpyAsync(d_tx.ptr, flat.data(), flat.size() * sizeof(float), cudaMemcpyHostToDevice, st));
         PU_CUDA_TRY(cudaMemcpyAsync(d_payload.ptr, payloads.data(), payloads.size(), cudaMemcpyHostToDevice, st));
-        PU_CUDA_TRY(cudaStreamSynchronize(st));       // `flat` / `payloads` are pageable and go out of scope
+        if (raw) {
+            if ((s = d_coded.reserve(coded_pool.size())) != PU_OK) return s;
+            PU_CUDA_TRY(cudaMemcpyAsync(d_coded.ptr, coded_pool.data(), coded_pool.size(), cudaMemcpyHostToDevice, st));
+        }
+        PU_CUDA_TRY(cudaStreamSynchronize(st));       // `flat` / `payloads` / `coded_pool` are pageable and go out of scope
         if (trace) fprintf(stderr, "[engine] mode %u: decoder %.3f s, demodulator %.3f s, TX pool %.3f s, noise levels + upload %.3f s\n", mode_index, secs(t0, t_ldpc),
                            secs(t_ldpc, t1), secs(t1, t2), secs(t2, now()));
         return PU_OK;
@@ -417,16 +427,41 @@ struct ModeEngine {
         return tools_cfo ? pu_tools_cfo_apply_batch(tools_cfo, out, B, L, PU_MEM_DEVICE, st) : PU_OK;
     }
 
+    // raw counts of the soft bits in llr (decoder order) against the coded bytes sent (Raw::coded row Raw::index[b]).  The acquiring
+    // receivers' n_llr (NULL for the others) marks the soft bits they did not deliver as erasures.  It counts in the receiver's order, so
+    // behind pu_llr_deinterleave_batch the counter finds the undelivered bits through the interleaver's permutation (its step).
+    struct Raw {
+        uint64_t* counters;                // [units of the batch][4]; NULL = no raw counts
+        const uint8_t* coded;
+        const uint32_t* index;
+        const uint32_t* bin;
+    };
+    pu_status count_raw(const Raw& r, const float* llr, size_t B, const int32_t* n_llr, cudaStream_t st) {
+        const size_t n = static_cast<size_t>(n_cw) * PU_LDPC_N;
+        size_t step = 0;
+        if (deinterleave) pu_channel_interleaver_perm(md->interleave_bps, PU_LDPC_N, nullptr, nullptr, &step);
+        return count_raw_errors(ctx, llr, n, n, n_llr, r.coded, n / 8, r.index, r.bin, B, 10.0f, r.counters, st, static_cast<uint32_t>(step));
+    }
+
+    // fresh payloads with raw counts: the coded bytes of the batch's payload rows, before interleaving, as the transmitter encodes them
+    pu_status encode_batch(const uint8_t* d_pay, size_t B, uint8_t* coded, cudaStream_t st) {
+        const size_t stride = static_cast<size_t>(n_cw) * (PU_LDPC_N / 8);
+        if (!frames) return pu_ldpc_encode_batch(ldpc, d_pay, kb, md->payload_bytes, B, coded, stride, PU_MEM_DEVICE, st);
+        size_t ncw = 0;
+        return pu_frame_encode_batch(ldpc, d_pay, pay_stride, frame_bytes, B, coded, stride, &ncw, PU_MEM_DEVICE, st);
+    }
+
     // frame modes: demodulate every codeword of the frame (llr [B][n_cw * 648]) -> decodeFrame (cw_* [B * n_cw] codeword scratch) ->
     // frame_out [B][frame_bytes], frame_len [B], info [B][5]; ncw [B] = codewords the acquiring receivers delivered
     pu_status receive_frames(const float* rx, size_t B, float* llr, int32_t* n_llr, int32_t* sync_i, float* sync_f, uint8_t* cw_bytes, uint8_t* cw_ok,
-                             int32_t* cw_iters, uint8_t* frame_out, int32_t* frame_len, int32_t* info, int32_t* ncw, cudaStream_t st) {
+                             int32_t* cw_iters, uint8_t* frame_out, int32_t* frame_len, int32_t* info, int32_t* ncw, const Raw& raw, cudaStream_t st) {
         pu_status s = PU_OK;
         const size_t stride = static_cast<size_t>(n_cw) * PU_LDPC_N;
         const unsigned wf = md->waveform;
         if (wf == PU_WF_OFDM) {
             if ((s = pu_ofdm_presynced_batch(ofdm, rx, B, L, 2, nullptr, nullptr, llr, stride, nullptr, nullptr, PU_MEM_DEVICE, st)) != PU_OK) return s;
             ncw = nullptr;
+            n_llr = nullptr;
         } else {
             PU_CUDA_TRY(cudaMemsetAsync(llr, 0, B * stride * sizeof(float), st));
             if (wf == PU_WF_OFDM_SC)
@@ -439,17 +474,26 @@ struct ModeEngine {
             PU_CUDA_TRY(cudaGetLastError());
         }
         if (deinterleave && (s = llr_deinterleave_enqueue(ctx, llr, B, stride, n_cw, md->interleave_bps, st)) != PU_OK) return s;
+        if (raw.counters && (s = count_raw(raw, llr, B, n_llr, st)) != PU_OK) return s;
         return frame_decode_enqueue(ctx, ldpc, llr, B, static_cast<int>(n_cw), ncw, cw_bytes, cw_ok, cw_iters, frame_out, frame_bytes, frame_len, info, st);
     }
 
     // demodulate -> decode (device pointers, stream st); scratch: llr [B][648], n_llr [B], sync [B][8] (int/float)
     pu_status receive(const float* rx, size_t B, float* llr, int32_t* n_llr, int32_t* sync_i, float* sync_f, uint8_t* info, uint8_t* ok, int32_t* iters,
-                      cudaStream_t st) {
+                      const Raw& raw, cudaStream_t st) {
         pu_status s = PU_OK;
         bool mask = false;
         const unsigned wf = md->waveform;
-        if (wf == PU_WF_OFDM)
+        if (wf == PU_WF_OFDM && !raw.counters)
             return pu_receive_decode_batch(ofdm, ldpc, rx, B, L, 2, nullptr, nullptr, info, kb, ok, iters, PU_MEM_DEVICE, st);
+        if (wf == PU_WF_OFDM) {          // the two halves of pu_receive_decode_batch's device path, with the soft bits counted in between
+            const int n_sym = static_cast<int>(L / static_cast<size_t>(pu_ofdm_symbol_samples(ofdm)));
+            if (static_cast<size_t>(std::max(0, n_sym - 2)) * static_cast<size_t>(pu_ofdm_bits_per_symbol(ofdm)) < PU_LDPC_N)
+                PU_CUDA_TRY(cudaMemsetAsync(llr, 0, B * PU_LDPC_N * sizeof(float), st));   // frames shorter than a codeword: erasures
+            if ((s = pu_ofdm_presynced_batch(ofdm, rx, B, L, 2, nullptr, nullptr, llr, PU_LDPC_N, nullptr, nullptr, PU_MEM_DEVICE, st)) != PU_OK) return s;
+            if ((s = count_raw(raw, llr, B, nullptr, st)) != PU_OK) return s;
+            return pu_ldpc_decode_batch(ldpc, llr, PU_LDPC_N, B, info, kb, ok, iters, PU_MEM_DEVICE, st);
+        }
         if (wf != PU_WF_DPSK && wf != PU_WF_MCDPSK) PU_CUDA_TRY(cudaMemsetAsync(llr, 0, B * PU_LDPC_N * sizeof(float), st));
         switch (wf) {
             case PU_WF_OFDM_SC:
@@ -473,6 +517,7 @@ struct ModeEngine {
         }
         if (s != PU_OK) return s;
         if (deinterleave && (s = llr_deinterleave_enqueue(ctx, llr, B, PU_LDPC_N, 1, md->interleave_bps, st)) != PU_OK) return s;
+        if (raw.counters && (s = count_raw(raw, llr, B, mask ? n_llr : nullptr, st)) != PU_OK) return s;
         if ((s = pu_ldpc_decode_batch(ldpc, llr, PU_LDPC_N, B, info, kb, ok, iters, PU_MEM_DEVICE, st)) != PU_OK) return s;
         if (mask) {
             mask_short_kernel<<<static_cast<unsigned>((B + 255) / 256), 256, 0, st>>>(ok, n_llr, B);
@@ -490,7 +535,9 @@ struct Manifest {
     ~Manifest() { if (f) fclose(f); }
 
     // reads every shard of `dir`; returns false on a key mismatch
-    bool load(const std::string& d, uint64_t key, uint64_t run_id, uint64_t n_units, std::vector<uint8_t>& done, std::vector<uint64_t>& rec /* [n_units][6] */) {
+    // nc = counters per record: 6, or 10 in a raw run (the 6, then the 4 raw counters)
+    bool load(const std::string& d, uint64_t key, uint64_t run_id, uint64_t n_units, int nc, std::vector<uint8_t>& done,
+              std::vector<uint64_t>& rec /* [n_units][nc] */) {
         dir = d;
         char own[64];
         snprintf(own, sizeof own, "shard-%016llx-", static_cast<unsigned long long>(run_id));
@@ -506,17 +553,20 @@ struct Manifest {
             if (!in) continue;
             char line[256];
             while (fgets(line, sizeof line, in)) {
-                unsigned long long k = 0, u = 0, c[6];
+                unsigned long long k = 0, u = 0, c[10];
                 if (line[0] == '#') {
                     if (sscanf(line, "# key %llx", &k) == 1 && k != key) ok = false;
                     continue;
                 }
-                // a torn last line (killed while appending) does not parse to 7 fields + the end mark and is ignored
+                // a torn last line (killed while appending) does not parse to 1 + nc fields + the end mark and is ignored
                 char endmark = 0;
-                if (sscanf(line, "%llu %llu %llu %llu %llu %llu %llu %c", &u, &c[0], &c[1], &c[2], &c[3], &c[4], &c[5], &endmark) != 8 || endmark != ';') continue;
+                const int got = nc == 6 ? sscanf(line, "%llu %llu %llu %llu %llu %llu %llu %c", &u, &c[0], &c[1], &c[2], &c[3], &c[4], &c[5], &endmark)
+                                        : sscanf(line, "%llu %llu %llu %llu %llu %llu %llu %llu %llu %llu %llu %c", &u, &c[0], &c[1], &c[2], &c[3], &c[4],
+                                                 &c[5], &c[6], &c[7], &c[8], &c[9], &endmark);
+                if (got != nc + 2 || endmark != ';') continue;
                 if (u >= n_units || done[u]) continue;
                 done[u] = 1;
-                for (int i = 0; i < 6; ++i) rec[u * 6 + i] = c[i];
+                for (int i = 0; i < nc; ++i) rec[u * nc + i] = c[i];
             }
             fclose(in);
         }
@@ -532,10 +582,12 @@ struct Manifest {
         fflush(f);
         return true;
     }
-    void append(uint64_t unit, const uint64_t* c) {
+    void append(uint64_t unit, const uint64_t* c, const uint64_t* raw /* NULL in a plain run */) {
         if (!f) return;
-        fprintf(f, "%llu %llu %llu %llu %llu %llu %llu ;\n", (unsigned long long)unit, (unsigned long long)c[0], (unsigned long long)c[1],
+        fprintf(f, "%llu %llu %llu %llu %llu %llu %llu", (unsigned long long)unit, (unsigned long long)c[0], (unsigned long long)c[1],
                 (unsigned long long)c[2], (unsigned long long)c[3], (unsigned long long)c[4], (unsigned long long)c[5]);
+        if (raw) fprintf(f, " %llu %llu %llu %llu", (unsigned long long)raw[0], (unsigned long long)raw[1], (unsigned long long)raw[2], (unsigned long long)raw[3]);
+        fprintf(f, " ;\n");
     }
     void flush() { if (f) fflush(f); }
 };
@@ -646,6 +698,10 @@ void pu_wilson_interval(uint64_t errors, uint64_t n, double z, double* lo, doubl
 }
 
 pu_status pu_linksim_run(pu_ctx* ctx, const pu_sweep_desc* d, uint64_t* counters, pu_sweep_stats* stats) {
+    return pu_linksim_run_raw(ctx, d, counters, nullptr, stats);
+}
+
+pu_status pu_linksim_run_raw(pu_ctx* ctx, const pu_sweep_desc* d, uint64_t* counters, uint64_t* raw, pu_sweep_stats* stats) {
     PU_REQUIRE(ctx && d && counters, "pu_linksim_run: NULL argument");
     pu::SweepPlan p;
     PU_REQUIRE(pu::make_plan(d, &p), "pu_linksim_run: invalid sweep description");
@@ -654,6 +710,8 @@ pu_status pu_linksim_run(pu_ctx* ctx, const pu_sweep_desc* d, uint64_t* counters
     const uint64_t n_units = p.unit0.back();
     const uint32_t n_points = p.point0.back();
     std::fill(counters, counters + static_cast<size_t>(n_points) * 6, uint64_t(0));
+    if (raw) std::fill(raw, raw + static_cast<size_t>(n_points) * 4, uint64_t(0));
+    const int nc = raw ? 10 : 6;          // counters per unit: the 6, then the 4 raw counters of a raw run
     pu_sweep_stats stt{};
     stt.units_total = n_units;
 
@@ -661,10 +719,10 @@ pu_status pu_linksim_run(pu_ctx* ctx, const pu_sweep_desc* d, uint64_t* counters
     std::vector<uint8_t> done(n_units, 0);
     std::vector<uint64_t> rec;
     pu::Manifest man;
-    const uint64_t key = pu::desc_key(d, p);
+    const uint64_t key = pu::desc_key(d, p, raw != nullptr);
     if (d->manifest_dir && d->manifest_dir[0]) {
-        rec.assign(n_units * 6, 0);
-        if (!man.load(d->manifest_dir, key, d->run_id, n_units, done, rec)) {
+        rec.assign(n_units * nc, 0);
+        if (!man.load(d->manifest_dir, key, d->run_id, n_units, nc, done, rec)) {
             pu::set_error("pu_linksim_run: %s holds the manifest of a different sweep (key mismatch); use an empty directory", d->manifest_dir);
             return PU_ERR_INVALID;
         }
@@ -678,7 +736,9 @@ pu_status pu_linksim_run(pu_ctx* ctx, const pu_sweep_desc* d, uint64_t* counters
             if (d->rank != 0) continue;        // resumed counters enter the job total once
             uint32_t m, s, nt; uint64_t t0;
             pu::unit_decode(d, p, u, &m, &s, &t0, &nt);
-            for (int i = 0; i < 6; ++i) counters[(p.point0[m] + s) * 6 + i] += rec[u * 6 + i];
+            for (int i = 0; i < 6; ++i) counters[(p.point0[m] + s) * 6 + i] += rec[u * nc + i];
+            if (raw)
+                for (int i = 0; i < 4; ++i) raw[(p.point0[m] + s) * 4 + i] += rec[u * nc + 6 + i];
         }
     }
     std::vector<uint32_t> owner(n_units);
@@ -691,7 +751,7 @@ pu_status pu_linksim_run(pu_ctx* ctx, const pu_sweep_desc* d, uint64_t* counters
     pu::Slot slots[2];
     pu::Buffer &d_rx = ctx->sweep[0], &d_llr = ctx->sweep[1], &d_info = ctx->sweep[2], &d_ok = ctx->sweep[3], &d_iters = ctx->sweep[4],
                &d_nllr = ctx->sweep[5], &d_sync = ctx->sweep[6], &d_ftx = ctx->sweep[15], &d_fpay = ctx->sweep[16], &d_fstd = ctx->sweep[17],
-               &d_fout = ctx->sweep[18], &d_finfo = ctx->sweep[19];
+               &d_fout = ctx->sweep[18], &d_finfo = ctx->sweep[19], &d_fcoded = ctx->sweep[20];
     for (int i = 0; i < 2; ++i) {
         pu::Slot& sl = slots[i];
         sl.h_desc = &ctx->sweep[7 + 4 * i]; sl.d_desc = &ctx->sweep[8 + 4 * i]; sl.d_cnt = &ctx->sweep[9 + 4 * i]; sl.h_cnt = &ctx->sweep[10 + 4 * i];
@@ -711,11 +771,14 @@ pu_status pu_linksim_run(pu_ctx* ctx, const pu_sweep_desc* d, uint64_t* counters
         PU_CUDA_TRY(cudaEventSynchronize(sl.ev));
         stt.wait_seconds += std::chrono::duration<double>(std::chrono::steady_clock::now() - t_wait).count();
         const uint64_t* hc = static_cast<const uint64_t*>(sl.h_cnt->ptr);
+        const uint64_t* hr = hc + sl.units.size() * 6;      // raw counters [units][4] behind the [units][6]
         for (size_t i = 0; i < sl.units.size(); ++i) {
             uint32_t m, s, nt; uint64_t t0;
             pu::unit_decode(d, p, sl.units[i], &m, &s, &t0, &nt);
             for (int k = 0; k < 6; ++k) counters[(p.point0[m] + s) * 6 + k] += hc[i * 6 + k];
-            man.append(sl.units[i], hc + i * 6);
+            if (raw)
+                for (int k = 0; k < 4; ++k) raw[(p.point0[m] + s) * 4 + k] += hr[i * 4 + k];
+            man.append(sl.units[i], hc + i * 6, raw ? hr + i * 4 : nullptr);
         }
         man.flush();
         stt.units_run += sl.units.size();
@@ -738,7 +801,7 @@ pu_status pu_linksim_run(pu_ctx* ctx, const pu_sweep_desc* d, uint64_t* counters
         const auto t_setup = std::chrono::steady_clock::now();
         const unsigned rate = d->modes[m].code_rate;      // one decoder per code rate for the whole run (its tables take longer to build than a mode's)
         if (rate < 8 && !decoders[rate] && (rs = pu_ldpc_create(ctx, static_cast<int>(rate), static_cast<int>(p.max_iter), &decoders[rate])) != PU_OK) break;
-        if ((rs = eng.build(ctx, &d->modes[m], m, p, st, rate < 8 ? decoders[rate] : nullptr)) != PU_OK) break;
+        if ((rs = eng.build(ctx, &d->modes[m], m, p, st, rate < 8 ? decoders[rate] : nullptr, raw != nullptr)) != PU_OK) break;
         const double t_build = std::chrono::duration<double>(std::chrono::steady_clock::now() - t_setup).count();
         stt.setup_seconds += t_build;
         if (std::getenv("PU_SWEEP_TRACE"))
@@ -756,6 +819,7 @@ pu_status pu_linksim_run(pu_ctx* ctx, const pu_sweep_desc* d, uint64_t* counters
         if (eng.fresh && ((rs = d_ftx.reserve(cap * L * sizeof(float))) != PU_OK || (rs = d_fpay.reserve(cap * eng.pay_stride)) != PU_OK ||
                           (rs = d_fstd.reserve(cap * sizeof(float))) != PU_OK))
             break;
+        if (eng.fresh && raw && (rs = d_fcoded.reserve(cap * ncw * (PU_LDPC_N / 8))) != PU_OK) break;
         // frame modes: reassembled frames; frame_len [cap], info [cap][5], codewords delivered [cap]
         if (eng.frames && ((rs = d_fout.reserve(cap * eng.frame_bytes)) != PU_OK || (rs = d_finfo.reserve(cap * 7 * sizeof(int32_t))) != PU_OK))
             break;
@@ -781,7 +845,7 @@ pu_status pu_linksim_run(pu_ctx* ctx, const pu_sweep_desc* d, uint64_t* counters
             // descriptors: tx_index u32 | noise_std f32 | bin u32 | seed u64 (8-byte aligned at the end)
             const size_t off_std = B * 4, off_bin = B * 8, off_seed = ((B * 12 + 7) / 8) * 8, desc_bytes = off_seed + B * 8;
             if ((rs = sl.h_desc->reserve(desc_bytes)) != PU_OK || (rs = sl.d_desc->reserve(desc_bytes)) != PU_OK ||
-                (rs = sl.d_cnt->reserve(nu * 6 * 8)) != PU_OK || (rs = sl.h_cnt->reserve(nu * 6 * 8)) != PU_OK)
+                (rs = sl.d_cnt->reserve(nu * nc * 8)) != PU_OK || (rs = sl.h_cnt->reserve(nu * nc * 8)) != PU_OK)
                 break;
             unsigned char* hd = static_cast<unsigned char*>(sl.h_desc->ptr);
             uint32_t* h_tx = reinterpret_cast<uint32_t*>(hd);
@@ -810,11 +874,12 @@ pu_status pu_linksim_run(pu_ctx* ctx, const pu_sweep_desc* d, uint64_t* counters
             unsigned char* dd = static_cast<unsigned char*>(sl.d_desc->ptr);
             auto launch = [&]() -> pu_status {
                 PU_CUDA_TRY(cudaMemcpyAsync(dd, hd, desc_bytes, cudaMemcpyHostToDevice, st));
-                PU_CUDA_TRY(cudaMemsetAsync(sl.d_cnt->ptr, 0, nu * 6 * 8, st));
+                PU_CUDA_TRY(cudaMemsetAsync(sl.d_cnt->ptr, 0, nu * nc * 8, st));
                 float* rx = static_cast<float*>(d_rx.ptr);
                 const float* tx_pool = static_cast<const float*>(eng.d_tx.ptr);
                 const float* stds = reinterpret_cast<const float*>(dd + off_std);
                 const uint8_t* payloads = static_cast<const uint8_t*>(eng.d_payload.ptr);
+                const uint8_t* coded = static_cast<const uint8_t*>(eng.d_coded.ptr);
                 size_t pool_count = eng.pool;
                 pu_status s2;
                 if (eng.fresh) {                 // payload -> encode -> modulate for every frame of the batch, then its own noise level
@@ -830,6 +895,8 @@ pu_status pu_linksim_run(pu_ctx* ctx, const pu_sweep_desc* d, uint64_t* counters
                     }
                     ctx->launches.fetch_add(1);
                     PU_CUDA_TRY(cudaGetLastError());
+                    if (raw && (s2 = eng.encode_batch(pay, B, static_cast<uint8_t*>(d_fcoded.ptr), st)) != PU_OK) return s2;
+                    if (raw) coded = static_cast<const uint8_t*>(d_fcoded.ptr);
                     if (d->modes[m].lead_samples || d->modes[m].tail_samples) PU_CUDA_TRY(cudaMemsetAsync(ftx, 0, B * L * sizeof(float), st));
                     if ((s2 = eng.tx_batch(pay, B, ftx, L, st)) != PU_OK) return s2;
                     if ((s2 = eng.finish_rows(ftx, B, st)) != PU_OK) return s2;
@@ -845,24 +912,25 @@ pu_status pu_linksim_run(pu_ctx* ctx, const pu_sweep_desc* d, uint64_t* counters
                 const uint32_t* tx_index = reinterpret_cast<const uint32_t*>(dd);
                 const uint32_t* bins = reinterpret_cast<const uint32_t*>(dd + off_bin);
                 uint64_t* cnt = static_cast<uint64_t*>(sl.d_cnt->ptr);
+                const pu::ModeEngine::Raw rw{raw ? cnt + nu * 6 : nullptr, coded, tx_index, bins};
                 if (eng.frames) {
                     uint8_t* fout = static_cast<uint8_t*>(d_fout.ptr);
                     int32_t* flen = static_cast<int32_t*>(d_finfo.ptr);
                     int32_t* finfo = flen + cap;
                     s2 = eng.receive_frames(rx, B, static_cast<float*>(d_llr.ptr), static_cast<int32_t*>(d_nllr.ptr), static_cast<int32_t*>(d_sync.ptr),
                                             reinterpret_cast<float*>(static_cast<int32_t*>(d_sync.ptr) + 4 * cap), info, ok, iters, fout, flen, finfo,
-                                            finfo + 5 * cap, st);
+                                            finfo + 5 * cap, rw, st);
                     if (s2 != PU_OK) return s2;
                     s2 = pu::count_frame_errors(ctx, fout, eng.frame_bytes, flen, finfo, payloads, eng.pay_stride, tx_index, bins, eng.frame_bytes,
                                                 static_cast<int>(ncw), B, cnt, st);
                 } else {
                     s2 = eng.receive(rx, B, static_cast<float*>(d_llr.ptr), static_cast<int32_t*>(d_nllr.ptr), static_cast<int32_t*>(d_sync.ptr),
-                                     reinterpret_cast<float*>(static_cast<int32_t*>(d_sync.ptr) + 4 * cap), info, ok, iters, st);
+                                     reinterpret_cast<float*>(static_cast<int32_t*>(d_sync.ptr) + 4 * cap), info, ok, iters, rw, st);
                     if (s2 != PU_OK) return s2;
                     s2 = pu_count_errors(ctx, info, kb, ok, iters, payloads, kb, tx_index, bins, d->modes[m].payload_bytes, B, cnt, st);
                 }
                 if (s2 != PU_OK) return s2;
-                PU_CUDA_TRY(cudaMemcpyAsync(sl.h_cnt->ptr, sl.d_cnt->ptr, nu * 6 * 8, cudaMemcpyDeviceToHost, st));
+                PU_CUDA_TRY(cudaMemcpyAsync(sl.h_cnt->ptr, sl.d_cnt->ptr, nu * nc * 8, cudaMemcpyDeviceToHost, st));
                 PU_CUDA_TRY(cudaEventRecord(sl.ev, st));
                 return PU_OK;
             };

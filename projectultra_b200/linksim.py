@@ -13,6 +13,10 @@ import numpy as np
 from . import capi
 
 COUNTER_NAMES = ("frames", "frame_errors", "bit_errors", "bits", "decode_failures", "iteration_sum")
+# pre-decoder counters of the soft bits the decoder is given (capi.count_raw_errors, pu_linksim_run_raw): soft bits, erasures (+-0, or not
+# delivered by an acquiring receiver), hard-decision errors among the rest, and those of them with |llr| >= RAW_STRONG
+RAW_COUNTER_NAMES = ("soft_bits", "erasures", "bit_errors", "strong_errors")
+RAW_STRONG = 10.0          # the clipLLR bound of the OFDM demappers and the clamp of the MC-DPSK demapper
 
 
 class ChannelConfig(C.Structure):
@@ -121,6 +125,26 @@ def interleave_codewords(coded, bps):
     return np.packbits(out, axis=1).reshape(-1)
 
 
+def erase_undelivered(llr, n_valid, n_bits, bps):
+    """llr[:, :n_bits] (decoder order, behind ChannelInterleaver(bps, 648)::deinterleave of every codeword) with +0 at every soft bit the
+    receiver did not deliver: n_valid[b] counts soft bits in the receiver's order, and decoder bit c * 648 + i came from its position
+    c * 648 + perm[i] (out[perm[i]] = in[i] on the transmit side).  A copy; the decoder's input stays as it is."""
+    import torch
+    perm = torch.from_numpy(capi.channel_interleaver_perm(bps)[0].astype(np.int64)).to(llr.device)
+    pos = (torch.arange(n_bits // 648, device=llr.device)[:, None] * 648 + perm[None, :]).reshape(-1)
+    out = llr[:, :n_bits].clone()
+    out[pos[None, :] >= n_valid.to(torch.int64)[:, None]] = 0.0
+    return out
+
+
+def count_raw(ctx, llr, coded, raw, n_bits, n_valid, index, bins, bps):
+    """Raw counts of soft bits in decoder order; n_valid (None = all delivered) counts the soft bits the receiver delivered in ITS order,
+    which a deinterleaver (bps > 0) permutes: the undelivered ones are then zeroed in a copy (erase_undelivered) before counting."""
+    if n_valid is not None and bps:
+        llr, n_valid = erase_undelivered(llr, n_valid, n_bits, bps), None
+    capi.count_raw_errors(ctx, llr, coded, raw, n_bits, n_valid, index, bins, RAW_STRONG)
+
+
 def wilson_interval(errors, n, z=1.96):
     """Wilson score interval for an error rate (the Monte-Carlo confidence interval of the north star)."""
     if n == 0:
@@ -147,7 +171,11 @@ class LinkSim:
     OFDM receiver deinterleaves in its LLR write (set_deinterleave), every other receiver through capi.llr_deinterleave_batch.
 
     Frames are identified by (snr index, trial index); frame -> (tx waveform, seed) is a pure function, so any
-    frame can be regenerated, and ranks take disjoint trial ranges with no data exchange (SURVEY §8e)."""
+    frame can be regenerated, and ranks take disjoint trial ranges with no data exchange (SURVEY §8e).
+
+    raw: an int64 [n_snr, 4] device tensor given to run_batch / receive_count accumulates RAW_COUNTER_NAMES of the soft bits the decoder
+    gets against the coded bits sent (the pool's coded bytes before interleaving, or pu_ldpc_encode_batch of the fresh payloads), as
+    pu_linksim_run_raw counts them; the presynced OFDM receiver then runs demodulator and decoder as two calls."""
 
     def __init__(self, ctx, cfg, channel="awgn", payload_bytes=40, pool=64, snr_convention=None, pool_seed=12345,
                  max_iter=50, device=None, code_rate=None, peak=None, layout="presynced", chunk=960, fresh_payload=False,
@@ -230,6 +258,7 @@ class LinkSim:
         self.payloads = (rng.integers(0, 256, (pool, payload_bytes), dtype=np.uint8) if payloads is None
                          else np.ascontiguousarray(payloads, dtype=np.uint8).reshape(pool, payload_bytes))
         coded = [capi.ldpc_encode(rate, p) for p in self.payloads]
+        self.coded_pool = torch.from_numpy(np.stack(coded)).to(self.device)      # [pool, 81], before interleaving: raw counts
         if self.interleave_bps:
             coded = [interleave_codewords(c, self.interleave_bps) for c in coded]
         waves = [np.pad(build(c), (self.lead, self.tail)) for c in coded]
@@ -275,6 +304,15 @@ class LinkSim:
             self.last_n_llr, self.last_sync, self.last_cfo = out[1], out[2], out[4]
             return out[0]
         return self.demod.demod_soft_batch(rx, llr_stride=648, llr=llr, want_cfo=False)[0]
+
+    def _acquiring(self):
+        return self.layout in ("sc", "chirp") or (self.kind == "dpsk" and self.acquire)
+
+    def count_raw(self, llr, coded, index, bins, raw):
+        """Raw counts of the first 648 soft bits of every row (decoder order); an acquiring receiver's n_llr marks the soft bits it did not
+        deliver as erasures."""
+        count_raw(self.ctx, llr, coded, raw, 648, self.last_n_llr if self._acquiring() else None, index, bins,
+                  0 if self.kind == "ofdm" and self.layout == "presynced" else self.interleave_bps)
 
     def noise_std_table(self, snr_points):
         key = tuple(float(s) for s in snr_points)
@@ -337,56 +375,70 @@ class LinkSim:
                                                          C.c_void_p(torch.cuda.current_stream().cuda_stream)))
         return payload, tx, std
 
-    def run_batch(self, batch, counters, rx=None, keep=False, snr_points=None):
-        """channel -> demod -> LDPC -> counters for one prepared batch (all on the current stream)."""
+    def run_batch(self, batch, counters, rx=None, keep=False, snr_points=None, raw=None):
+        """channel -> demod -> LDPC -> counters (and raw counts into `raw`) for one prepared batch (all on the current stream)."""
         if self.fresh_payload:
             import torch
             assert snr_points is not None, "fresh-payload batches need the SNR table to set each frame's noise level"
             payload, tx, std = self.fresh_frames(batch, snr_points)
             idx = torch.arange(tx.shape[0], dtype=torch.int32, device=self.device)
             rx = channel_apply(self.ctx, self.ch, tx, idx, std, batch["seed"], rx)
-            if self.kind == "ofdm" and self.layout == "presynced":
+            coded = self.ldpc.encode_batch(payload[:, :self.payload_bytes]) if raw is not None else None
+            if self.kind == "ofdm" and self.layout == "presynced" and raw is None:
                 info, ok, iters = receive_decode(self.ofdm, self.ldpc, rx)
+            elif self.kind == "ofdm" and self.layout == "presynced":
+                llr = self.demod.presynced_batch(rx, 2, llr_stride=648, want_aux=False)[0]
+                capi.count_raw_errors(self.ctx, llr, coded, raw, 648, None, None, batch["bins"], RAW_STRONG)
+                info, ok, iters = self.ldpc.decode_batch(llr)
             else:
-                info, ok, iters = self.ldpc.decode_batch(self.demod_llr(rx))
+                llr = self.demod_llr(rx)
+                if raw is not None:
+                    self.count_raw(llr, coded, None, batch["bins"], raw)
+                info, ok, iters = self.ldpc.decode_batch(llr)
                 if self.layout in ("sc", "chirp") or (self.kind == "dpsk" and self.acquire):
                     ok = ok * (self.last_n_llr >= 648).to(ok.dtype)
             count_errors(self.ctx, info, ok, iters, payload, idx, batch["bins"], self.payload_bytes, counters)
             self.last_payload, self.last_tx, self.last_std = payload, tx, std
             return (rx, info, ok, iters) if keep else None
         rx = self.make_rx(batch, rx)
-        info, ok, iters = self.receive_count(batch, rx, counters)
+        info, ok, iters = self.receive_count(batch, rx, counters, raw=raw)
         return (rx, info, ok, iters) if keep else None
 
     def make_rx(self, batch, rx=None):
         """Channel outputs of a prepared batch (pool waveforms): pu_channel_apply_batch on the current stream."""
         return channel_apply(self.ctx, self.ch, self.tx_pool, batch["tx_index"], batch["noise_std"], batch["seed"], rx)
 
-    def receive_count(self, batch, rx, counters, ev=None, bufs=None):
+    def receive_count(self, batch, rx, counters, ev=None, bufs=None, raw=None):
         """demod -> LDPC -> counters for channel outputs `rx` of `batch`.  ev: optional list of >= 4 CUDA events recorded before the
         demodulator, between demodulator and decoder, behind the decoder and behind the counting kernel (bench.py's per-stage times).
-        bufs: optional dict of preallocated device tensors {llr, info, ok, iters}."""
+        bufs: optional dict of preallocated device tensors {llr, info, ok, iters}.  raw: optional int64 [n_snr, 4] device tensor of
+        RAW_COUNTER_NAMES, accumulated in place (the soft bits are counted between demodulator and decoder)."""
         bufs = bufs or {}
         rec = (lambda i: ev[i].record()) if ev is not None else (lambda i: None)
+        count_raw = ((lambda llr: self.count_raw(llr, self.coded_pool, batch["tx_index"], batch["bins"], raw)) if raw is not None
+                     else (lambda llr: None))
         rec(0)
         if self.kind == "ofdm" and self.layout in ("sc", "chirp"):
             # no sync or fewer than 648 soft bits is a lost frame (tools/test_mode_snr.cpp:72-77): the decoder's verdict on
             # the zero-filled row is overridden
             llr = self.demod_llr(rx)
+            count_raw(llr)
             rec(1)
             info, ok, iters = self.ldpc.decode_batch(llr, bufs.get("info"), bufs.get("ok"), bufs.get("iters"))
             ok = ok * (self.last_n_llr >= 648).to(ok.dtype)
-        elif self.kind == "ofdm" and ev is None and not bufs:
+        elif self.kind == "ofdm" and ev is None and not bufs and raw is None:
             info, ok, iters = receive_decode(self.ofdm, self.ldpc, rx)
         elif self.kind == "ofdm":
             llr = bufs.get("llr")
             if llr is not None and self.ofdm.n_llr(rx.shape[1]) < 648:
                 llr.zero_()                                              # frames shorter than a codeword: erasures
             llr = self.demod.presynced_batch(rx, 2, llr_stride=648, llr=llr, want_aux=False)[0]
+            count_raw(llr)
             rec(1)
             info, ok, iters = self.ldpc.decode_batch(llr, bufs.get("info"), bufs.get("ok"), bufs.get("iters"))
         else:
             llr = self.demod_llr(rx, bufs.get("llr"))
+            count_raw(llr)
             rec(1)
             info, ok, iters = self.ldpc.decode_batch(llr, bufs.get("info"), bufs.get("ok"), bufs.get("iters"))
             if (self.kind == "dpsk" and self.acquire) or (self.kind == "mcdpsk" and self.layout == "chirp"):
@@ -397,18 +449,19 @@ class LinkSim:
         rec(3)
         return info, ok, iters
 
-    def sweep(self, snr_points, trials_per_point, rank=0, world=1, batch_frames=1 << 15, base_seed=0xB200):
+    def sweep(self, snr_points, trials_per_point, rank=0, world=1, batch_frames=1 << 15, base_seed=0xB200, raw=False):
         """FER/BER sweep; this rank takes trials t with t % world == rank.  Returns an int64 [n_snr, 6] device tensor
-        holding THIS rank's counters (all-reduce it with torch.distributed for the job total)."""
+        holding THIS rank's counters (all-reduce it with torch.distributed for the job total); raw=True returns (counters, raw [n_snr, 4])."""
         import torch
         counters = torch.zeros((len(snr_points), 6), dtype=torch.int64, device=self.device)
+        table = torch.zeros((len(snr_points), 4), dtype=torch.int64, device=self.device) if raw else None
         mine = np.arange(rank, trials_per_point, world, dtype=np.int64)
         si = np.repeat(np.arange(len(snr_points), dtype=np.int64), len(mine))
         tr = np.tile(mine, len(snr_points))
         for off in range(0, len(si), batch_frames):
             b = self.make_batch(snr_points, si[off:off + batch_frames], tr[off:off + batch_frames], base_seed)
-            self.run_batch(b, counters, snr_points=snr_points)
-        return counters
+            self.run_batch(b, counters, snr_points=snr_points, raw=table)
+        return (counters, table) if raw else counters
 
 
 FRAME_COUNTER_NAMES = ("frames", "frame_errors", "codewords_failed", "codewords", "header_failures", "unused")
@@ -452,7 +505,9 @@ class FrameLinkSim:
     counters [n_snr, 6] = FRAME_COUNTER_NAMES.  payloads: explicit [pool, payload_bytes] array (e.g. the sweep driver's pool,
     capi.Sweep.payload; frame i then carries seq i + 1 as there); peak: the tools' peak normalisation of every TX waveform; interleave_bps > 0:
     ChannelInterleaver(interleave_bps, 648) on every codeword (interleave_codewords before modulating, capi.llr_deinterleave_batch on the
-    soft bits of all codewords before decodeFrame), as the sweep driver's frame modes do."""
+    soft bits of all codewords before decodeFrame), as the sweep driver's frame modes do.  raw: an int64 [n_snr, 4] device tensor given to
+    run_batch accumulates RAW_COUNTER_NAMES over all n_cw * 648 soft bits of every frame (codewords the receiver did not deliver are
+    erasures)."""
 
     def __init__(self, ctx, cfg, channel="awgn", payload_bytes=200, pool=16, pool_seed=12345, max_iter=50, precision="exact", code_rate=None,
                  payloads=None, peak=None, interleave_bps=0, layout="presynced", lead_samples=0, tail_samples=0):
@@ -477,6 +532,7 @@ class FrameLinkSim:
             payloads = np.ascontiguousarray(payloads, dtype=np.uint8).reshape(pool, payload_bytes)
         self.frames_host = [v2_data_frame(payloads[i], self.rate, seq=i + 1) for i in range(pool)]
         cws = [capi.frame_encode(self.rate, f) for f in self.frames_host]
+        self.coded_pool = torch.from_numpy(np.stack([c.reshape(-1) for c in cws])).to(self.device)    # before interleaving: raw counts
         self.interleave_bps = int(interleave_bps)
         if self.interleave_bps:
             cws = [interleave_codewords(c, self.interleave_bps).reshape(c.shape) for c in cws]
@@ -508,8 +564,8 @@ class FrameLinkSim:
         return dict(tx_index=to(tx_index.view(np.int32), np.int32), noise_std=to(std, np.float32), seed=to(seeds.view(np.int64), np.int64),
                     bins=to(snr_idx, np.int64), host=dict(tx_index=tx_index, noise_std=std, seed=seeds, snr_idx=snr_idx))
 
-    def run_batch(self, batch, counters, keep=False):
-        """channel -> demod (every codeword of the frame) -> decodeFrame -> counters, on the current stream."""
+    def run_batch(self, batch, counters, keep=False, raw=None):
+        """channel -> demod (every codeword of the frame) -> decodeFrame -> counters (and raw counts into `raw`), on the current stream."""
         import torch
         rx = channel_apply(self.ctx, self.ch, self.tx_pool, batch["tx_index"], batch["noise_std"], batch["seed"])
         if self.layout == "chirp":
@@ -518,6 +574,9 @@ class FrameLinkSim:
             llr = self.ofdm.presynced_batch(rx, 2, llr_stride=self.n_cw * 648, want_aux=False)[0]
         if self.interleave_bps:
             capi.llr_deinterleave_batch(self.ctx, llr, self.n_cw, self.interleave_bps)
+        if raw is not None:       # soft bits the chirp receiver did not deliver are erasures
+            count_raw(self.ctx, llr, self.coded_pool, raw, self.n_cw * 648, n_llr if self.layout == "chirp" else None, batch["tx_index"],
+                      batch["bins"].to(torch.int32), self.interleave_bps)
         frames, flen, info = self.ldpc.frame_decode_batch(llr, self.n_cw, frame_cap=self.frame_len)
         want = self.frame_pool[batch["tx_index"].long()]
         good = (info[:, 0] == 1) & (flen == self.frame_len) & (frames == want).all(dim=1)
@@ -537,15 +596,16 @@ class FrameLinkSim:
         counters.index_add_(0, batch["bins"], upd)
         return (rx, llr, frames, flen, info, good) if keep else None
 
-    def sweep(self, snr_points, trials_per_point, rank=0, world=1, batch_frames=1 << 13, base_seed=0xB200):
+    def sweep(self, snr_points, trials_per_point, rank=0, world=1, batch_frames=1 << 13, base_seed=0xB200, raw=False):
         import torch
         counters = torch.zeros((len(snr_points), 6), dtype=torch.int64, device=self.device)
+        table = torch.zeros((len(snr_points), 4), dtype=torch.int64, device=self.device) if raw else None
         mine = np.arange(rank, trials_per_point, world, dtype=np.int64)
         si = np.repeat(np.arange(len(snr_points), dtype=np.int64), len(mine))
         tr = np.tile(mine, len(snr_points))
         for off in range(0, len(si), batch_frames):
-            self.run_batch(self.make_batch(snr_points, si[off:off + batch_frames], tr[off:off + batch_frames], base_seed), counters)
-        return counters
+            self.run_batch(self.make_batch(snr_points, si[off:off + batch_frames], tr[off:off + batch_frames], base_seed), counters, raw=table)
+        return (counters, table) if raw else counters
 
 
 def shard_trials(trials_per_point, rank, world):
@@ -562,13 +622,20 @@ def allreduce_counters(counters):
     return counters
 
 
-def summarize(counters, snr_points):
-    """Rows of {snr_db, frames, fer, ber, fer_ci, avg_iters} from a counter table (host)."""
+def summarize(counters, snr_points, raw=None):
+    """Rows of {snr_db, frames, fer, ber, fer_ci, avg_iters} from a counter table (host).  With a raw table (RAW_COUNTER_NAMES) every row
+    also has raw_ber = bit_errors / (soft_bits - erasures), erasure_rate = erasures / soft_bits and strong_error_share = strong_errors /
+    bit_errors.  The raw BER has no confidence interval: the soft bits of one frame share its noise, fading and timing, so they are not
+    independent trials and a binomial interval over bits would be far too narrow."""
     c = counters.detach().cpu().numpy() if hasattr(counters, "detach") else np.asarray(counters)
+    r4 = None if raw is None else (raw.detach().cpu().numpy() if hasattr(raw, "detach") else np.asarray(raw))
     rows = []
-    for s, r in zip(snr_points, c):
+    for i, (s, r) in enumerate(zip(snr_points, c)):
         frames, ferr, berr, bits, dfail, its = (int(v) for v in r)
         rows.append(dict(snr_db=float(s), frames=frames, fer=ferr / max(frames, 1), ber=berr / max(bits, 1),
                          fer_ci=wilson_interval(ferr, frames), decode_fail=dfail / max(frames, 1),
                          avg_iters=its / max(frames, 1)))
+        if r4 is not None:
+            soft, era, rerr, strong = (int(v) for v in r4[i])
+            rows[-1].update(raw_ber=rerr / max(soft - era, 1), erasure_rate=era / max(soft, 1), strong_error_share=strong / max(rerr, 1))
     return rows

@@ -5,7 +5,7 @@
 //
 //   torchrun-style launch (RANK / WORLD_SIZE / LOCAL_RANK in the environment), or a single process:
 //     projectultra_b200/pu_sweep --table reduced --trials 16384 [--block 2048] [--manifest DIR] [--out rows.jsonl] [--fresh] [--frame-bytes N]
-//                                [--interleave]
+//                                [--interleave] [--raw]
 //   tables: smoke (4 modes, seconds), reduced (one mode per waveform family and channel + the chirp-acquired CFO rows of the regression matrix), config5 (105 modes x 40 SNR points),
 //   frames (whole-frame FER of protocol-v2 DATA frames of 200 and 1000 payload bytes, or N with --frame-bytes, over AWGN / good / poor)
 //   --interleave: every OFDM and MC-DPSK codeword through ChannelInterleaver(bits per symbol, 648) as the reference's IWaveform path
@@ -251,9 +251,12 @@ int main(int argc, char** argv) {
     const uint32_t n_points = pu_sweep_point_count(&d);
     if (n_points == 0) { fprintf(stderr, "pu_sweep: invalid table\n"); return 2; }
 
-    std::vector<uint64_t> counters(static_cast<size_t>(n_points) * 6 + 3 * world, 0);
+    // --raw: pre-decoder counters {soft_bits, erasures, bit_errors, strong_errors} per point (pu_linksim_run_raw), summed with the rest
+    const bool want_raw = flag(argc, argv, "--raw");
+    std::vector<uint64_t> counters(static_cast<size_t>(n_points) * 6 + 3 * world + (want_raw ? static_cast<size_t>(n_points) * 4 : 0), 0);
+    uint64_t* raw = want_raw ? counters.data() + static_cast<size_t>(n_points) * 6 + 3 * world : nullptr;
     pu_sweep_stats st{};
-    const pu_status rs = pu_linksim_run(ctx, &d, counters.data(), &st);
+    const pu_status rs = pu_linksim_run_raw(ctx, &d, counters.data(), raw, &st);
     if (rs != PU_OK) { fprintf(stderr, "pu_sweep[%d]: pu_linksim_run: %s: %s\n", rank, pu_status_string(rs), pu_last_error()); return 3; }
     // per-rank run time / frames / launches ride behind the counters: slot `rank` is this rank's, the sum fills in the others
     uint64_t* tail = counters.data() + static_cast<size_t>(n_points) * 6;
@@ -281,24 +284,31 @@ int main(int argc, char** argv) {
             if (md.interleave_bps) snprintf(il, sizeof il, ", \"interleave_bps\": %u", md.interleave_bps);
             for (uint32_t s = 0; s < md.n_snr; ++s, ++at) {
                 const uint64_t* c = &counters[static_cast<size_t>(at) * 6];
+                char rw[192] = "";
+                if (raw) {      // raw BER over the soft bits that are not erasures; strong errors: |llr| >= 10 (the demappers' clip)
+                    const uint64_t* r = raw + static_cast<size_t>(at) * 4;
+                    snprintf(rw, sizeof rw, ", \"soft_bits\": %llu, \"raw_bit_errors\": %llu, \"raw_ber\": %.6g, \"erasure_rate\": %.6g, \"strong_error_share\": %.6g",
+                             (unsigned long long)r[0], (unsigned long long)r[2], r[0] > r[1] ? double(r[2]) / double(r[0] - r[1]) : 0.0,
+                             r[0] ? double(r[1]) / r[0] : 0.0, r[2] ? double(r[3]) / r[2] : 0.0);
+                }
                 double lo, hi;
                 pu_wilson_interval(c[1], c[0], 1.96, &lo, &hi);
                 frames_all += c[0];
                 if (md.frame_payload_bytes) {     // whole-frame counters {frames, frame_errors, codewords_failed, codewords, header_failures, 0}
                     fprintf(out, "{\"mode\": %u, \"waveform\": \"%s\", \"modem\": \"%s\", \"code_rate\": \"%s\", \"channel\": \"%s\", \"cfo_hz\": %.1f, \"snr_db\": %.2f, "
                                  "\"frame_payload_bytes\": %u, \"codewords\": %llu, \"frames\": %llu, \"frame_errors\": %llu, \"fer\": %.6g, \"fer_ci95\": [%.6g, %.6g], "
-                                 "\"codeword_fail_rate\": %.6g, \"header_fail_rate\": %.6g%s}\n",
+                                 "\"codeword_fail_rate\": %.6g, \"header_fail_rate\": %.6g%s%s}\n",
                             m, kWaveform[md.waveform], desc, kRate[md.code_rate], kChannel[md.channel], md.cfo_hz, md.snr_first_db + s * md.snr_step_db,
                             md.frame_payload_bytes, (unsigned long long)(c[0] ? c[3] / c[0] : 0), (unsigned long long)c[0], (unsigned long long)c[1],
-                            c[0] ? double(c[1]) / c[0] : 0.0, lo, hi, c[3] ? double(c[2]) / c[3] : 0.0, c[0] ? double(c[4]) / c[0] : 0.0, il);
+                            c[0] ? double(c[1]) / c[0] : 0.0, lo, hi, c[3] ? double(c[2]) / c[3] : 0.0, c[0] ? double(c[4]) / c[0] : 0.0, il, rw);
                     continue;
                 }
                 fprintf(out, "{\"mode\": %u, \"waveform\": \"%s\", \"modem\": \"%s\", \"code_rate\": \"%s\", \"channel\": \"%s\", \"cfo_hz\": %.1f, \"snr_db\": %.2f, "
                              "\"frames\": %llu, \"frame_errors\": %llu, \"fer\": %.6g, \"fer_ci95\": [%.6g, %.6g], \"ber\": %.6g, \"decode_fail\": %.6g, "
-                             "\"avg_iters\": %.4g%s}\n",
+                             "\"avg_iters\": %.4g%s%s}\n",
                         m, kWaveform[md.waveform], desc, kRate[md.code_rate], kChannel[md.channel], md.cfo_hz, md.snr_first_db + s * md.snr_step_db,
                         (unsigned long long)c[0], (unsigned long long)c[1], c[0] ? double(c[1]) / c[0] : 0.0, lo, hi, c[3] ? double(c[2]) / c[3] : 0.0,
-                        c[0] ? double(c[4]) / c[0] : 0.0, c[0] ? double(c[5]) / c[0] : 0.0, il);
+                        c[0] ? double(c[4]) / c[0] : 0.0, c[0] ? double(c[5]) / c[0] : 0.0, il, rw);
             }
         }
         double tmax = 0, tsum = 0;
