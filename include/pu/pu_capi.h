@@ -151,8 +151,7 @@ PU_API int pu_ofdm_last_kernel(const pu_ofdm* h);
  *     The 512-FFT differential no-pilot modes at zero CFO take ofdm_fast512.cu; every other whole-frame call (pilots, coherent QAM,
  *     CFO, 1024-FFT pilot modes, acquired frames) takes the general warp kernel with FMA butterflies and MUFU sin/cos in the CFO
  *     rotator (the rotator's phases stay the reference's float recurrence); the remaining kernels (1024-FFT differential
- *     no-pilot, debug dumps) have no fast form and run exact.
- * The environment variable PU_OFDM_PRECISION=exact|fast overrides the handle's setting (A/B runs of unmodified callers). */
+ *     no-pilot, debug dumps) have no fast form and run exact. */
 typedef enum pu_precision { PU_PRECISION_EXACT = 0, PU_PRECISION_FAST = 1 } pu_precision;
 PU_API pu_status pu_ofdm_set_precision(pu_ofdm* h, pu_precision mode);
 PU_API int pu_ofdm_get_precision(const pu_ofdm* h);

@@ -241,11 +241,8 @@ pu_status pu_receive_decode_batch(pu_ofdm* ofdm, pu_ldpc* ldpc, const float* sam
     const bool src_pinned = cudaPointerGetAttributes(&attr, samples) == cudaSuccess && attr.type == cudaMemoryTypeHost;
     (void)cudaGetLastError();
     const size_t slab = std::min<size_t>(B, 4096);
-    static const bool windowed_ok = getenv("PU_E2E_WHOLE_FRAMES") == nullptr;   // A/B switch: copy whole frames
-    const size_t out_row = kb + 1 + sizeof(int32_t);
     const size_t iters_off = ((slab * kb + 15) / 16) * 16;
     const size_t out_bytes = iters_off + slab * sizeof(int32_t) + slab;
-    (void)out_row;
     if (stream) {   // order the lanes after work already queued on the caller's stream
         PU_CUDA_TRY(cudaEventRecord(ctx->pipe_ev, st));
         for (auto& sl : ctx->pipe) PU_CUDA_TRY(cudaStreamWaitEvent(sl.stream, ctx->pipe_ev, 0));
@@ -290,7 +287,7 @@ pu_status pu_receive_decode_batch(pu_ofdm* ofdm, pu_ldpc* ldpc, const float* sam
         // the first training symbol: one strided (3-D) DMA moves exactly those (M1: 12 x 512 of 7 332 samples = 84 % of the frame);
         // the cyclic prefixes, guards and the first LTS symbol never cross PCIe.  Anything else is copied whole.
         int w_first = 0, w_nsym = 0, w_sym = 0, w_cp = 0, w_nfft = 0;
-        const bool windowed = windowed_ok && !cfo_hz && !cfo_phase &&
+        const bool windowed = !cfo_hz && !cfo_phase &&
                               pu_ofdm_diff512_window(ofdm, din, nb, L, training_symbols, &w_first, &w_nsym, &w_sym, &w_cp, &w_nfft);
         if (!src_pinned) {   // pageable source: stage through the lane's pinned buffer (only the windows, when windowed)
             float* stage = static_cast<float*>(sl.h_in.ptr);

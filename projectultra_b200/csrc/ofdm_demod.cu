@@ -169,7 +169,7 @@ __global__ void __launch_bounds__(WARPG ? 512 : NFFT / 8, 1) ofdm_presynced_kern
     const float* __restrict__ cfo_hz, const float* __restrict__ cfo_phase,
     float* __restrict__ llr_out, size_t llr_stride, int llr_limit,
     float* __restrict__ snr_db_out, float* __restrict__ final_cfo_out, float* __restrict__ dbg, unsigned group_bytes,
-    const int* __restrict__ frame_start, const int* __restrict__ frame_nsym, int phase_sync) {
+    const int* __restrict__ frame_start, const int* __restrict__ frame_nsym) {
     constexpr int LOG2N = (NFFT == 512) ? 9 : 10;
     constexpr int T = WARPG ? 32 : NFFT / 8;
     using G = WgGeom<NFFT>;
@@ -177,10 +177,9 @@ __global__ void __launch_bounds__(WARPG ? 512 : NFFT / 8, 1) ofdm_presynced_kern
     const int tid = WARPG ? static_cast<int>(threadIdx.x & 31) : static_cast<int>(threadIdx.x);
     const int wig = WARPG ? static_cast<int>(threadIdx.x >> 5) : 0;
     const size_t frame = WARPG ? static_cast<size_t>(blockIdx.x) * (blockDim.x >> 5) + wig : blockIdx.x;
-    // phase_sync (warp form): all warps of the CTA meet at a barrier at the top of every symbol, so that they walk the same part of
-    // this long kernel at the same time and share its instruction-cache lines; frames past the batch then idle instead of leaving
+    // warp form: all warps of the CTA meet at a barrier at the top of every symbol, so that they walk the same part of this long
+    // kernel at the same time and share its instruction-cache lines; frames past the batch idle instead of leaving
     const bool no_frame = WARPG && frame >= B;
-    if (no_frame && !phase_sync) return;
     const int n_symbols_cta = n_symbols;
     unsigned char* smem_raw = smem_all + static_cast<size_t>(wig) * group_bytes;
     // CTA mode: [NFFT + NFFT/8] FFT buffer, then [sym_len] rotator phases.  Warp mode: [BUF] transpose buffer (its first
@@ -264,8 +263,8 @@ __global__ void __launch_bounds__(WARPG ? 512 : NFFT / 8, 1) ofdm_presynced_kern
     };
     if constexpr (WARPG) stage(next_fft_symbol(-1));
     int llr_pos = 0;   // LLRs emitted so far (same for all threads)
-    for (int s = 0; s < (WARPG && phase_sync ? n_symbols_cta : n_symbols); ++s) {
-        if (WARPG && phase_sync) {
+    for (int s = 0; s < (WARPG ? n_symbols_cta : n_symbols); ++s) {
+        if constexpr (WARPG) {
             __syncthreads();
             if (s >= n_symbols) continue;
         }
@@ -1147,13 +1146,7 @@ struct pu_ofdm {
     int max_symbols = 0;
     int last_kernel = 0;
     int precision = PU_PRECISION_EXACT;
-    bool fast() const {      // PU_OFDM_PRECISION overrides the handle (read once)
-        static const int env = [] {
-            const char* v = getenv("PU_OFDM_PRECISION");
-            return !v ? -1 : (v[0] == 'f' || v[0] == 'F' || v[0] == '1') ? 1 : 0;
-        }();
-        return env >= 0 ? env == 1 : precision == PU_PRECISION_FAST;
-    }
+    bool fast() const { return precision == PU_PRECISION_FAST; }
     size_t smem_bytes = 0;
 
     pu_status ensure_nco(int n_symbols) {
@@ -1282,8 +1275,7 @@ static pu_status launch_ofdm(pu_ofdm* h, const float* d_samples, size_t B, size_
     const int limit = static_cast<int>(std::min<size_t>(llr_stride, static_cast<size_t>(total_llr)));
     const unsigned grid = static_cast<unsigned>(B);
     (void)cudaGetLastError();
-    static const bool no_p512 = getenv("PU_OFDM_NO_PACKED512") != nullptr;   // A/B switch for tests and profiling
-    if (!d_fstart && !d_fnsym && !d_cfo && !d_phase && !d_dbg && !no_p512 && pu::ofdm_diff_supported(h->dev, n_symbols, training) &&
+    if (!d_fstart && !d_fnsym && !d_cfo && !d_phase && !d_dbg && pu::ofdm_diff_supported(h->dev, n_symbols, training) &&
         pu::ofdm_diff512_supported(h->dev, n_symbols, training, d_samples, L, B)) {
         if (h->fast() && pu::ofdm_fast512_supported(h->dev, n_symbols, training, d_samples, L, B, llr_stride)) {
             // PU_PRECISION_FAST: the same pipeline with FMA-contracted butterflies (ofdm_fast512.cu)
@@ -1318,22 +1310,20 @@ static pu_status launch_ofdm(pu_ofdm* h, const float* d_samples, size_t B, size_
         twa.a[m] = make_float2(w.real(), w.imag());
     }
     // Warp-granular variant (one frame per warp): needs every used bin within +-CW of DC (the pruned pass B of the warp FFT)
-    static const bool no_warpg = getenv("PU_OFDM_NO_WARPG") != nullptr;   // A/B switch for tests and profiling
     const int cw = p.nfft == 512 ? 16 : 32;
     bool near_dc = true;
     for (int b : p.data_bin) near_dc = near_dc && ((b >= 1 && b < cw) || b > p.nfft - cw);
     for (int b : p.pilot_bin) near_dc = near_dc && ((b >= 1 && b < cw) || b > p.nfft - cw);
-    if (!d_dbg && !no_warpg && near_dc) {
-        // one CTA per SM with as many frames as shared memory holds, warps re-aligned at every symbol (default; r29: M3 32QAM 3.16 ->
-        // 2.49 ms, M1 16QAM 7.19 -> 6.08 ms per 53k frames); PU_OFDM_WARPG_SYNC=0 selects small CTAs without the barrier
-        static const bool wsync = !(getenv("PU_OFDM_WARPG_SYNC") != nullptr && atoi(getenv("PU_OFDM_WARPG_SYNC")) == 0);
-        const int warps = wsync ? (p.nfft == 512 ? 16 : 14) : (p.nfft == 512 ? 4 : 3);
+    if (!d_dbg && near_dc) {
+        // one CTA per SM with as many frames as shared memory holds, warps re-aligned at every symbol (r29: M3 32QAM 3.16 -> 2.49 ms,
+        // M1 16QAM 7.19 -> 6.08 ms per 53k frames against small CTAs of 3-4 warps without the barrier)
+        const int warps = p.nfft == 512 ? 16 : 14;
         const size_t buf_f2 = static_cast<size_t>(p.nfft + (p.nfft >> (p.nfft == 512 ? 4 : 5)) + 2 * cw);
         const unsigned group = static_cast<unsigned>((buf_f2 * sizeof(float2) + sizeof(pu::RxShared) + 15) & ~size_t(15));
         const unsigned wgrid = static_cast<unsigned>((B + warps - 1) / warps);
         const bool diff = pu::is_differential(p.cfg.modulation);
         using WK = void (*)(pu::OfdmDev, pu::WgTw, const float*, size_t, size_t, int, int, const float*, const float*, float*, size_t, int,
-                            float*, float*, float*, unsigned, const int*, const int*, int);
+                            float*, float*, float*, unsigned, const int*, const int*);
         const bool fastk = h->fast();     // PU_PRECISION_FAST: FMA butterflies + MUFU rotator sin/cos (see the kernel's FAST parameter)
         const WK wk = fastk ? (p.nfft == 512 ? (diff ? pu::ofdm_presynced_kernel<512, true, 1, true> : pu::ofdm_presynced_kernel<512, true, 2, true>)
                                              : (diff ? pu::ofdm_presynced_kernel<1024, true, 1, true> : pu::ofdm_presynced_kernel<1024, true, 2, true>))
@@ -1342,7 +1332,7 @@ static pu_status launch_ofdm(pu_ofdm* h, const float* d_samples, size_t B, size_
         static std::atomic<uint64_t> attrw[8];      // per kernel instance, one bit per device (pu_async.cuh: smem_optin)
         PU_CUDA_TRY(pu::smem_optin(attrw[(fastk ? 4 : 0) + (p.nfft == 512 ? 0 : 2) + (diff ? 0 : 1)], wk, 232448));
         wk<<<wgrid, warps * 32, static_cast<size_t>(warps) * group, st>>>(h->dev, twa, d_samples, L, B, n_symbols, training, d_cfo, d_phase, d_llr,
-                                                                           llr_stride, limit, d_snr, d_fcfo, nullptr, group, d_fstart, d_fnsym, wsync ? 1 : 0);
+                                                                           llr_stride, limit, d_snr, d_fcfo, nullptr, group, d_fstart, d_fnsym);
         h->last_kernel = fastk ? 6 : 4;
         h->ctx->launches.fetch_add(1);
         PU_CUDA_TRY(cudaGetLastError());
@@ -1352,12 +1342,12 @@ static pu_status launch_ofdm(pu_ofdm* h, const float* d_samples, size_t B, size_
         static std::atomic<uint64_t> attr512{0};
         PU_CUDA_TRY(pu::smem_optin(attr512, pu::ofdm_presynced_kernel<512, false, 0>, 65536));
         pu::ofdm_presynced_kernel<512, false, 0><<<grid, 64, h->smem_bytes, st>>>(h->dev, twa, d_samples, L, B, n_symbols, training, d_cfo, d_phase,
-                                                                            d_llr, llr_stride, limit, d_snr, d_fcfo, d_dbg, 0u, d_fstart, d_fnsym, 0);
+                                                                            d_llr, llr_stride, limit, d_snr, d_fcfo, d_dbg, 0u, d_fstart, d_fnsym);
     } else {
         static std::atomic<uint64_t> attr1024{0};
         PU_CUDA_TRY(pu::smem_optin(attr1024, pu::ofdm_presynced_kernel<1024, false, 0>, 65536));
         pu::ofdm_presynced_kernel<1024, false, 0><<<grid, 128, h->smem_bytes, st>>>(h->dev, twa, d_samples, L, B, n_symbols, training, d_cfo, d_phase,
-                                                                              d_llr, llr_stride, limit, d_snr, d_fcfo, d_dbg, 0u, d_fstart, d_fnsym, 0);
+                                                                              d_llr, llr_stride, limit, d_snr, d_fcfo, d_dbg, 0u, d_fstart, d_fnsym);
     }
     h->last_kernel = 1;
     h->ctx->launches.fetch_add(1);
@@ -1753,7 +1743,7 @@ pu_ctx* pu_ofdm_context(pu_ofdm* h) { return h ? h->ctx : nullptr; }
 // false when the call would take another kernel (which may read anything).
 bool pu_ofdm_diff512_window(pu_ofdm* h, const float* d_samples, size_t B, size_t L, int training, int* first, int* n_symbols, int* sym_len,
                             int* cp, int* nfft) {
-    if (!h || getenv("PU_OFDM_NO_PACKED512")) return false;
+    if (!h) return false;
     const pu::OfdmPlan& p = h->plan;
     const int ns = static_cast<int>(L / p.sym_len);
     if (ns < 1 || static_cast<size_t>(ns) * p.sym_len != L) return false;

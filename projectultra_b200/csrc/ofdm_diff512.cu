@@ -29,8 +29,12 @@
 //   * the <= 2 % of carriers that fail the saturation filter are queued per warp (equalised symbol, predecessor,
 //     nv, destination) and the exact libm-restatement demapper runs on 32 queued carriers at a time with all lanes
 //     busy, instead of on one or two lanes per symbol.
-//   * one 128-bit shared-memory transpose per element (re_f, re_f1, im_f, im_f1) between the two FFT passes.
+//   * one shared-memory transpose between the two FFT passes, the real and the imaginary halves one after the other
+//     through a buffer of half the size (two more __syncwarp, twice the LDS/STS instructions, room for more warps).
 // HBM traffic: every sample of the symbols that are used is read exactly once, LLRs are written once.
+// Measured and not kept (profiles/r04_ofdm512_variants.txt, r05): a 3-stage ring (0.70 ms per 53 248 frames against 0.54 ms),
+// a 128-bit transpose buffer of full size (0.69 ms), and 16 warps with the transpose done in place in the ring stage and the
+// pass-B twiddles in shared memory to stay under 128 registers (0.56 ms: the kernel is not occupancy-bound).
 #include <cfloat>
 
 #include "ofdm_dev.cuh"
@@ -42,9 +46,9 @@ namespace pu {
 
 
 constexpr int kP512MaxWarps = 12;       // frame pairs in flight per CTA (one warp each)
-constexpr int kP512MaxWarpsInplace = 16; // ... of the in-place-transpose variant
+constexpr int kP512Stages = 2;          // ring depth of the per-warp sample staging
 constexpr int kP512MaxSym = 40;
-constexpr int kP512Buf = 512 + 32;      // float4 per warp: element p lives at p + (p >> 4)
+constexpr int kP512Buf = 512 + 32;      // transpose slots (u64) per warp: element p lives at p + (p >> 4)
 constexpr size_t kP512SmemMax = 227 * 1024;
 
 struct P512Tw { u64 re[8], im[8]; };    // pass-A twiddles tw[32 m] as broadcast pairs (w.x, w.x), (w.y, w.y)
@@ -82,42 +86,31 @@ constexpr int kP512StageFloats = 1024;  // one ring stage: 512 samples (after th
 
 struct P512Smem {     // offsets (bytes) into dynamic shared memory, computed identically on host and device
     size_t nco;                                              // CTA-wide: NCO slices of the processed symbols
-    size_t tws;                                              // CTA-wide: pass-B twiddles per lane as (re, re, im, im) (TWS variants)
     size_t warp0, warp_stride;                               // then one block per warp:
     size_t S, T, q_rx, q_rxp, q_h, q_frame, q_item, bars; //   offsets inside a warp block
-    size_t stage_floats;                                     // distance between ring stages
     size_t total;
 };
-// inplace: the transpose between the FFT passes reuses the ring stage whose samples were just taken (plus 256 bytes of
-// padding behind it) instead of a buffer of its own, so a warp needs 10.5 KB and sixteen warps fit next to the NCO table.
-__host__ __device__ inline P512Smem p512_layout(int n_proc, int warps, int stages, bool half, bool inplace) {
+__host__ __device__ inline P512Smem p512_layout(int n_proc, int warps) {
     P512Smem L;
     size_t o = 0;
     auto take = [&o](size_t bytes) { const size_t at = o; o += (bytes + 15) & ~size_t(15); return at; };
     L.nco = take(static_cast<size_t>(n_proc) * 512 * sizeof(float2));
-    L.tws = take(inplace ? 9 * 32 * sizeof(float4) : 0);
     L.warp0 = (o + 127) & ~size_t(127);
     o = 0;
-    L.stage_floats = inplace ? (kP512Buf * sizeof(float2)) / sizeof(float) : kP512StageFloats;
-    L.S = take(static_cast<size_t>(stages) * L.stage_floats * sizeof(float));
-    L.T = inplace ? L.S : take(kP512Buf * (half ? sizeof(float2) : sizeof(float4)));
+    L.S = take(static_cast<size_t>(kP512Stages) * kP512StageFloats * sizeof(float));
+    L.T = take(kP512Buf * sizeof(float2));
     L.q_rx = take(kP512Queue * sizeof(float2));
     L.q_rxp = take(kP512Queue * sizeof(float2));
     L.q_h = take(kP512Queue * sizeof(float2));
     L.q_frame = take(kP512Queue * sizeof(unsigned));
     L.q_item = take(kP512Queue * sizeof(int));
-    L.bars = take(static_cast<size_t>(stages) * sizeof(u64));
+    L.bars = take(static_cast<size_t>(kP512Stages) * sizeof(u64));
     L.warp_stride = (o + 127) & ~size_t(127);
     L.total = L.warp0 + static_cast<size_t>(warps) * L.warp_stride;
     return L;
 }
 
-// D: ring depth of the per-warp sample staging.  HALF: transpose the real and imaginary halves one after the other through a
-// buffer of half the size (two more __syncwarp, twice the LDS/STS instructions, room for more warps per SM).
-// INPLACE (needs HALF): see p512_layout; the pass-B twiddles then come from shared memory instead of 36 registers, which
-// brings the kernel under the 128 registers that 16 resident warps leave per thread.
-template <int D, bool HALF, bool INPLACE, int MAXW>
-__global__ void __launch_bounds__(MAXW * 32, 1) ofdm_diff512_kernel(
+__global__ void __launch_bounds__(kP512MaxWarps * 32, 1) ofdm_diff512_kernel(
     OfdmDev d, P512Tw twa, u64 Z, const float* __restrict__ samples, size_t frame_stride, size_t B, int n_symbols, int training,
     float* __restrict__ llr_out, size_t llr_stride, int llr_limit, float* __restrict__ snr_db_out, float* __restrict__ final_cfo_out) {
     constexpr int EPL = 16;
@@ -126,14 +119,12 @@ __global__ void __launch_bounds__(MAXW * 32, 1) ofdm_diff512_kernel(
     const int nd = d.n_data;
     const int first = training > 0 ? training - 1 : 0;   // data H uses the LAST training symbol only (:179-185)
     const int n_proc = n_symbols - first;
-    static_assert(!INPLACE || HALF, "the in-place transpose moves one 8-byte half at a time");
-    const P512Smem L = p512_layout(n_proc, W, D, HALF, INPLACE);
-    const int SS = static_cast<int>(L.stage_floats);
+    const P512Smem L = p512_layout(n_proc, W);
+    constexpr int SS = kP512StageFloats;
     float2* nco_s = reinterpret_cast<float2*>(smem_raw + L.nco);                       // [n_proc][16][32] (cos, -sin)
     unsigned char* wb = smem_raw + L.warp0 + warp * L.warp_stride;
     float* S = reinterpret_cast<float*>(wb + L.S);
-    float4* tb = reinterpret_cast<float4*>(wb + L.T);                                   // INPLACE: re-pointed at the current stage every step
-    float4* tws = reinterpret_cast<float4*>(smem_raw + L.tws);
+    u64* tb = reinterpret_cast<u64*>(wb + L.T);
     float2* q_rx = reinterpret_cast<float2*>(wb + L.q_rx);       // queued carriers: FFT bin of the symbol,
     float2* q_rxp = reinterpret_cast<float2*>(wb + L.q_rxp);     //   bin of the preceding symbol,
     float2* q_h = reinterpret_cast<float2*>(wb + L.q_h);         //   channel estimate of the carrier
@@ -148,7 +139,7 @@ __global__ void __launch_bounds__(MAXW * 32, 1) ofdm_diff512_kernel(
 
     if (lane == 0) {
 #pragma unroll
-        for (int i = 0; i < D; ++i) mbar_init(&bars[i], 1);
+        for (int i = 0; i < kP512Stages; ++i) mbar_init(&bars[i], 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     // NCO slices of the processed symbols (loop invariant: resident in shared memory for the life of the CTA); entry
@@ -172,8 +163,6 @@ __global__ void __launch_bounds__(MAXW * 32, 1) ofdm_diff512_kernel(
     size_t ip_pair = gw;
     int ip_sym = 0;
     auto issue = [&](int stage) {
-        // INPLACE: the stage was last written through the generic proxy (transpose); order that before the bulk copy's writes
-        if constexpr (INPLACE) asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
         const size_t f0 = 2 * ip_pair, f1 = (f0 + 1 < B) ? f0 + 1 : f0;     // odd tail: the upper half recomputes frame f (never stored)
         const size_t so = static_cast<size_t>(first + ip_sym) * d.sym_len + d.cp;
         mbar_expect_tx(&bars[stage], 2 * sym_bytes);
@@ -183,7 +172,7 @@ __global__ void __launch_bounds__(MAXW * 32, 1) ofdm_diff512_kernel(
     };
     if (lane == 0) {
 #pragma unroll
-        for (int i = 0; i < D; ++i)
+        for (int i = 0; i < kP512Stages; ++i)
             if (static_cast<size_t>(i) < total_steps) issue(i);
     }
 
@@ -202,32 +191,6 @@ __global__ void __launch_bounds__(MAXW * 32, 1) ofdm_diff512_kernel(
         const float2 a = __ldg(&d.twiddle[b8 ? (c + 240) : c]);
         wlast_re = pk(a.x, a.x); wlast_im = pk(a.y, a.y);
     }
-    if constexpr (INPLACE) {      // the same pairs, parked in shared memory by warp 0: [0..3] low, [4..7] high, [8] last stage
-        if (warp == 0) {
-#pragma unroll
-            for (int q = 0; q < 4; ++q) {
-                float x0, x1, y0, y1;
-                upk(wl_re[q], x0, x1); upk(wl_im[q], y0, y1);
-                tws[q * 32 + lane] = make_float4(x0, x1, y0, y1);
-                upk(wh_re[q], x0, x1); upk(wh_im[q], y0, y1);
-                tws[(4 + q) * 32 + lane] = make_float4(x0, x1, y0, y1);
-            }
-            float x0, x1, y0, y1;
-            upk(wlast_re, x0, x1); upk(wlast_im, y0, y1);
-            tws[8 * 32 + lane] = make_float4(x0, x1, y0, y1);
-        }
-    }
-    if constexpr (INPLACE) __syncthreads();   // (prologue) the twiddle table is visible to every warp
-    auto tw_get = [&](int i, u64& re, u64& im) {     // i as in the shared table; the register copy is dead code under INPLACE
-        if constexpr (INPLACE) {
-            const float4 e = tws[i * 32 + lane];
-            re = pk(e.x, e.y); im = pk(e.z, e.w);
-        } else {
-            if (i < 4) { re = wl_re[i]; im = wl_im[i]; }
-            else if (i < 8) { re = wh_re[i - 4]; im = wh_im[i - 4]; }
-            else { re = wlast_re; im = wlast_im; }
-        }
-    };
     // the carrier this lane ends the FFT with: bins 1..nhi on lanes (0, c), bins 512-nlo..511 on lanes (1, c)
     int idx = -1;
     if (b8 == 0) { if (c >= 1 && c <= nhi) idx = nlo + c - 1; }
@@ -287,7 +250,6 @@ __global__ void __launch_bounds__(MAXW * 32, 1) ofdm_diff512_kernel(
         const int s = first + sidx;
         mbar_wait(&bars[stage], parity);
         const float* x0 = S + stage * SS;
-        if constexpr (INPLACE) tb = reinterpret_cast<float4*>(S + stage * SS);
         const float* x1 = x0 + 512;
         const float2* nc = nco_s + sidx * 512 + lane;                 // [q][lane]: entry of sample brev5(lane) + 32 brev4(q)
         // ---- pass A: lane g owns bit-reversed positions 16 g .. 16 g + 15 = samples brev5(g) + 32 brev4(q)
@@ -302,10 +264,7 @@ __global__ void __launch_bounds__(MAXW * 32, 1) ofdm_diff512_kernel(
             v[q].im = pk(__fmaf_rn(o.y, xa, zf), __fmaf_rn(o.y, xb, zf));
         }
         __syncwarp();                                                  // every lane has taken its samples out of the stage
-        // refill it with the step D ahead -- at once when the stage is only a staging buffer; INPLACE: after the transposes
-        // (and after the SNR scratch of a training step) have finished with it
-        const bool snr_step = snr_db_out && (s < training || (sidx == 0 && training == 0));
-        if (!INPLACE && lane == 0 && t + D < total_steps) issue(stage);
+        if (lane == 0 && t + kP512Stages < total_steps) issue(stage);     // refill it with the step a full ring ahead
 #pragma unroll
         for (int tt = 1; tt <= 4; ++tt) {
             const int half = 1 << (tt - 1);
@@ -318,52 +277,28 @@ __global__ void __launch_bounds__(MAXW * 32, 1) ofdm_diff512_kernel(
                 else bfly2(v[a], v[a + half], twa.re[m], twa.im[m], Z);
             }
         }
-        if constexpr (HALF) {
-            u64* tb2 = reinterpret_cast<u64*>(tb);
+        // ---- transpose: p = 16 lane + q at slot p + (p >> 4); pass B: lane (b8, c) owns p = c + 16 j + 256 b8
 #pragma unroll
-            for (int q = 0; q < EPL; ++q) tb2[17 * lane + q] = v[q].re;       // p = 16 lane + q at p + (p >> 4)
-            __syncwarp();
+        for (int q = 0; q < EPL; ++q) tb[17 * lane + q] = v[q].re;
+        __syncwarp();
 #pragma unroll
-            for (int j = 0; j < EPL; ++j) v[j].re = tb2[c + 17 * j + 272 * b8];
-            __syncwarp();
+        for (int j = 0; j < EPL; ++j) v[j].re = tb[c + 17 * j + 272 * b8];
+        __syncwarp();
 #pragma unroll
-            for (int q = 0; q < EPL; ++q) tb2[17 * lane + q] = v[q].im;
-            __syncwarp();
+        for (int q = 0; q < EPL; ++q) tb[17 * lane + q] = v[q].im;
+        __syncwarp();
 #pragma unroll
-            for (int j = 0; j < EPL; ++j) v[j].im = tb2[c + 17 * j + 272 * b8];
-        } else {
-#pragma unroll
-            for (int q = 0; q < EPL; ++q) {
-                float a0, a1, b0, b1;
-                upk(v[q].re, a0, a1); upk(v[q].im, b0, b1);
-                tb[17 * lane + q] = make_float4(a0, a1, b0, b1);       // p = 16 lane + q at p + (p >> 4)
-            }
-            __syncwarp();
-            // ---- pass B: lane (b8, c) owns p = c + 16 j + 256 b8
-#pragma unroll
-            for (int j = 0; j < EPL; ++j) {
-                const float4 e = tb[c + 17 * j + 272 * b8];
-                v[j].re = pk(e.x, e.y); v[j].im = pk(e.z, e.w);
-            }
-        }
+        for (int j = 0; j < EPL; ++j) v[j].im = tb[c + 17 * j + 272 * b8];
         __syncwarp();                                                  // the transpose buffer may be rewritten (next step / SNR scratch)
-        if (INPLACE && !snr_step && lane == 0 && t + D < total_steps) issue(stage);
-        {
-            u64 wr, wi;
-            tw_get(0, wr, wi);
 #pragma unroll
-            for (int j = 0; j < EPL; j += 2) bfly2(v[j], v[j + 1], wr, wi, Z);
-        }
+        for (int j = 0; j < EPL; j += 2) bfly2(v[j], v[j + 1], wl_re[0], wl_im[0], Z);
 #pragma unroll
         for (int q = 1; q < 4; ++q) {
             const int step = 1 << (q + 1), hh = 1 << q;
-            u64 lr, li, hr, hi;
-            tw_get(q, lr, li);
-            tw_get(4 + q, hr, hi);
 #pragma unroll
             for (int j = 0; j < EPL; j += step) {
-                v[j] = bfly2_lo(v[j], v[j + hh], lr, li, Z);
-                v[j + step - 1] = bfly2_hi(v[j + step - 1 - hh], v[j + step - 1], hr, hi, Z);
+                v[j] = bfly2_lo(v[j], v[j + hh], wl_re[q], wl_im[q], Z);
+                v[j + step - 1] = bfly2_hi(v[j + step - 1 - hh], v[j + step - 1], wh_re[q], wh_im[q], Z);
             }
         }
         // stage 9 pairs lane (0,c) [A] with lane (1,c) [B]: bin c = A0 + w B0 on lane (0,c); bin 496+c = A15 - w B15 on lane (1,c)
@@ -371,9 +306,7 @@ __global__ void __launch_bounds__(MAXW * 32, 1) ofdm_diff512_kernel(
         C2 recv;
         recv.re = __shfl_xor_sync(0xffffffffu, send.re, 16);
         recv.im = __shfl_xor_sync(0xffffffffu, send.im, 16);
-        u64 wlr, wli;
-        tw_get(8, wlr, wli);
-        const C2 bin = b8 ? bfly2_hi(recv, v[EPL - 1], wlr, wli, Z) : bfly2_lo(v[0], recv, wlr, wli, Z);
+        const C2 bin = b8 ? bfly2_hi(recv, v[EPL - 1], wlast_re, wlast_im, Z) : bfly2_lo(v[0], recv, wlast_re, wlast_im, Z);
         float2 rx[2];
         upk(bin.re, rx[0].x, rx[1].x); upk(bin.im, rx[0].y, rx[1].y);
 
@@ -412,7 +345,6 @@ __global__ void __launch_bounds__(MAXW * 32, 1) ofdm_diff512_kernel(
             }
             if (final_cfo_out && lane < 2 && (lane == 0 || have1)) final_cfo_out[f0 + lane] = 0.0f;
         }
-        if (INPLACE && snr_step && lane == 0 && t + D < total_steps) issue(stage);
         if (s >= training) {
             // ---- equalize (:747-770) + demodulateSymbol (demodulator.cpp:279-316) + soft_demap.hpp on the lane that owns the
             //      carrier, for both frames.  The equalised symbols themselves are only formed on the exact path (flush):
@@ -453,29 +385,15 @@ __global__ void __launch_bounds__(MAXW * 32, 1) ofdm_diff512_kernel(
             rxp = bin;
         }
         if (++sidx == n_proc) { sidx = 0; pair += GW; }
-        if (++stage == D) { stage = 0; parity ^= 1u; }
+        if (++stage == kP512Stages) { stage = 0; parity ^= 1u; }
     }
     while (qcount > 0) flush();
 }
 
-// Variant switches (read once; defaults = the fastest measured, profiles/r04_ofdm512_variants.txt and later):
-//   PU_P512_INPLACE (default 0)  in-place transpose + shared-memory twiddles, up to 16 warps (<= 128 registers); measured
-//                                0.56 ms against 0.54 ms for 12 warps with a transpose buffer of their own (r05): not occupancy-bound
-//   PU_P512_THALF   (default 1)  half-size transpose buffer            PU_P512_STAGES (2|3)  ring depth
-//   PU_P512_WARPS                upper bound on warps per CTA
-static int p512_env(const char* name, int dflt) {
-    const char* v = getenv(name);
-    return v ? atoi(v) : dflt;
-}
-static bool p512_inplace() { static const int env = p512_env("PU_P512_INPLACE", 0); return env != 0; }
-static bool p512_half() { static const int env = p512_env("PU_P512_THALF", 1); return env != 0 || p512_inplace(); }
-static int p512_stages() { static const int env = p512_env("PU_P512_STAGES", 0); return (env == 3 && !p512_inplace()) ? 3 : 2; }
 // Warps per CTA: as many independent frame-pair pipelines as shared memory holds (NCO slices + one block per warp).
-static int p512_warps(int n_proc, int stages, bool half, bool inplace) {
-    static const int env = p512_env("PU_P512_WARPS", 0);
-    int w = inplace ? kP512MaxWarpsInplace : kP512MaxWarps;
-    if (env > 0 && env < w) w = env;
-    while (w > 1 && p512_layout(n_proc, w, stages, half, inplace).total > kP512SmemMax) --w;
+static int p512_warps(int n_proc) {
+    int w = kP512MaxWarps;
+    while (w > 1 && p512_layout(n_proc, w).total > kP512SmemMax) --w;
     return w;
 }
 
@@ -491,7 +409,7 @@ bool ofdm_diff512_supported(const OfdmDev& d, int n_symbols, int training, const
     if (n_symbols - first < 1) return false;
     const int nlo = d.n_data / 2, nhi = d.n_data - nlo;
     if (!(nlo < 16 && nhi < 16)) return false;
-    return p512_layout(n_symbols - first, 1, p512_stages(), p512_half(), p512_inplace()).total <= kP512SmemMax;
+    return p512_layout(n_symbols - first, 1).total <= kP512SmemMax;
 }
 
 cudaError_t ofdm_diff512_launch(const OfdmDev& d, const float2* host_twiddle, const float* samples, size_t B, size_t frame_stride,
@@ -506,26 +424,19 @@ cudaError_t ofdm_diff512_launch(const OfdmDev& d, const float2* host_twiddle, co
         twa.im[m] = (static_cast<u64>(xi) << 32) | xi;
     }
     const int first = training > 0 ? training - 1 : 0;
-    const int stages = p512_stages();
-    const bool half = p512_half(), inplace = p512_inplace();
-    const int warps = p512_warps(n_symbols - first, stages, half, inplace);
-    const P512Smem L = p512_layout(n_symbols - first, warps, stages, half, inplace);
-    using Kernel = void (*)(OfdmDev, P512Tw, u64, const float*, size_t, size_t, int, int, float*, size_t, int, float*, float*);
-    const Kernel kernels[5] = {ofdm_diff512_kernel<2, false, false, kP512MaxWarps>, ofdm_diff512_kernel<2, true, false, kP512MaxWarps>,
-                               ofdm_diff512_kernel<3, false, false, kP512MaxWarps>, ofdm_diff512_kernel<3, true, false, kP512MaxWarps>,
-                               ofdm_diff512_kernel<2, true, true, kP512MaxWarpsInplace>};
-    static std::atomic<uint64_t> attr_done[5];
-    const int which = inplace ? 4 : (stages == 3 ? 2 : 0) + (half ? 1 : 0);
+    const int warps = p512_warps(n_symbols - first);
+    const P512Smem L = p512_layout(n_symbols - first, warps);
+    static std::atomic<uint64_t> attr_done{0};
     {
-        const cudaError_t e = smem_optin(attr_done[which], kernels[which], static_cast<int>(kP512SmemMax));
+        const cudaError_t e = smem_optin(attr_done, ofdm_diff512_kernel, static_cast<int>(kP512SmemMax));
         if (e != cudaSuccess) return e;
     }
     const size_t max_ctas = static_cast<size_t>(sm_count > 0 ? sm_count : 148);      // persistent: one CTA per SM
     const size_t want_ctas = ((B + 1) / 2 + warps - 1) / warps;
     const unsigned grid = static_cast<unsigned>(want_ctas < max_ctas ? want_ctas : max_ctas);
     const u64 Z = 0x8000000080000000ull;    // (-0.0f, -0.0f): see the header comment
-    kernels[which]<<<grid, warps * 32, L.total, st>>>(d, twa, Z, samples, frame_stride, B, n_symbols, training, llr,
-                                                                                     llr_stride, llr_limit, snr_db, final_cfo);
+    ofdm_diff512_kernel<<<grid, warps * 32, L.total, st>>>(d, twa, Z, samples, frame_stride, B, n_symbols, training, llr,
+                                                                                         llr_stride, llr_limit, snr_db, final_cfo);
     return cudaGetLastError();
 }
 

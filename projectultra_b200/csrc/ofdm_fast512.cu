@@ -29,6 +29,10 @@
 // go through the same libm-restatement demapper as the bit-exact kernel on bins that differ from the reference's by
 // less than the reference's own bins differ from a float64 DFT; LLRs within 1e-4 * max(|ref|, 0.5); decoded bytes
 // identical on every frame the reference decodes with margin.
+// Like ofdm_diff512.cu, the transpose moves the real and the imaginary halves one after the other through a buffer of half the
+// size.  Measured and not kept: 16 warps with the transpose done in place in the ring stage (128 registers) ran at 0.3645 ms
+// against 0.3618 ms per 53 248 frames for 12 warps with their own buffer (v02: with four warps per scheduler the FMA pipe
+// (math-pipe throttle 0.94 per issue) and the shared-memory pipe (68 %) are the limits, not latency).
 #include <cfloat>
 
 #include "ofdm_dev.cuh"
@@ -39,7 +43,7 @@
 namespace pu {
 
 constexpr int kF512MaxWarps = 12;
-constexpr int kF512MaxWarpsInplace = 16;
+constexpr int kF512Stages = 2;              // ring depth of the per-warp sample staging
 constexpr int kF512MaxSym = 40;
 constexpr int kF512Buf = 512 + 32;          // transpose slots per warp: element p lives at p + (p >> 4)
 constexpr int kF512Queue = 64;              // per-warp queue of carriers waiting for the exact demapper (flushed 32 at a time)
@@ -55,12 +59,9 @@ struct F512Smem {      // byte offsets into dynamic shared memory, identical on 
     size_t dst;        // CTA-wide [n_proc][32] 4 x u16: LLR destinations of the lane's carrier in that symbol (0xffff = none)
     size_t warp0, warp_stride;
     size_t S, T, q_rx, q_rxp, q_h, q_frame, q_item, bars;
-    size_t stage_floats;   // distance between ring stages
     size_t total;
 };
-// inplace (needs half): the transpose reuses the ring stage whose samples were just taken (plus 256 bytes of padding behind it)
-// instead of a buffer of its own, so a warp needs 10.6 KB and sixteen warps fit next to the CTA-wide tables.
-__host__ __device__ inline F512Smem f512_layout(int n_proc, int warps, int stages, bool half, bool inplace) {
+__host__ __device__ inline F512Smem f512_layout(int n_proc, int warps) {
     F512Smem L;
     size_t o = 0;
     auto take = [&o](size_t bytes) { const size_t at = o; o += (bytes + 15) & ~size_t(15); return at; };
@@ -68,15 +69,14 @@ __host__ __device__ inline F512Smem f512_layout(int n_proc, int warps, int stage
     L.dst = take(static_cast<size_t>(n_proc) * 32 * 4 * sizeof(unsigned short));
     L.warp0 = (o + 127) & ~size_t(127);
     o = 0;
-    L.stage_floats = inplace ? (kF512Buf * sizeof(float2)) / sizeof(float) : kF512StageFloats;
-    L.S = take(static_cast<size_t>(stages) * L.stage_floats * sizeof(float));
-    L.T = inplace ? L.S : take(kF512Buf * (half ? sizeof(float2) : sizeof(float4)));
+    L.S = take(static_cast<size_t>(kF512Stages) * kF512StageFloats * sizeof(float));
+    L.T = take(kF512Buf * sizeof(float2));
     L.q_rx = take(kF512Queue * sizeof(float2));
     L.q_rxp = take(kF512Queue * sizeof(float2));
     L.q_h = take(kF512Queue * sizeof(float2));
     L.q_frame = take(kF512Queue * sizeof(unsigned));
     L.q_item = take(kF512Queue * sizeof(int));
-    L.bars = take(static_cast<size_t>(stages) * sizeof(u64));
+    L.bars = take(static_cast<size_t>(kF512Stages) * sizeof(u64));
     L.warp_stride = (o + 127) & ~size_t(127);
     L.total = L.warp0 + static_cast<size_t>(warps) * L.warp_stride;
     return L;
@@ -135,10 +135,7 @@ __device__ __forceinline__ FC2 f_hi(FC2 a, FC2 b, float wr, float wi) {      // 
     return r;
 }
 
-// D: ring depth of the per-warp sample staging.  HALF: the transpose moves the real and the imaginary halves one after the
-// other through a buffer of half the size (twice the LDS/STS instructions, room for more warps per SM).
-template <int D, bool HALF, bool INPLACE, int MAXW>
-__global__ void __launch_bounds__(MAXW * 32, 1) ofdm_fast512_kernel(
+__global__ void __launch_bounds__(kF512MaxWarps * 32, 1) ofdm_fast512_kernel(
     OfdmDev d, const float* __restrict__ samples, size_t frame_stride, size_t B, int n_symbols, int training,
     float* __restrict__ llr_out, size_t llr_stride, int llr_limit, float* __restrict__ snr_db_out, float* __restrict__ final_cfo_out) {
     constexpr int EPL = 16;
@@ -147,14 +144,13 @@ __global__ void __launch_bounds__(MAXW * 32, 1) ofdm_fast512_kernel(
     const int nd = d.n_data;
     const int first = training > 0 ? training - 1 : 0;   // data H uses the LAST training symbol only (:179-185)
     const int n_proc = n_symbols - first;
-    static_assert(!INPLACE || HALF, "the in-place transpose moves one 8-byte half at a time");
-    const F512Smem L = f512_layout(n_proc, W, D, HALF, INPLACE);
-    const int SS = static_cast<int>(L.stage_floats);
+    const F512Smem L = f512_layout(n_proc, W);
+    constexpr int SS = kF512StageFloats;
     float2* nco_s = reinterpret_cast<float2*>(smem_raw + L.nco);
     uint2* dst_s = reinterpret_cast<uint2*>(smem_raw + L.dst);                        // [n_proc][32]
     unsigned char* wb = smem_raw + L.warp0 + warp * L.warp_stride;
     float* S = reinterpret_cast<float*>(wb + L.S);
-    float4* tb = reinterpret_cast<float4*>(wb + L.T);
+    u64* tb = reinterpret_cast<u64*>(wb + L.T);
     float2* q_rx = reinterpret_cast<float2*>(wb + L.q_rx);       // queued carriers: FFT bin of the symbol,
     float2* q_rxp = reinterpret_cast<float2*>(wb + L.q_rxp);     //   bin of the preceding symbol (or h),
     float2* q_h = reinterpret_cast<float2*>(wb + L.q_h);         //   channel estimate of the carrier
@@ -173,7 +169,7 @@ __global__ void __launch_bounds__(MAXW * 32, 1) ofdm_fast512_kernel(
 
     if (lane == 0) {
 #pragma unroll
-        for (int i = 0; i < D; ++i) mbar_init(&bars[i], 1);
+        for (int i = 0; i < kF512Stages; ++i) mbar_init(&bars[i], 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     // NCO slices of the processed symbols, resident for the life of the CTA; entry [sy][q][lane] belongs to sample
@@ -214,8 +210,6 @@ __global__ void __launch_bounds__(MAXW * 32, 1) ofdm_fast512_kernel(
     size_t ip_pair = gw;      // producer cursor (lane 0 only): step -> (pair, symbol)
     int ip_sym = 0;
     auto issue = [&](int stage) {
-        // INPLACE: the stage was last written through the generic proxy (transpose); order that before the bulk copy's writes
-        if constexpr (INPLACE) asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
         const size_t f0 = 2 * ip_pair, f1 = (f0 + 1 < B) ? f0 + 1 : f0;     // odd tail: the upper half recomputes frame f (never stored)
         const size_t so = static_cast<size_t>(first + ip_sym) * d.sym_len + d.cp;
         mbar_expect_tx(&bars[stage], 2 * sym_bytes);
@@ -225,7 +219,7 @@ __global__ void __launch_bounds__(MAXW * 32, 1) ofdm_fast512_kernel(
     };
     if (lane == 0) {
 #pragma unroll
-        for (int i = 0; i < D; ++i)
+        for (int i = 0; i < kF512Stages; ++i)
             if (static_cast<size_t>(i) < total_steps) issue(i);
     }
 
@@ -303,7 +297,6 @@ __global__ void __launch_bounds__(MAXW * 32, 1) ofdm_fast512_kernel(
         mbar_wait(&bars[stage], parity);
         const float* x0 = S + stage * SS;
         const float* x1 = x0 + 512;
-        if constexpr (INPLACE) tb = reinterpret_cast<float4*>(S + stage * SS);
         const float2* nc = nco_s + sidx * 512 + lane;                 // [q][lane]: entry of sample brev5(lane) + 32 brev4(q)
         // ---- pass A, stage 1 fused with the mixer: elements (2p, 2p+1) = samples (n, n + 256), twiddle 1
         FC2 v[EPL];
@@ -319,10 +312,7 @@ __global__ void __launch_bounds__(MAXW * 32, 1) ofdm_fast512_kernel(
             v[qb].re = fma2(xb, bc(-ob.x), pr); v[qb].im = fma2(xb, bc(-ob.y), pi);
         }
         __syncwarp();                                                  // every lane has taken its samples out of the stage
-        // refill it with the step D ahead -- at once when the stage is only a staging buffer; INPLACE: after the transpose (and after
-        // the SNR scratch of a training step) has finished with it
-        const bool snr_step = snr_db_out && (s < training || (sidx == 0 && training == 0));
-        if (!INPLACE && lane == 0 && t + D < total_steps) issue(stage);
+        if (lane == 0 && t + kF512Stages < total_steps) issue(stage);     // refill it with the step a full ring ahead
         int sg[EPL];
 #pragma unroll
         for (int q = 0; q < EPL; ++q) sg[q] = 1;
@@ -337,35 +327,18 @@ __global__ void __launch_bounds__(MAXW * 32, 1) ofdm_fast512_kernel(
             }
         }
         // ---- transpose: p = 16 lane + q at slot p + (p >> 4); pass B: lane (b8, c) owns p = c + 16 j + 256 b8
-        if constexpr (HALF) {
-            u64* tb2 = reinterpret_cast<u64*>(tb);
 #pragma unroll
-            for (int q = 0; q < EPL; ++q) tb2[17 * lane + q] = v[q].re;
-            __syncwarp();
+        for (int q = 0; q < EPL; ++q) tb[17 * lane + q] = v[q].re;
+        __syncwarp();
 #pragma unroll
-            for (int j = 0; j < EPL; ++j) v[j].re = tb2[c + 17 * j + 272 * b8];
-            __syncwarp();
+        for (int j = 0; j < EPL; ++j) v[j].re = tb[c + 17 * j + 272 * b8];
+        __syncwarp();
 #pragma unroll
-            for (int q = 0; q < EPL; ++q) tb2[17 * lane + q] = v[q].im;
-            __syncwarp();
+        for (int q = 0; q < EPL; ++q) tb[17 * lane + q] = v[q].im;
+        __syncwarp();
 #pragma unroll
-            for (int j = 0; j < EPL; ++j) v[j].im = tb2[c + 17 * j + 272 * b8];
-        } else {
-#pragma unroll
-            for (int q = 0; q < EPL; ++q) {
-                float a0, a1, b0, b1;
-                upk(v[q].re, a0, a1); upk(v[q].im, b0, b1);
-                tb[17 * lane + q] = make_float4(a0, a1, b0, b1);
-            }
-            __syncwarp();
-#pragma unroll
-            for (int j = 0; j < EPL; ++j) {
-                const float4 e = tb[c + 17 * j + 272 * b8];
-                v[j].re = pk(e.x, e.y); v[j].im = pk(e.z, e.w);
-            }
-        }
+        for (int j = 0; j < EPL; ++j) v[j].im = tb[c + 17 * j + 272 * b8];
         __syncwarp();                                                  // the transpose buffer may be rewritten (next step / SNR scratch)
-        if (INPLACE && !snr_step && lane == 0 && t + D < total_steps) issue(stage);
         // ---- pass B, pruned to the two bins this lane pair produces.  Stage 5: full butterflies, odd elements stored negated.
 #pragma unroll
         for (int j = 0; j < EPL; j += 2) {
@@ -432,7 +405,6 @@ __global__ void __launch_bounds__(MAXW * 32, 1) ofdm_fast512_kernel(
             }
             if (final_cfo_out && lane < 2 && (lane == 0 || have1)) final_cfo_out[f0 + lane] = 0.0f;
         }
-        if (INPLACE && snr_step && lane == 0 && t + D < total_steps) issue(stage);
         if (s >= training) {
             // ---- equalize (:747-770) + demodulateSymbol (demodulator.cpp:279-316) + soft_demap.hpp on the lane that owns the carrier,
             //      both frames at once: d = sym * conj(prev) = bin * conj(previous bin) / |h|^2
@@ -517,27 +489,14 @@ __global__ void __launch_bounds__(MAXW * 32, 1) ofdm_fast512_kernel(
             rxp = bin;
         }
         if (++sidx == n_proc) { sidx = 0; pair += GW; }
-        if (++stage == D) { stage = 0; parity ^= 1u; }
+        if (++stage == kF512Stages) { stage = 0; parity ^= 1u; }
     }
     while (qcount > 0) flush();
 }
 
-// Variant switches (read once): PU_F512_INPLACE (default 0) in-place transpose, up to 16 warps at 128 registers -- measured
-// equal to 12 warps with their own transpose buffer (v02: 0.3645 against 0.3618 ms per 53 248 frames: with four warps per
-// scheduler the FMA pipe (math-pipe throttle 0.94 per issue) and the shared-memory pipe (68 %) are the limits, not latency);
-// PU_F512_THALF (default 1) half-size transpose buffer; PU_F512_STAGES (2|3) ring depth; PU_F512_WARPS upper bound on warps per CTA.
-static int f512_env(const char* name, int dflt) {
-    const char* v = getenv(name);
-    return v ? atoi(v) : dflt;
-}
-static bool f512_inplace() { static const int env = f512_env("PU_F512_INPLACE", 0); return env != 0; }
-static bool f512_half() { static const int env = f512_env("PU_F512_THALF", 1); return env != 0 || f512_inplace(); }
-static int f512_stages() { static const int env = f512_env("PU_F512_STAGES", 2); return (env == 3 && !f512_inplace()) ? 3 : 2; }
-static int f512_warps(int n_proc, int stages, bool half, bool inplace) {
-    static const int env = f512_env("PU_F512_WARPS", 0);
-    int w = inplace ? kF512MaxWarpsInplace : kF512MaxWarps;
-    if (env > 0 && env < w) w = env;
-    while (w > 1 && f512_layout(n_proc, w, stages, half, inplace).total > kF512SmemMax) --w;
+static int f512_warps(int n_proc) {
+    int w = kF512MaxWarps;
+    while (w > 1 && f512_layout(n_proc, w).total > kF512SmemMax) --w;
     return w;
 }
 
@@ -555,27 +514,20 @@ bool ofdm_fast512_supported(const OfdmDev& d, int n_symbols, int training, const
     if (!(nlo < 16 && nhi < 16)) return false;
     const size_t total_llr = static_cast<size_t>(n_symbols - training) * d.n_data * d.bps;
     if (total_llr >= 0xffffu || (d.llr_perm && static_cast<size_t>(d.perm_len) >= 0xffffu) || llr_stride == 0) return false;
-    return f512_layout(n_symbols - first, 1, f512_stages(), f512_half(), f512_inplace()).total <= kF512SmemMax;
+    return f512_layout(n_symbols - first, 1).total <= kF512SmemMax;
 }
 
 cudaError_t ofdm_fast512_launch(const OfdmDev& d, const float* samples, size_t B, size_t frame_stride, int n_symbols, int training,
                                 float* llr, size_t llr_stride, int llr_limit, float* snr_db, float* final_cfo, int sm_count, cudaStream_t st) {
     const int first = training > 0 ? training - 1 : 0;
-    const int stages = f512_stages();
-    const bool half = f512_half(), inplace = f512_inplace();
-    const int warps = f512_warps(n_symbols - first, stages, half, inplace);
-    const F512Smem L = f512_layout(n_symbols - first, warps, stages, half, inplace);
-    using Kernel = void (*)(OfdmDev, const float*, size_t, size_t, int, int, float*, size_t, int, float*, float*);
-    const Kernel kernels[5] = {ofdm_fast512_kernel<2, false, false, kF512MaxWarps>, ofdm_fast512_kernel<2, true, false, kF512MaxWarps>,
-                               ofdm_fast512_kernel<3, false, false, kF512MaxWarps>, ofdm_fast512_kernel<3, true, false, kF512MaxWarps>,
-                               ofdm_fast512_kernel<2, true, true, kF512MaxWarpsInplace>};
-    const int which = inplace ? 4 : (stages == 3 ? 2 : 0) + (half ? 1 : 0);
-    static std::atomic<uint64_t> attr_done[5];
-    if (const cudaError_t e = smem_optin(attr_done[which], kernels[which], static_cast<int>(kF512SmemMax)); e != cudaSuccess) return e;
+    const int warps = f512_warps(n_symbols - first);
+    const F512Smem L = f512_layout(n_symbols - first, warps);
+    static std::atomic<uint64_t> attr_done{0};
+    if (const cudaError_t e = smem_optin(attr_done, ofdm_fast512_kernel, static_cast<int>(kF512SmemMax)); e != cudaSuccess) return e;
     const size_t max_ctas = static_cast<size_t>(sm_count > 0 ? sm_count : 148);      // persistent: one CTA per SM
     const size_t want_ctas = ((B + 1) / 2 + warps - 1) / warps;
     const unsigned grid = static_cast<unsigned>(want_ctas < max_ctas ? want_ctas : max_ctas);
-    kernels[which]<<<grid, warps * 32, L.total, st>>>(d, samples, frame_stride, B, n_symbols, training, llr, llr_stride, llr_limit, snr_db, final_cfo);
+    ofdm_fast512_kernel<<<grid, warps * 32, L.total, st>>>(d, samples, frame_stride, B, n_symbols, training, llr, llr_stride, llr_limit, snr_db, final_cfo);
     return cudaGetLastError();
 }
 

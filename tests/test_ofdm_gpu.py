@@ -229,7 +229,7 @@ def test_warp_fft_kernel_is_bit_identical(ctx, preset, mod):
             # M1 DBPSK (25 symbols after the first LTS) does not fit its shared-memory budget and stays on the warp-FFT kernel
             assert fast_kernel == "ofdm_diff512_kernel", (fast_kernel, training, Lcut)
         elif preset == "m1" and mod == R.DBPSK:
-            # fits the packed kernel only in its in-place-transpose variant (PU_P512_INPLACE=1)
+            # whole frames exceed the packed kernel's shared-memory budget, cut ones may fit it
             assert fast_kernel in ("ofdm_diff512_kernel", "ofdm_diff_kernel", "ofdm_presynced_kernel"), (fast_kernel, training, Lcut)
         else:
             assert fast_kernel in ("ofdm_diff_kernel", "ofdm_presynced_kernel"), (fast_kernel, training, Lcut)

@@ -1,5 +1,5 @@
 """Quick demod-kernel-only timing of the bench workload (M1 512-FFT DQPSK presynced frames over AWGN), used during
-development to compare kernel variants:  [PU_P512_WARPS=.. PU_P512_STAGES=.. PU_P512_THALF=.. PU_OFDM_NO_PACKED512=1]
+development to compare kernel changes:
 python tools/ofdm_quick_bench.py [frames_per_point] [mode: m1|m3]"""
 import os
 import sys
